@@ -54,7 +54,14 @@ def errors(model, logits, loss, want):
 def test_oracle_mirror_reproduces_legacy_fixture(case):
     want = np.load(os.path.join(GOLDEN, case + ".npz"))
     oscn.set_numerics("fp32")
-    model, logits, loss = run(oscn, case, "cpu")
+    # the fixtures were recorded with 8 intra-op threads: the oracle's fp32 gradient sums are split by thread, so the
+    # replay reproduces them bit for bit only with the same count, whatever the host's core count
+    threads = torch.get_num_threads()
+    torch.set_num_threads(8)
+    try:
+        model, logits, loss = run(oscn, case, "cpu")
+    finally:
+        torch.set_num_threads(threads)
     assert [n for n, _ in model.named_parameters()] == [str(n) for n in want["param_names"]]
     assert sum(p.numel() for p in model.parameters()) == int(want["n_params"][0])
     errs = errors(model, logits, loss, want)

@@ -1,113 +1,67 @@
-"""Checks against the REFERENCE'S OWN FILES, imported from /root/reference (build container only: the GPU box has no
-reference, the tests skip there).  No GPU needed: transforms are numpy, and constructing a network only allocates
-parameters.
+"""Checks against what the REFERENCE'S OWN FILES produce, recorded in tests/golden/reference_files.json
+(tests/golden/make_reference_files.py says how; the reference tree is not part of this repository).  No GPU needed:
+transforms are numpy, and constructing a network only allocates parameters.
 
   * the host input transforms == the reference's torch_geometric-free twins
     (src/utils/core/larcvio/data_transforms.py:50-142; src/io/data_transforms.py:21-49,198-252 are the same functions
-    behind an unconditional `import torch_geometric`, absent here);
+    behind an unconditional `import torch_geometric`) on the same seeded synthetic batches;
   * the reference's `build_networks` (src/networks/classification_head.py:30-55 -> src/networks/resnet.py:10-161,
-    sparse_building_blocks.py) constructs, UNMODIFIED, on the PRODUCT `sparseconvnet` package, with the state_dict
-    keys, shapes and parameter counts of the repo's mirror (sparseeventid_b200/networks.py).
+    sparse_building_blocks.py) constructed on the PRODUCT `sparseconvnet` package: the repo's mirror
+    (sparseeventid_b200/networks.py) built on the product package has its state_dict keys, shapes, dtypes and
+    parameter counts, and every sparse layer is the product's class.
 """
-import importlib.util
+import hashlib
+import json
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="reference tree not present")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_files.json")
 
 
-def _load(path, name):
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def _record(dataset):
+    with open(GOLDEN) as f:
+        return json.load(f)[dataset]
 
 
 @pytest.mark.parametrize("dataset", ["dune3d", "dune2d"])
 def test_host_transform_matches_reference_twin(dataset):
     from sparseeventid_b200 import data_transforms as mine
     from sparseeventid_b200 import synthetic
-    ref = _load(os.path.join(REF, "src/utils/core/larcvio/data_transforms.py"), "ref_larcvio_transforms")
+    want = _record(dataset)["transform"]
     if dataset == "dune3d":
         arr = synthetic.larcv_batch_3d(5, seed=77, max_voxels=4000)
-        want, got = ref.larcvsparse_to_scnsparse_3d(arr), mine.larcvsparse_to_scnsparse_3d(arr)
+        got = mine.larcvsparse_to_scnsparse_3d(arr)
     else:
         arr = synthetic.larcv_batch_2d(5, seed=77, max_voxels=4000)
-        want, got = ref.larcvsparse_to_scnsparse_2d(arr), mine.larcvsparse_to_scnsparse_2d(arr)
-    assert type(got) is type(want) and len(got) == len(want) == 3
-    for a, b in zip(got[:2], want[:2]):
-        assert a.dtype == b.dtype and a.shape == b.shape and np.array_equal(a, b)
-    assert got[2] == want[2]
+        got = mine.larcvsparse_to_scnsparse_2d(arr)
+    assert type(got).__name__ == want["type"] and len(got) == 3
+    rows = np.asarray(want["sample_rows"])
+    for a, name in zip(got[:2], ("coords", "feats")):
+        w = want[name]
+        assert str(a.dtype) == w["dtype"] and list(a.shape) == w["shape"], name
+        assert np.array_equal(a[rows], np.asarray(want["sample_" + name], dtype=a.dtype)), name
+        assert hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest() == w["sha256"], name
+    assert got[2] == want["batch_size"]
     assert got[0].shape[0] > 1000
 
 
-def _stub_config_modules():
-    """hydra / omegaconf only register dataclasses in src/config; stub them exactly as tests/golden/make_golden.py does."""
-    hydra = types.ModuleType("hydra")
-    core = types.ModuleType("hydra.core")
-    cs = types.ModuleType("hydra.core.config_store")
-
-    class ConfigStore:
-        _inst = None
-
-        @classmethod
-        def instance(cls):
-            cls._inst = cls._inst or cls()
-            return cls._inst
-
-        def store(self, *a, **k):
-            pass
-
-    cs.ConfigStore = ConfigStore
-    hydra.core, core.config_store = core, cs
-    om = types.ModuleType("omegaconf")
-    om.MISSING = "???"
-    return {"hydra": hydra, "hydra.core": core, "hydra.core.config_store": cs, "omegaconf": om}
-
-
 @pytest.mark.parametrize("dataset", ["dune3d", "dune2d"])
-def test_reference_build_networks_constructs_on_product_package(dataset):
+def test_product_networks_match_reference_layout(dataset):
     import sparseconvnet as product
     from sparseeventid_b200 import networks as mirror
     assert product.__name__ == "sparseconvnet" and "sparseeventid_b200" in product.SubmanifoldConvolution.__module__
-    saved = {k: sys.modules.get(k) for k in list(sys.modules) if k == "src" or k.startswith("src.")}
-    stubs = _stub_config_modules()
-    saved.update({k: sys.modules.get(k) for k in stubs})
-    sys.modules.update(stubs)
-    sys.path.insert(0, REF)
-    try:
-        for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-            del sys.modules[k]
-        from src.config.framework import DataMode
-        from src.config.network import ConvRepresentation
-        from src.networks.classification_head import build_networks
-        params = types.SimpleNamespace(data=types.SimpleNamespace(dimension=mirror.DIMENSION[dataset]),
-                                       framework=types.SimpleNamespace(mode=DataMode.sparse), encoder=ConvRepresentation())
-        encoder, head = build_networks(params, list(mirror.IMAGE_SIZE[dataset]), mirror.OUTPUT_SHAPE)
-        ref_model = mirror.EventIDModel(encoder, head)
-        my_model = mirror.EventIDModel(*mirror.build_networks(product, dataset))
-        ref_sd, my_sd = ref_model.state_dict(), my_model.state_dict()
-        assert list(ref_sd.keys()) == list(my_sd.keys())
-        for k in ref_sd:
-            assert ref_sd[k].shape == my_sd[k].shape and ref_sd[k].dtype == my_sd[k].dtype, k
-        n_ref = sum(p.numel() for p in ref_model.parameters())
-        assert n_ref == sum(p.numel() for p in my_model.parameters())
-        assert n_ref == {"dune3d": 20881994, "dune2d": 7173578}[dataset]      # SURVEY.md App. B census
-        # every sparse layer of the reference's encoder is the product's class (nothing fell back to a stub)
-        leaves = [m for m in encoder.modules() if not list(m.children()) and list(m.parameters(recurse=False))]
-        assert len(leaves) > 50, len(leaves)
-        assert {type(m).__module__ for m in leaves} == {"sparseeventid_b200.scn.modules"}
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-            del sys.modules[k]
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+    want = _record(dataset)["layout"]
+    encoder, head = mirror.build_networks(product, dataset)
+    model = mirror.EventIDModel(encoder, head)
+    got = [[k, list(v.shape), str(v.dtype)] for k, v in model.state_dict().items()]
+    assert [e[0] for e in got] == [e[0] for e in want["state_dict"]]
+    for g, w in zip(got, want["state_dict"]):
+        assert g == w, g[0]
+    n = sum(p.numel() for p in model.parameters())
+    assert n == want["n_params"] == {"dune3d": 20881994, "dune2d": 7173578}[dataset]      # SURVEY.md App. B census
+    # every sparse layer of the encoder is the product's class (nothing fell back to a stub)
+    leaves = [m for m in encoder.modules() if not list(m.children()) and list(m.parameters(recurse=False))]
+    assert len(leaves) > 50, len(leaves)
+    assert {type(m).__module__ for m in leaves} == {"sparseeventid_b200.scn.modules"}
