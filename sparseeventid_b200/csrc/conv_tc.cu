@@ -700,6 +700,12 @@ static int g_knob[4] = {-1, -1, -1, -1};      // grid, T, SA, SB: -1 = read the 
 extern "C" void scn_tc_debug_knobs(int grid, int t, int sa, int sb) {
   g_knob[0] = grid; g_knob[1] = t; g_knob[2] = sa; g_knob[3] = sb;
 }
+// the configuration of the last k_conv_tc launch (developer entry like the knobs, for the tests' coverage check):
+// grid, T, NM, nbuf, ksplit, SA, SB, min and max tiles per CTA; written on the host just before the launch
+static int32_t g_last_launch[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+extern "C" void scn_tc_debug_last_launch(int32_t* out) {
+  for (int i = 0; i < 9; ++i) out[i] = g_last_launch[i];
+}
 
 int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nbr, int K, int64_t n_rows,
                    int64_t n_pad, int n_in, int n_out, const void* bimg, const float* bias, __nv_bfloat16* out,
@@ -805,6 +811,12 @@ int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nb
       SCN_CUDA(cudaFuncSetAttribute(tc::k_conv_tc<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       attr_set = true;
     }
+  }
+  if (grid < 1) return SCN_OK;                   // no output row
+  {
+    const int32_t rec[9] = {grid, p.T, p.NM, p.nbuf, p.ksplit, p.SA, p.SB, p.num_tiles / grid,
+                            (p.num_tiles + grid - 1) / grid};
+    for (int i = 0; i < 9; ++i) g_last_launch[i] = rec[i];
   }
   auto launch = [&](auto kern) -> int {
     SCN_CUDA(scn_launch_pdl(kern, dim3((unsigned)grid), dim3(tc::THREADS), smem, s, p));

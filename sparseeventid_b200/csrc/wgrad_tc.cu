@@ -12,7 +12,7 @@
 // table holds every row and gets proportionally more CTAs), so dW receives one pass of atomics per CTA.
 // Roles: producer warps (each walks its share of 128-row blocks, ballots the neighbour indices, appends the live pairs
 // to a ring and emits a stage whenever 64 are pending; LDGSTS copies that signal their own landing), one issuing warp
-// that consumes whichever producer has a stage ready (order is irrelevant for a sum), 4 epilogue warps
+// that consumes the producers' stages in a fixed round-robin order (so dW is bitwise reproducible), 4 epilogue warps
 // (tcgen05.ld -> red.global.add.f32).
 //
 // Replaces SCN's dConvolution_KMxKN_backward_dW_A/B (SURVEY.md 2.2); reference call sites
@@ -231,19 +231,27 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
 #pragma unroll
     for (int w = 0; w < PROD_WARPS; ++w) consumed[w] = 0;
     bool first = true;
-    uint32_t idle = 0;
     for (;;) {
-      bool all_done = true, progressed = false;
+      bool all_done = true;
 #pragma unroll
       for (int w = 0; w < PROD_WARPS; ++w) {
         if (w >= NPW) continue;
-        // one lane's view of the flags, broadcast: the branch below must be warp-uniform
-        const uint32_t dn = __shfl_sync(0xffffffffu, ld_acquire_u32(done + 4u * (uint32_t)w), 0);
-        if (dn != 0u && (uint32_t)consumed[w] + 1u == dn) continue;           // this warp is finished and drained
-        all_done = false;
+        // Stages are consumed in a FIXED order (round robin over the producers, each in its own order), so the fp32
+        // accumulation order in TMEM, and with it every bit of dW, does not depend on timing: wait for producer w's
+        // next stage, or for w to be finished and drained.  (Taking whichever producer was ready first made repeated
+        // launches differ in the last bits.)  One lane's view of the flags, broadcast: the branches must be warp-uniform.
         const int slot = w + (consumed[w] & 1) * NPW;
-        const uint32_t f = __shfl_sync(0xffffffffu, ld_acquire_u32(seq + 4u * (uint32_t)slot), 0);
-        if ((f & 0x7fffffffu) != (uint32_t)consumed[w] + 1u) continue;         // its next stage is not issued yet
+        bool drained = false;
+        uint32_t f = 0, idle = 0;
+        for (;;) {
+          const uint32_t dn = __shfl_sync(0xffffffffu, ld_acquire_u32(done + 4u * (uint32_t)w), 0);
+          if (dn != 0u && (uint32_t)consumed[w] + 1u == dn) { drained = true; break; }
+          f = __shfl_sync(0xffffffffu, ld_acquire_u32(seq + 4u * (uint32_t)slot), 0);
+          if ((f & 0x7fffffffu) == (uint32_t)consumed[w] + 1u) break;         // its next stage is issued
+          if (++idle > 8u * SPIN_LIMIT) __trap();                             // polls of ONE producer (not all NPW)
+        }
+        if (drained) continue;
+        all_done = false;
         __syncwarp();
         mbar_wait(afull(slot), f >> 31);                                       // ... and landed
         tc_fence_after();
@@ -267,11 +275,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
         __syncwarp();
         first = false;
         ++consumed[w];
-        progressed = true;
       }
       if (all_done) break;
-      if (!progressed && ++idle > SPIN_LIMIT) __trap();
-      if (progressed) idle = 0;
     }
     // `first` still true <=> no pair at all in this CTA's range: the epilogue must not add the (uninitialised) accumulator.
     // Written before the commit: the epilogue reads it after the commit's barrier has completed.
@@ -385,6 +390,13 @@ void scn_wgrad_set_bias_fold(const float* colsum, float* dbias, int C, int accum
 }
 bool scn_wgrad_bias_fold_pending() { return wg::g_fold.colsum != nullptr; }
 
+// the configuration of the last k_wgrad_tc launch (developer entry like scn_tc_debug_knobs, for the tests' coverage
+// check): grid, s_other, s_centre, pairs per stage, slots, nca, ncb; written on the host just before the launch
+static int32_t g_wg_last_launch[7] = {0, 0, 0, 0, 0, 0, 0};
+extern "C" void scn_wgrad_debug_last_launch(int32_t* out) {
+  for (int i = 0; i < 7; ++i) out[i] = g_wg_last_launch[i];
+}
+
 bool scn_wgrad_tc_enabled() {
   static int v = -1;
   if (v < 0) {
@@ -457,6 +469,10 @@ int scn_wgrad_tc(const __nv_bfloat16* x, const __nv_bfloat16* dout, const int32_
   }();
   const int CC = Cin * Cout;
   p.part = use_slabs ? wg::wgrad_slabs((size_t)grid * CC * sizeof(float), s) : nullptr;
+  {
+    const int32_t rec[7] = {grid, p.s_other, p.s_centre, pairs, slots, p.nca, p.ncb};
+    for (int i = 0; i < 7; ++i) g_wg_last_launch[i] = rec[i];
+  }
   auto launch = [&](auto kern) -> int {
     SCN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     SCN_CUDA(scn_launch_pdl(kern, dim3((unsigned)grid), dim3(wg::THREADS), smem, s, p));

@@ -36,6 +36,19 @@ def blob_sites(n, grid, batch, seed):
     return np.concatenate(out, 0).astype(np.int64)
 
 
+# bench.py's first batch: host_batch(64, 1234 + 100000 * rank + 1000 * i) with rank = i = 0
+BENCH_BATCH, BENCH_SEED = 64, 1234
+
+
+def bench_batch(batch=BENCH_BATCH, seed=BENCH_SEED):
+    """The benchmark's first batch (64 synthetic dune3d events, ~5e5 active sites): float64 coordinates, float32 features,
+    batch size."""
+    from sparseeventid_b200 import synthetic
+    from sparseeventid_b200.data_transforms import larcvsparse_to_scnsparse_3d
+    c, f, bs = larcvsparse_to_scnsparse_3d(synthetic.larcv_batch_3d(batch, seed=seed))
+    return np.ascontiguousarray(c, dtype=np.float64), np.ascontiguousarray(f, dtype=np.float32), bs
+
+
 def rel_err(a, b):
     a = torch.as_tensor(a).detach().double().cpu()
     b = torch.as_tensor(b).detach().double().cpu()

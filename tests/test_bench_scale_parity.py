@@ -21,19 +21,14 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import init_deterministic
+from helpers import BENCH_BATCH as BATCH
+from helpers import BENCH_SEED as SEED
+from helpers import bench_batch, init_deterministic
 from oracle import scn_oracle as O
 from oracle import sparseconvnet_oracle as oscn
 from sparseeventid_b200 import networks, synthetic
-from sparseeventid_b200.data_transforms import larcvsparse_to_scnsparse_3d
 
-BATCH, SEED = 64, 1234          # bench.py host_batch(64, 1234 + 100000 * rank + 1000 * i) with rank = i = 0
 TOL = 2e-3
-
-
-def bench_batch(batch=BATCH):
-    c, f, bs = larcvsparse_to_scnsparse_3d(synthetic.larcv_batch_3d(batch, seed=SEED))
-    return np.ascontiguousarray(c, dtype=np.float64), np.ascontiguousarray(f, dtype=np.float32), bs
 
 
 def rules_to_table(rules, n_out):
