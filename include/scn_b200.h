@@ -153,10 +153,13 @@ int scn_rulebook_pairs(const int32_t* nbr, int K, int64_t n, int64_t n_pad, int3
  * and one pair-reduction covers every wgrad:
  *     dW[k] += sum_o in[nbr[k][o], :]^T . dout[o, :]
  * `precision`: SCN_PREC_BF16 = bf16 operands on tensor cores, fp32 accumulate (features may be
- * stored fp32 or bf16); SCN_PREC_FP32 = exact fp32 FMA path (fp32 features only).
+ * stored fp32 or bf16); SCN_PREC_FP32 = exact fp32 FMA path (fp32 features only); SCN_PREC_TF32 =
+ * fp32 features, TF32 operands on the tcgen05 tensor cores (10-bit mantissa), fp32 accumulate; shapes
+ * outside the tcgen05 kernels run the exact fp32 FMA path, the one-channel stem its hi/lo bf16 split.
  * ------------------------------------------------------------------------------------------ */
 #define SCN_PREC_FP32 0
 #define SCN_PREC_BF16 1
+#define SCN_PREC_TF32 2
 
 /* Re-lays the fp32 SCN weight W[K][Cin][Cout] for one of the uses above.
  *   transpose=0: B_k = W[k] (Cin x Cout);  transpose=1: B_k = W[src]^T with src = mirror ? K-1-k : k.
@@ -165,13 +168,15 @@ int scn_conv_prep_weights(const float* W, int K, int Cin, int Cout, int transpos
                           int precision, int feat_dtype, void* out, void* stream);
 /* Every weight image of a network in one launch (a trainer calls it once per step, then passes skip_prep = 1 to the
  * module entry points below).  descs: DEVICE array of n x 8 int64 {W pointer, image pointer, K, Cin, Cout,
- * transpose | mirror << 1, index of the image's first element in the concatenated index space, unused}; total =
+ * transpose | mirror << 1, index of the image's first element in the concatenated index space, precision (an image
+ * for SCN_PREC_TF32 holds TF32 values, any other value builds the bf16 image)}; total =
  * sum of K*Cin*Cout.  Only for images of the tcgen05 path (scn_conv_path == 2); an image whose n_in is not a multiple
  * of 64 must have been zero-filled once (its unused half rows are never written). */
 int scn_conv_prep_weights_batched(const void* descs, int n, int64_t total, void* stream);
 /* Which kernel family runs a (K, n_in, n_out) contraction for features of feat_dtype:
  *   0 exact fp32 FMA (B_k fp32 [k][c][n]);  1 mma.sync tensor cores (B_k bf16 [k][n][c]);
- *   2 tcgen05 tensor cores + TMEM (B_k as pre-swizzled 128-byte-row bf16 tiles).
+ *   2 tcgen05 tensor cores + TMEM (B_k as pre-swizzled 128-byte-row tiles: bf16, or TF32 for SCN_PREC_TF32 with
+ *     fp32 features).
  * scn_conv_prep_bytes is the size of the buffer scn_conv_prep_weights fills for that path. */
 int scn_conv_path(int K, int n_in, int n_out, int precision, int feat_dtype);
 size_t scn_conv_prep_bytes(int K, int n_in, int n_out, int precision, int feat_dtype);

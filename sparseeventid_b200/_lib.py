@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("SCN_B200_LIB") or os.path.join(_HERE, "lib", "libscn_
 
 SCN_F32, SCN_BF16 = 0, 1
 COORD_CODES = {torch.int64: 0, torch.int32: 1, torch.float32: 2, torch.float64: 3}
-PREC_FP32, PREC_BF16 = 0, 1
+PREC_FP32, PREC_BF16, PREC_TF32 = 0, 1, 2
 
 _p, _i, _i64, _f, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t
 

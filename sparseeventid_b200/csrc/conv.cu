@@ -1,5 +1,5 @@
 // Convolution arithmetic, first generation: output-stationary gather-GEMM on the neighbour table.
-//   * exact fp32 FMA kernels (precision SCN_PREC_FP32, odd channel counts, and the Cin=1 stem)
+//   * exact fp32 FMA kernels (precision SCN_PREC_FP32, odd channel counts, and the Cin=1 stem in that mode)
 //   * bf16-operand / fp32-accumulate tensor-core kernels built on mma.sync (HMMA) -- the
 //     baseline that conv_tc.cu (tcgen05 + TMEM) supersedes for the hot layer shapes.
 // Replaces SCN's Convolution.cu dConvolution_KMxKN_forward/backward_dW (SURVEY.md 2.2; reference
@@ -9,20 +9,19 @@
 // conv_tc.cu (tcgen05 path)
 bool scn_tc_disabled();
 bool scn_tc_shape_ok(int K, int n_in, int n_out);
-size_t scn_tc_image_bytes(int K, int n_in, int n_out);
-int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mirror, void* out, cudaStream_t s);
+size_t scn_tc_image_bytes(int K, int n_in, int n_out, int tf32);
+int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mirror, int tf32, void* out, cudaStream_t s);
 bool scn_wgrad_tc_enabled();
 bool scn_stem_tc_enabled();                       // stem_tc.cu
 bool scn_stem_tc_shape_ok(int K, int n_in, int n_out);
 int scn_stem_tc_forward(const void* x, int x_dtype, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, const float* W,
-                        const float* bias, __nv_bfloat16* out, cudaStream_t s);
-int scn_stem_tc_wgrad(const void* x, int x_dtype, const __nv_bfloat16* dout, const int32_t* nbr, int K, int64_t n_rows,
+                        const float* bias, void* out, int out_dtype, cudaStream_t s);
+int scn_stem_tc_wgrad(const void* x, int x_dtype, const void* dout, int dout_dtype, const int32_t* nbr, int K, int64_t n_rows,
                       int64_t n_pad, float* dW, cudaStream_t s);
-int scn_wgrad_tc(const __nv_bfloat16* x, const __nv_bfloat16* dout, const int32_t* nbr, int K, int64_t n_rows,
-                 int64_t n_pad, int Cin, int Cout, float* dW, cudaStream_t s);
-int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nbr, int K, int64_t n_rows,
-                   int64_t n_pad, int n_in, int n_out, const void* bimg, const float* bias, __nv_bfloat16* out,
-                   cudaStream_t s);
+int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int Cin, int Cout,
+                 int tf32, float* dW, cudaStream_t s);
+int scn_tc_forward(const void* in, int64_t n_in_rows, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int n_in,
+                   int n_out, const void* bimg, const float* bias, void* out, int tf32, cudaStream_t s);
 
 namespace {
 
@@ -531,12 +530,16 @@ int wgrad_generic_t(const TI* in, const TO* dout, const int32_t* nbr, int K, int
 
 }  // namespace
 
-// 0: exact fp32 FMA kernels; 1: mma.sync (HMMA) kernels, Bt[k][n][c] bf16; 2: tcgen05 kernel, swizzled image
+// 0: exact fp32 FMA kernels; 1: mma.sync (HMMA) kernels, Bt[k][n][c] bf16; 2: tcgen05 kernel, swizzled image (bf16
+// features with SCN_PREC_BF16, fp32 features with SCN_PREC_TF32)
 static int conv_path(int K, int n_in, int n_out, int precision, int feat_dtype) {
-  if (precision == SCN_PREC_BF16 && feat_dtype == SCN_BF16 && !scn_tc_disabled() && scn_tc_shape_ok(K, n_in, n_out))
-    return 2;
+  const bool tc_mode = (precision == SCN_PREC_BF16 && feat_dtype == SCN_BF16) ||
+                       (precision == SCN_PREC_TF32 && feat_dtype == SCN_F32);
+  if (tc_mode && !scn_tc_disabled() && scn_tc_shape_ok(K, n_in, n_out)) return 2;
   return mma_ok(K, n_in, n_out, precision) ? 1 : 0;
 }
+// the tcgen05 path of a precision runs its TF32 instantiation
+static int tc_tf32(int precision) { return precision == SCN_PREC_TF32 ? 1 : 0; }
 
 extern "C" int scn_conv_path(int K, int n_in, int n_out, int precision, int feat_dtype) {
   return conv_path(K, n_in, n_out, precision, feat_dtype);
@@ -544,7 +547,7 @@ extern "C" int scn_conv_path(int K, int n_in, int n_out, int precision, int feat
 
 extern "C" size_t scn_conv_prep_bytes(int K, int n_in, int n_out, int precision, int feat_dtype) {
   switch (conv_path(K, n_in, n_out, precision, feat_dtype)) {
-    case 2: return scn_tc_image_bytes(K, n_in, n_out);
+    case 2: return scn_tc_image_bytes(K, n_in, n_out, tc_tf32(precision));
     case 1: return (size_t)K * n_in * n_out * 2;
     default: return (size_t)K * n_in * n_out * 4;
   }
@@ -558,7 +561,7 @@ extern "C" int scn_conv_prep_weights(const float* W, int K, int Cin, int Cout, i
   int64_t total = (int64_t)K * Cin * Cout;
   unsigned g = grid_for(total, 256);
   const int path = conv_path(K, n_in, n_out, precision, feat_dtype);
-  if (path == 2) return scn_tc_prep(W, K, Cin, Cout, transpose, mirror, out, s);
+  if (path == 2) return scn_tc_prep(W, K, Cin, Cout, transpose, mirror, tc_tf32(precision), out, s);
   if (path == 1)
     k_prep_weights<__nv_bfloat16, 1><<<g, 256, 0, s>>>(W, K, Cin, Cout, transpose, mirror, (__nv_bfloat16*)out);
   else
@@ -575,8 +578,7 @@ extern "C" int scn_conv_forward(const void* in, int in_dtype, int64_t n_in_rows,
   if (!in || !nbr || !Bprep || !out || K < 1 || n_pad < n_out_rows || (n_pad & 127)) return SCN_ERR_ARG;
   if (precision == SCN_PREC_FP32 && (in_dtype != SCN_F32 || out_dtype != SCN_F32)) return SCN_ERR_ARG;
   if (in_dtype == out_dtype && conv_path(K, n_in, n_out, precision, in_dtype) == 2)
-    return scn_tc_forward((const __nv_bfloat16*)in, n_in_rows, nbr, K, n_out_rows, n_pad, n_in, n_out, Bprep, bias,
-                          (__nv_bfloat16*)out, s);
+    return scn_tc_forward(in, n_in_rows, nbr, K, n_out_rows, n_pad, n_in, n_out, Bprep, bias, out, tc_tf32(precision), s);
   if (mma_ok(K, n_in, n_out, precision) && in_dtype == out_dtype) {
     if (in_dtype == SCN_F32)
       return conv_mma_t<float>((const float*)in, nbr, K, n_out_rows, n_pad, n_in, n_out, (const __nv_bfloat16*)Bprep,
@@ -588,10 +590,11 @@ extern "C" int scn_conv_forward(const void* in, int in_dtype, int64_t n_in_rows,
   }
   if (mma_ok(K, n_in, n_out, precision)) return SCN_ERR_UNSUPPORTED;   // Bprep is bf16 for this shape
   const float* B = (const float*)Bprep;
-  // the stem (one input channel) as a dense GEMM over the neighbour table on tensor cores (stem_tc.cu); the exact fp32
-  // mode keeps the FFMA kernel
-  if (precision != SCN_PREC_FP32 && out_dtype == SCN_BF16 && scn_stem_tc_enabled() && scn_stem_tc_shape_ok(K, n_in, n_out))
-    return scn_stem_tc_forward(in, in_dtype, nbr, K, n_out_rows, n_pad, B, bias, (__nv_bfloat16*)out, s);
+  // the stem (one input channel) as a dense GEMM over the neighbour table on tensor cores (stem_tc.cu): bf16 outputs,
+  // and fp32 outputs in the tf32 mode; the exact fp32 mode keeps the FFMA kernel
+  if (precision != SCN_PREC_FP32 && (out_dtype == SCN_BF16 || precision == SCN_PREC_TF32) && scn_stem_tc_enabled() &&
+      scn_stem_tc_shape_ok(K, n_in, n_out))
+    return scn_stem_tc_forward(in, in_dtype, nbr, K, n_out_rows, n_pad, B, bias, out, out_dtype, s);
   if (in_dtype == SCN_F32 && out_dtype == SCN_F32)
     return conv_generic_t<float, float>((const float*)in, nbr, K, n_out_rows, n_pad, n_in, n_out, B, bias, (float*)out, s);
   if (in_dtype == SCN_F32 && out_dtype == SCN_BF16)
@@ -613,17 +616,19 @@ extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, in
   if (n_rows == 0) return SCN_OK;
   if (!in || !dout || !nbr || !dW || K < 1 || n_pad < n_rows) return SCN_ERR_ARG;
   if (precision == SCN_PREC_FP32 && (in_dtype != SCN_F32 || dout_dtype != SCN_F32)) return SCN_ERR_ARG;
-  if (precision == SCN_PREC_BF16 && in_dtype == SCN_BF16 && dout_dtype == SCN_BF16 && !scn_tc_disabled() &&
-      scn_wgrad_tc_enabled() && (n_pad & 127) == 0) {
+  const bool tc_bf16 = precision == SCN_PREC_BF16 && in_dtype == SCN_BF16 && dout_dtype == SCN_BF16;
+  const bool tc_tf = precision == SCN_PREC_TF32 && in_dtype == SCN_F32 && dout_dtype == SCN_F32;
+  if ((tc_bf16 || tc_tf) && !scn_tc_disabled() && scn_wgrad_tc_enabled() && (n_pad & 127) == 0) {
     // tcgen05 path.  The number of rows of `in` is not part of this entry point's signature; the kernel addresses
     // gathered rows through 32-bit offsets in 16-byte units, i.e. feature matrices up to 64 GB.
-    int rc = scn_wgrad_tc((const __nv_bfloat16*)in, (const __nv_bfloat16*)dout, nbr, K, n_rows, n_pad, n_in, n_out, dW, s);
+    int rc = scn_wgrad_tc(in, dout, nbr, K, n_rows, n_pad, n_in, n_out, tc_tf ? 1 : 0, dW, s);
     if (rc != SCN_ERR_UNSUPPORTED) return rc;
   }
-  // the stem (one input channel): dense GEMM over the neighbour table on tensor cores (stem_tc.cu)
-  if (precision != SCN_PREC_FP32 && dout_dtype == SCN_BF16 && (n_pad & 127) == 0 && scn_stem_tc_enabled() &&
-      scn_stem_tc_shape_ok(K, n_in, n_out))
-    return scn_stem_tc_wgrad(in, in_dtype, (const __nv_bfloat16*)dout, nbr, K, n_rows, n_pad, dW, s);
+  // the stem (one input channel): dense GEMM over the neighbour table on tensor cores (stem_tc.cu); bf16 dout, and fp32
+  // dout in the tf32 mode
+  if (precision != SCN_PREC_FP32 && (dout_dtype == SCN_BF16 || precision == SCN_PREC_TF32) && (n_pad & 127) == 0 &&
+      scn_stem_tc_enabled() && scn_stem_tc_shape_ok(K, n_in, n_out))
+    return scn_stem_tc_wgrad(in, in_dtype, dout, dout_dtype, nbr, K, n_rows, n_pad, dW, s);
   if (mma_ok(K, n_in, n_out, precision) && in_dtype == dout_dtype) {
     if (in_dtype == SCN_F32)
       return wgrad_mma_t<float>((const float*)in, (const float*)dout, nbr, K, n_rows, n_pad, n_in, n_out, dW, s);

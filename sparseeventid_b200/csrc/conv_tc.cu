@@ -1,5 +1,5 @@
 // Output-stationary gather-GEMM convolution on 5th-generation tensor cores (sm_100a only):
-//     out[o, :] = bias + sum_k  in[nbr[k][o], :] . B_k            (bf16 operands, fp32 accumulate)
+//     out[o, :] = bias + sum_k  in[nbr[k][o], :] . B_k            (bf16 or TF32 operands, fp32 accumulate)
 //
 // One persistent CTA per SM owns a contiguous range of 128-row output tiles (an even split of the tiles over the
 // grid) and walks it in GROUPS of T tiles whose accumulators live in TMEM together (T * n_out <= 256 columns with two
@@ -17,6 +17,12 @@
 //     result.  Only the first stage of a tile, which initialises the accumulator, is written in full,
 //   * 4 epilogue warps drain finished accumulators (tcgen05.ld), add bias, convert and store.
 // Every output row is written exactly once: no atomics, deterministic.
+//
+// TF32 instantiation (precision SCN_PREC_TF32, fp32 features): the same machinery at byte level -- a stage is still one
+// 128-byte row per output row, now 32 fp32 channels, and one tcgen05.mma (kind::tf32, K = 8) still consumes 32 bytes of
+// it, so only the channels per stage (32), the instruction descriptor, the weight image and the fp32 epilogue differ.
+// The MMA reads the fp32 bits of the gathered rows as they are (the tensor core uses their upper 19 bits); the weight
+// image holds values rounded to TF32 (cvt.rna).  No offset pairing: a 32-channel fp32 row already fills a stage.
 //
 // Synchronisation notes.  A slot's mbarriers must see consecutive phases from each waiter (a parity wait cannot tell
 // phase r from r-2), hence one producer warp per pair of slots; the issuing warps run up to SA stages apart, so the
@@ -41,7 +47,8 @@
 namespace tc {
 
 constexpr int BM = 128;                 // output rows per tile == TMEM lanes
-constexpr int KC = 64;                  // channels per pipeline stage (one 128-byte swizzle row)
+constexpr int KC = 64;                  // bf16 channels per pipeline stage (one 128-byte swizzle row)
+constexpr int KC_TF32 = 32;             // fp32 channels per pipeline stage
 constexpr int A_BYTES = BM * 128;       // 16 KB
 constexpr int EPI_WARPS = 4;            // warps 0..3  (TMEM lane quarter = warp index)
 constexpr int NGRP = 4;                 // producer groups: stage n is gathered by group n mod NGRP ...
@@ -66,25 +73,42 @@ __device__ __forceinline__ uint64_t make_desc_sw128(uint32_t saddr) {
   d |= (uint64_t)2 << 61;       // LayoutType::SWIZZLE_128B
   return d;
 }
-// kind::f16 instruction descriptor: bf16 x bf16 -> fp32, A and B K-major, M=128, N=n
 // base + 16 * units as ONE instruction (IMAD.WIDE.U32 with a 64-bit addend)
 __device__ __forceinline__ const unsigned char* mad_wide16(uint32_t units, const unsigned char* base) {
   uint64_t r;
   asm("mad.wide.u32 %0, %1, 16, %2;" : "=l"(r) : "r"(units), "l"((uint64_t)(uintptr_t)base));
   return reinterpret_cast<const unsigned char*>((uintptr_t)r);
 }
+// instruction descriptor: fp32 accumulate, A and B K-major, M=128, N=n; a/b format bf16 (kind::f16) or TF32 (kind::tf32)
+template <bool TF32>
 __device__ __forceinline__ uint32_t make_idesc(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+  constexpr uint32_t fmt = TF32 ? 2u : 1u;
+  return (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+}
+// 8 consecutive output values of a row, out + idx .. out + idx + 7: one 16-byte store (bf16) or two (fp32)
+template <bool TF32>
+__device__ __forceinline__ void store8(void* out, int64_t idx, const float* f) {
+  if constexpr (TF32) {
+    float4* d = reinterpret_cast<float4*>(reinterpret_cast<float*>(out) + idx);
+    d[0] = make_float4(f[0], f[1], f[2], f[3]);
+    d[1] = make_float4(f[4], f[5], f[6], f[7]);
+  } else {
+    uint4 u;
+    u.x = pack_bf16x2(f[0], f[1]); u.y = pack_bf16x2(f[2], f[3]);
+    u.z = pack_bf16x2(f[4], f[5]); u.w = pack_bf16x2(f[6], f[7]);
+    *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(out) + idx) = u;
+  }
 }
 struct Params {
-  const __nv_bfloat16* in;      // [n_in_rows, n_in]
+  const void* in;               // [n_in_rows, n_in] bf16 (fp32 for the TF32 instantiation)
   const int32_t* nbr;           // [K][n_pad]
   const unsigned char* bimg;    // [K*nch][n_out][128 B] pre-swizzled weight tiles, one per stage
   const float* bias;            // [n_out] or null
-  __nv_bfloat16* out;           // [n_rows, n_out]
+  void* out;                    // [n_rows, n_out], the element type of `in`
   int64_t n_rows, n_pad;
   int K, n_in, n_out;
-  int last_kc;                  // channels in the last 64-channel chunk of an offset (64 or 32)
+  int nch;                      // channel chunks (stages) per offset
+  int last_kc;                  // channels in the last chunk of an offset (bf16: 64 or 32; TF32: 32)
   int T;                        // tiles per group
   int SA, SB;                   // A / B ring depth
   int num_tiles;
@@ -98,8 +122,14 @@ struct Params {
 
 // NCH: 64-channel chunks per offset = ceil(n_in / 64).  PAIR (n_in == 32, NCH == 1): one stage holds TWO offsets,
 // 32 channels each (chunks 0-3 from offset 2q, chunks 4-7 from offset 2q+1), halving the stage count.
-template <int NCH, bool PAIR>
+// TF32: fp32 features and TF32 MMAs, 32-channel chunks; NCH == 0 takes the chunk count (1..8) from p.nch, so that one
+// instantiation serves every width.
+template <int NCH, bool PAIR, bool TF32 = false>
 __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
+  static_assert(!(TF32 && PAIR), "a 32-channel fp32 row fills a stage");
+  constexpr int ESZ = TF32 ? 4 : 2;                        // bytes per element
+  constexpr int KCE = 128 / ESZ;                           // channels per full stage
+  const int nch = NCH > 0 ? NCH : p.nch;
   extern __shared__ unsigned char smem_raw[];
   pdl_launch_dependents();                                 // the next kernel's CTAs may be scheduled as ours retire (common.cuh)
   const uint32_t raw = smem_u32(smem_raw);
@@ -151,7 +181,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
   const int my_groups = (my_tiles + T - 1) / T;
   auto tiles_in_group = [&](int g) { return my_tiles - g * T < T ? my_tiles - g * T : T; };
   const int NSTEP = PAIR ? (p.K + 1) / 2 : p.K;            // offsets (offset pairs) per tile
-  const int Q = NSTEP * NCH;                                // stages per tile
+  const int Q = NSTEP * nch;                                // stages per tile
   // K-split: a CTA with ONE tile (the deep levels: fewer tiles than SMs) would run all its stages through one issuing
   // warp, a serial chain of ~800 cycles per stage.  With two classes the stages are dealt q = 0, 2, 4, ... / 1, 3, 5, ...
   // to two issuing warps with separate TMEM accumulators (columns 0 and n_out), which the epilogue adds.
@@ -208,8 +238,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
     constexpr int IPP = 32 / LPI;                        // items per pass
     const int chunk = lane % LPI, isub = lane / LPI;
     // list items: .x source row offset / 16 B (-1: zeros), .y smem address
-    const uint32_t row_vec = (uint32_t)p.n_in >> 3;      // 16-byte units per feature row (list offsets are in these units)
-    const int last_chunks = p.last_kc >> 3;
+    const uint32_t row_vec = (uint32_t)p.n_in >> (TF32 ? 2 : 3);   // 16-byte units per feature row (list offsets are in these units)
+    const int last_chunks = p.last_kc * ESZ / 16;
     const uint32_t lt = (1u << lane) - 1u;
     const uint32_t csw = (uint32_t)chunk << 4;
     // swizzled address of (row 32 wq + lane, 16-byte chunk 0) in slot 0 (upper half, PAIR: ^ 0x40)
@@ -225,7 +255,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
     const int64_t qstride = (int64_t)p.n_pad * (PAIR ? 2 : 1);
     auto next_q = [&]() {
       ++q;
-      if (++cc == NCH) { cc = 0; qptr += qstride; }
+      if (++cc == nch) { cc = 0; qptr += qstride; }
     };
     auto step = [&]() {
       if (ksplit) {                                      // this class's stages: q = cls, cls + 2, ... of the only tile
@@ -255,14 +285,14 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
       if (valid()) step();
     // Neighbour indices are fetched TWO stages ahead (the cursor runs ahead of the stage being gathered): one stage of
     // lead (~500 cycles of this warp's own work) does not cover an L2 round trip under load.  A fetch returns the
-    // stage's (q << 2 | cc), or -1 when no stage is left, so the cursor never has to be rewound.
+    // stage's (q << 3 | cc), or -1 when no stage is left, so the cursor never has to be rewound.
     auto fetch = [&](int& jl_, int& jh_, int& q_) {
       q_ = -1; jl_ = -1; jh_ = -1;
       if (valid()) {
         const int32_t* src = qptr + t * BM;
         jl_ = ldg_nc32(src);
         if (PAIR && (2 * q + 1 < p.K)) jh_ = ldg_nc32(src + p.n_pad);
-        q_ = (q << 2) | cc;
+        q_ = (q << 3) | cc;
         for (int i = 0; i < gpc; ++i) step();
       }
     };
@@ -274,8 +304,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
       if (wq == 0) mark(grp, it, 0);
       int2* list = reinterpret_cast<int2*>(lists + (pw * 2 + (it & 1)) * LIST_BYTES);   // two list buffers per warp, alternating
       const int slot = cls * spc + ls;
-      const int ccur = qc & 3;                           // 64-channel chunk of the offset
-      const bool full = qc < (ksplit ? 8 : 4);           // first stage of an accumulator (q == 0; K-split: q < 2): unmasked MMA, every row written
+      const int ccur = qc & 7;                           // channel chunk of the offset
+      const bool full = qc < (ksplit ? 16 : 8);          // first stage of an accumulator (q == 0; K-split: q < 2): unmasked MMA, every row written
       const uint32_t dst = drow + (uint32_t)slot * A_BYTES;
       // ---- live rows -> list (full stage: every row, missing ones as zeros) ----------------------------------
       const uint32_t bl = __ballot_sync(0xffffffffu, jl >= 0);
@@ -316,7 +346,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
         if (PAIR) amask[slot * 8 + 4 + wq] = ~bh;
       }
       const int npass = (nlive + IPP - 1) / IPP;         // <= 8
-      const bool lane_on = PAIR ? true : chunk < (ccur == NCH - 1 ? last_chunks : 8);
+      const bool lane_on = PAIR ? true : chunk < (ccur == nch - 1 ? last_chunks : 8);
       const unsigned char* src0 = reinterpret_cast<const unsigned char*>(p.in) + ((uint32_t)ccur * 128u + csw);
       if (lane_on && !(exp_flags & 1)) {
         if (!full) {
@@ -388,7 +418,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
     // are dealt to NM = 1, 2 or 4 issuing warps (classes): warp m issues tiles m, m + NM, ...
     const int m = warp - WARP_MMA;                                    // == class
     if (m < NM) {
-      const uint32_t idesc = make_idesc(p.n_out);
+      const uint32_t idesc = make_idesc<TF32>(p.n_out);
       const uint64_t da0 = make_desc_sw128(a_base), db0 = make_desc_sw128(b_base);
       const int nbuf = p.nbuf;
       int bslot = 0;
@@ -398,10 +428,11 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
       int it = 0;
       // one stage: wait for its four quarters (and their masks), issue its MMAs into columns `col`, free the A slot
       auto issue_stage = [&](int q, uint32_t col, uint64_t db, bool first) {
-        const int cc = PAIR ? 0 : q % NCH;
-        const int step = PAIR ? q : q / NCH;
-        // PAIR with an odd K: the last stage holds one offset only, its upper 32 channels are never written
-        const int nk = PAIR ? ((2 * step + 1 < p.K) ? 4 : 2) : ((cc == NCH - 1 ? p.last_kc : KC) >> 4);
+        const int cc = PAIR ? 0 : q % nch;
+        const int step = PAIR ? q : q / nch;
+        // MMAs of 32 bytes of K each.  PAIR with an odd K: the last stage holds one offset only, its upper 32 channels
+        // are never written
+        const int nk = PAIR ? ((2 * step + 1 < p.K) ? 4 : 2) : ((cc == nch - 1 ? p.last_kc : KCE) * ESZ / 32);
         const int aslot = m * spc + ls;
         mark(4 + m, it, 0);
         mbar_wait(afull(aslot), around & 1u);                // all four quarters of the stage have landed (and their masks)
@@ -432,8 +463,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
           for (int kk = 0; kk < 4; ++kk) {
             if (kk < nk && !(exp_flags & 2)) {
               const bool hi = PAIR && kk >= 2;
-              umma_masked(tmem_d, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc, (!first || kk > 0) ? 1u : 0u,
-                          hi ? h0 : m0, hi ? h1 : m1, hi ? h2 : m2, hi ? h3 : m3);
+              umma_masked<TF32>(tmem_d, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc, (!first || kk > 0) ? 1u : 0u,
+                                hi ? h0 : m0, hi ? h1 : m1, hi ? h2 : m2, hi ? h3 : m3);
             }
           }
           umma_commit(aempty(aslot));                                  // frees the A slot when these MMAs retire
@@ -492,7 +523,6 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
         uint32_t a[16], b[16];
         tmem_ld16x2(taddr + (uint32_t)c0, taddr + (uint32_t)(p.n_out + c0), a, b);
         if (row < p.n_rows && !(exp_flags & 4)) {
-          uint4* dst = reinterpret_cast<uint4*>(p.out + row * p.n_out + c0);
 #pragma unroll
           for (int gq = 0; gq < 2; ++gq) {
             float f[8];
@@ -500,10 +530,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
             for (int e = 0; e < 8; ++e)
               f[e] = __uint_as_float(a[gq * 8 + e]) + __uint_as_float(b[gq * 8 + e]) +
                      (p.bias ? __ldg(p.bias + c0 + gq * 8 + e) : 0.f);
-            uint4 u;
-            u.x = pack_bf16x2(f[0], f[1]); u.y = pack_bf16x2(f[2], f[3]);
-            u.z = pack_bf16x2(f[4], f[5]); u.w = pack_bf16x2(f[6], f[7]);
-            dst[gq] = u;
+            store8<TF32>(p.out, row * p.n_out + c0 + gq * 8, f);
           }
         }
       }
@@ -524,17 +551,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
           uint32_t v[32];
           tmem_ld32(taddr + (uint32_t)c0, v);
           if (row < p.n_rows && !(exp_flags & 4)) {
-            uint4* dst = reinterpret_cast<uint4*>(p.out + row * p.n_out + c0);
 #pragma unroll
             for (int gq = 0; gq < 4; ++gq) {
               float f[8];
 #pragma unroll
               for (int e = 0; e < 8; ++e)
                 f[e] = __uint_as_float(v[gq * 8 + e]) + (p.bias ? __ldg(p.bias + c0 + gq * 8 + e) : 0.f);
-              uint4 u;
-              u.x = pack_bf16x2(f[0], f[1]); u.y = pack_bf16x2(f[2], f[3]);
-              u.z = pack_bf16x2(f[4], f[5]); u.w = pack_bf16x2(f[6], f[7]);
-              dst[gq] = u;
+              store8<TF32>(p.out, row * p.n_out + c0 + gq * 8, f);
             }
           }
         }
@@ -556,8 +579,9 @@ __global__ void __launch_bounds__(THREADS, 1) k_conv_tc(const Params p) {
 
 // Weight image: one tile per stage q = k*nch + c/64: n_out rows of 128 bytes; the 16-byte chunk (c%64)/8 of row n
 // is stored at chunk position chunk ^ (n & 7) (the SWIZZLE_128B pattern); unused half rows stay zero.
+// tf32: q = k*nch + c/32, chunk (c%32)/4, values rounded to TF32 (cvt.rna) and stored as fp32 bits.
 __global__ void k_prep_weights_tc(const float* __restrict__ W, int K, int Cin, int Cout, int transpose, int mirror,
-                                  int nch, int pair, __nv_bfloat16* __restrict__ img) {
+                                  int nch, int pair, int tf32, void* __restrict__ img) {
   const int n_in = transpose ? Cout : Cin, n_out = transpose ? Cin : Cout;
   int64_t total = (int64_t)K * n_in * n_out;
   int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -568,15 +592,20 @@ __global__ void k_prep_weights_tc(const float* __restrict__ W, int K, int Cin, i
   int src_k = (transpose && mirror) ? K - 1 - k : k;
   int ci = transpose ? n : c, co = transpose ? c : n;
   float v = W[((int64_t)src_k * Cin + ci) * Cout + co];
+  if (tf32) {
+    const int q = k * nch + c / KC_TF32, chunk = (c % KC_TF32) >> 2;
+    reinterpret_cast<float*>(img)[((size_t)q * n_out + n) * 32 + (size_t)((chunk ^ (n & 7)) << 2) + (c & 3)] = to_tf32_rna(v);
+    return;
+  }
   // pair (n_in == 32): stage q = k/2, chunks 0-3 <- offset 2q, chunks 4-7 <- offset 2q+1
   const int q = pair ? (k >> 1) : k * nch + c / KC;
   const int chunk = pair ? (k & 1) * 4 + (c >> 3) : (c % KC) >> 3;
   size_t off = ((size_t)q * n_out + n) * 64 + (size_t)((chunk ^ (n & 7)) << 3) + (c & 7);
-  img[off] = __float2bfloat16_rn(v);
+  reinterpret_cast<__nv_bfloat16*>(img)[off] = __float2bfloat16_rn(v);
 }
 
 // All weight images of a network in ONE launch (the trainer calls it once per step instead of 112 per-module launches):
-// descs = n x 8 int64 {W, img, K, Cin, Cout, transpose | mirror << 1, first element index, unused}; element i of the
+// descs = n x 8 int64 {W, img, K, Cin, Cout, transpose | mirror << 1, first element index, precision}; element i of the
 // concatenated index space belongs to the descriptor d with first[d] <= i < first[d + 1].  A thread builds ONE 16-byte
 // chunk of an image (8 consecutive input channels of one output channel): units of a descriptor are numbered
 // (offset, 8-channel block, output channel) with the output channel fastest, so that the forward image's strided reads
@@ -598,7 +627,9 @@ __global__ void __launch_bounds__(256) k_prep_weights_tc_batched(const long long
   unsigned char* img = reinterpret_cast<unsigned char*>(d[1]);
   const int K = (int)d[2], Cin = (int)d[3], Cout = (int)d[4], transpose = (int)(d[5] & 1), mirror = (int)((d[5] >> 1) & 1);
   const int n_in = transpose ? Cout : Cin, n_out = transpose ? Cin : Cout;
-  const int nch = (n_in + KC - 1) / KC, pair = n_in == 32;
+  const bool tf32 = d[7] == SCN_PREC_TF32;
+  const int kc = tf32 ? KC_TF32 : KC;
+  const int nch = (n_in + kc - 1) / kc, pair = !tf32 && n_in == 32;
   const int u = (int)((e - d[6]) >> 3);               // unit within the descriptor
   const int per_k = (n_in >> 3) * n_out;
   const int k = u / per_k;
@@ -615,6 +646,15 @@ __global__ void __launch_bounds__(256) k_prep_weights_tc_batched(const long long
     const float* src = W + ((long long)src_k * Cin + c0) * Cout + nn;
 #pragma unroll
     for (int j = 0; j < 8; ++j) v[j] = __ldg(src + (long long)j * Cout);
+  }
+  if (tf32) {                                         // the 8 channels are 16-byte chunks c, c + 1 (4 fp32 each)
+    const int q = k * nch + c0 / KC_TF32, chunk = (c0 % KC_TF32) >> 2;
+    unsigned char* row = img + ((size_t)q * n_out + nn) * 128;
+    *reinterpret_cast<float4*>(row + ((chunk ^ (nn & 7)) << 4)) =
+        make_float4(to_tf32_rna(v[0]), to_tf32_rna(v[1]), to_tf32_rna(v[2]), to_tf32_rna(v[3]));
+    *reinterpret_cast<float4*>(row + (((chunk + 1) ^ (nn & 7)) << 4)) =
+        make_float4(to_tf32_rna(v[4]), to_tf32_rna(v[5]), to_tf32_rna(v[6]), to_tf32_rna(v[7]));
+    return;
   }
   // pair (n_in == 32): stage q = k/2, chunks 0-3 <- offset 2q, chunks 4-7 <- offset 2q+1
   const int q = pair ? (k >> 1) : k * nch + c0 / KC;
@@ -662,21 +702,26 @@ bool scn_tc_shape_ok(int K, int n_in, int n_out) {
   return K >= 1 && (n_in % 32) == 0 && (n_out % 32) == 0 && n_in >= 32 && n_in <= 256 && n_out >= 32 && n_out <= 256;
 }
 
-// n_in == 32: two offsets share a 64-channel stage
-static bool tc_pair(int n_in) { return n_in == 32; }
+// bf16, n_in == 32: two offsets share a 64-channel stage
+static bool tc_pair(int n_in, int tf32) { return !tf32 && n_in == 32; }
+// channel chunks (stages) per offset: 64 bf16 or 32 fp32 channels each
+static int tc_nch(int n_in, int tf32) {
+  const int kc = tf32 ? tc::KC_TF32 : tc::KC;
+  return (n_in + kc - 1) / kc;
+}
 
-size_t scn_tc_image_bytes(int K, int n_in, int n_out) {
-  const size_t stages = tc_pair(n_in) ? (size_t)(K + 1) / 2 : (size_t)K * ((n_in + tc::KC - 1) / tc::KC);
+size_t scn_tc_image_bytes(int K, int n_in, int n_out, int tf32) {
+  const size_t stages = tc_pair(n_in, tf32) ? (size_t)(K + 1) / 2 : (size_t)K * tc_nch(n_in, tf32);
   return stages * n_out * 128;
 }
 
-int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mirror, void* out, cudaStream_t s) {
+int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mirror, int tf32, void* out, cudaStream_t s) {
   const int n_in = transpose ? Cout : Cin, n_out = transpose ? Cin : Cout;
-  const int nch = (n_in + tc::KC - 1) / tc::KC;
-  if ((n_in % tc::KC) != 0) SCN_CUDA(cudaMemsetAsync(out, 0, scn_tc_image_bytes(K, n_in, n_out), s));
+  const int nch = tc_nch(n_in, tf32);
+  if (!tf32 && (n_in % tc::KC) != 0) SCN_CUDA(cudaMemsetAsync(out, 0, scn_tc_image_bytes(K, n_in, n_out, tf32), s));
   int64_t total = (int64_t)K * Cin * Cout;
   tc::k_prep_weights_tc<<<grid_for(total, 256), 256, 0, s>>>(W, K, Cin, Cout, transpose, mirror, nch,
-                                                             tc_pair(n_in) ? 1 : 0, (__nv_bfloat16*)out);
+                                                             tc_pair(n_in, tf32) ? 1 : 0, tf32, out);
   SCN_LAUNCH_CHECK();
   return SCN_OK;
 }
@@ -707,10 +752,11 @@ extern "C" void scn_tc_debug_last_launch(int32_t* out) {
   for (int i = 0; i < 9; ++i) out[i] = g_last_launch[i];
 }
 
-int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nbr, int K, int64_t n_rows,
-                   int64_t n_pad, int n_in, int n_out, const void* bimg, const float* bias, __nv_bfloat16* out,
-                   cudaStream_t s) {
-  if ((uint64_t)n_in_rows * (uint64_t)(n_in >> 3) >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;   // 32-bit offsets in 16-byte units (64 GB)
+// in / out: bf16, or fp32 with tf32 != 0 (TF32 MMAs)
+int scn_tc_forward(const void* in, int64_t n_in_rows, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int n_in,
+                   int n_out, const void* bimg, const float* bias, void* out, int tf32, cudaStream_t s) {
+  const uint64_t row_units = (uint64_t)n_in * (tf32 ? 4u : 2u) / 16u;                // 16-byte units per input row
+  if ((uint64_t)n_in_rows * row_units >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;   // 32-bit offsets in 16-byte units (64 GB)
   if (g_knob[0] < 0) {
     g_knob[0] = env_int("SCN_B200_TC_GRID"); g_knob[1] = env_int("SCN_B200_TC_T");
     g_knob[2] = env_int("SCN_B200_TC_SA"); g_knob[3] = env_int("SCN_B200_TC_SB");
@@ -725,8 +771,10 @@ int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nb
 #endif
   p.in = in; p.nbr = nbr; p.bimg = (const unsigned char*)bimg; p.bias = bias; p.out = out;
   p.n_rows = n_rows; p.n_pad = n_pad; p.K = K; p.n_in = n_in; p.n_out = n_out;
-  const int nch = (n_in + tc::KC - 1) / tc::KC;
-  p.last_kc = n_in - (nch - 1) * tc::KC;
+  const bool pair = tc_pair(n_in, tf32);
+  const int nch = tc_nch(n_in, tf32);
+  p.nch = nch;
+  p.last_kc = n_in - (nch - 1) * (tf32 ? tc::KC_TF32 : tc::KC);
   p.num_tiles = (int)((n_rows + tc::BM - 1) / tc::BM);
   // Tiles per group.  A group's T tiles are dealt to NM = 1, 2 or 4 classes (one issuing warp + producer group each) and
   // every class walks its tiles' stages as ONE serial chain (~1400 cycles per stage), so a CTA's time is, in units of
@@ -738,7 +786,7 @@ int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nb
   int max_ctas = kNumSMs;
   if (force_grid > 0 && force_grid < max_ctas) max_ctas = force_grid;
   const int per_cta = (p.num_tiles + max_ctas - 1) / max_ctas;
-  const int q_per_tile = (tc_pair(n_in) ? (K + 1) / 2 : K) * nch;
+  const int q_per_tile = (pair ? (K + 1) / 2 : K) * nch;
   int T = 1;
   p.nbuf = 2;
   {
@@ -770,13 +818,12 @@ int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nb
   // classes anyway (T == 2 or 3: the deep levels with one or two tiles per CTA) or one tile per CTA and room for a second
   // accumulator; SCN_B200_TC_KSPLIT=0 turns it off.
   p.ksplit = 0;
-  const int stages_per_tile = (tc_pair(n_in) ? (K + 1) / 2 : K) * nch;
+  const int stages_per_tile = (pair ? (K + 1) / 2 : K) * nch;
   if (g_ksplit_enabled() && stages_per_tile >= 2) {          // both accumulators must receive a first stage
     if (p.NM == 1 && per_cta == 1 && 2 * n_out <= 512) { p.NM = 2; p.nbuf = 1; p.ksplit = 1; }
     else if (p.NM == 2) p.ksplit = 1;
   }
   const uint32_t b_bytes = (uint32_t)n_out * 128u;
-  const bool pair = tc_pair(n_in);
   constexpr int NBAR = 2 * tc::MAX_A + 2 * tc::MAX_B + 4;
   const uint32_t fixed = 1024u + 8u * NBAR + 16u + (uint32_t)tc::MAX_A * tc::MASK_BYTES +
                          2u * (uint32_t)tc::PROD_WARPS * tc::LIST_BYTES + 16u;
@@ -809,6 +856,7 @@ int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nb
       SCN_CUDA(cudaFuncSetAttribute(tc::k_conv_tc<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       SCN_CUDA(cudaFuncSetAttribute(tc::k_conv_tc<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       SCN_CUDA(cudaFuncSetAttribute(tc::k_conv_tc<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      SCN_CUDA(cudaFuncSetAttribute(tc::k_conv_tc<0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
       attr_set = true;
     }
   }
@@ -823,6 +871,7 @@ int scn_tc_forward(const __nv_bfloat16* in, int64_t n_in_rows, const int32_t* nb
     SCN_LAUNCH_CHECK();
     return SCN_OK;
   };
+  if (tf32) return nch <= 8 ? launch(tc::k_conv_tc<0, false, true>) : SCN_ERR_UNSUPPORTED;
   if (pair) return launch(tc::k_conv_tc<1, true>);
   switch (nch) {
     case 1: return launch(tc::k_conv_tc<1, false>);

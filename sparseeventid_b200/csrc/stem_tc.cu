@@ -11,12 +11,15 @@
 //     wgrad:    dW[128 x 32]      += A^T[128 x 16 rows] . dout[16 rows x 32]
 // Precision: x and W are fp32 in HBM; each is split into bf16 hi + lo parts (x = hi + lo to 2^-17) and the products
 // hi.hi + lo.hi + hi.lo are accumulated in fp32, i.e. ~fp32 accuracy (the lo.lo term is below 2^-16 relative); dout is
-// bf16 already.  Used in the "bf16" / "mixed" precision modes; the "fp32" mode keeps the exact FFMA kernels.
+// bf16 already in the "bf16" mode.  In the "tf32" mode (fp32 features) the output is stored fp32 and the fp32 dout of
+// the weight gradient is split like x: hi.hi + lo.hi + hi.lo.  Used in the "bf16", "mixed" (bf16 outputs only) and
+// "tf32" precision modes; the "fp32" mode keeps the exact FFMA kernels.
 // HBM-bound by the table (4 K n bytes: 248 MB for the bench batch).
 //
 // Replaces SCN's Convolution forward / backward for the reference's initial_convolution
 // (src/networks/resnet.py:30-36: SubmanifoldConvolution(nIn=1, nOut=n_initial_filters, filter_size=5)).
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -41,13 +44,21 @@ __device__ __forceinline__ void split2(float v0, float v1, uint32_t& hi, uint32_
 }
 __device__ __forceinline__ float ldx(const float* x, int j) { return j >= 0 ? __ldg(x + j) : 0.f; }
 __device__ __forceinline__ float ldx(const __nv_bfloat16* x, int j) { return j >= 0 ? __bfloat162float(x[j]) : 0.f; }
+// two adjacent output values of a row: bf16x2 or float2
+__device__ __forceinline__ void st2(__nv_bfloat16* p, float a, float b) { *reinterpret_cast<uint32_t*>(p) = pack_bf16x2(a, b); }
+__device__ __forceinline__ void st2(float* p, float a, float b) { *reinterpret_cast<float2*>(p) = make_float2(a, b); }
+// one element of dout as the raw bf16 bits (bf16 dout) or as fp32
+__device__ __forceinline__ unsigned short ldd(const __nv_bfloat16* d, int64_t i) {
+  return reinterpret_cast<const unsigned short*>(d)[i];
+}
+__device__ __forceinline__ float ldd(const float* d, int64_t i) { return d[i]; }
 
 // Forward.  One warp per 16-row tile (grid-stride); thread (g = lane / 4, t = lane % 4) of the m16n8k16 layout holds
 // A[g | g + 8][2t, 2t + 1, 2t + 8, 2t + 9] of every 16-offset block: eight table entries, eight gathered scalars.
-template <typename TI>
+template <typename TI, typename TO>
 __global__ void __launch_bounds__(256) k_stem_fwd(const TI* __restrict__ x, const int32_t* __restrict__ nbr, int K, int64_t n_rows,
                                                   int64_t n_pad, const float* __restrict__ W, const float* __restrict__ bias,
-                                                  __nv_bfloat16* __restrict__ out) {
+                                                  TO* __restrict__ out) {
   __shared__ uint2 s_bhi[MAXKT * 4 * 32], s_blo[MAXKT * 4 * 32];     // B fragments of (offset block, 8-column block, lane)
   pdl_launch_dependents();
   pdl_wait();
@@ -112,8 +123,8 @@ __global__ void __launch_bounds__(256) k_stem_fwd(const TI* __restrict__ x, cons
 #pragma unroll
     for (int nt = 0; nt < 4; ++nt) {
       const int col = nt * 8 + 2 * t;
-      if (r0 + g < n_rows) *reinterpret_cast<uint32_t*>(out + (r0 + g) * NOUT + col) = pack_bf16x2(acc[nt][0], acc[nt][1]);
-      if (r0 + g + 8 < n_rows) *reinterpret_cast<uint32_t*>(out + (r0 + g + 8) * NOUT + col) = pack_bf16x2(acc[nt][2], acc[nt][3]);
+      if (r0 + g < n_rows) st2(out + (r0 + g) * NOUT + col, acc[nt][0], acc[nt][1]);
+      if (r0 + g + 8 < n_rows) st2(out + (r0 + g + 8) * NOUT + col, acc[nt][2], acc[nt][3]);
     }
   }
 }
@@ -124,9 +135,10 @@ __global__ void __launch_bounds__(256) k_stem_fwd(const TI* __restrict__ x, cons
 // operand is A^T[offset][row]: thread (g, t) needs x[nbr[k][r0 + 2t, 2t + 1 (+ 8)]] for k = g, g + 8 of each offset
 // block -- pairs of adjacent table entries, one 8-byte load each.  The B operand dout[row][channel] is read with the
 // fragment's own (strided, L1-resident) 2-byte accesses.  Blocks add their partial dW with fp32 atomics at the end
-// (one pass of 4 K values per block).
-template <typename TI>
-__global__ void __launch_bounds__(256, 2) k_stem_wgrad(const TI* __restrict__ x, const __nv_bfloat16* __restrict__ dout,
+// (one pass of 4 K values per block).  An fp32 dout (tf32 mode) is split into hi + lo fragments like x, and the products
+// hi.hi + lo.hi + hi.lo are accumulated.
+template <typename TI, typename TD>
+__global__ void __launch_bounds__(256, 2) k_stem_wgrad(const TI* __restrict__ x, const TD* __restrict__ dout,
                                                        const int32_t* __restrict__ nbr, int K, int64_t n_rows, int64_t n_pad,
                                                        float* __restrict__ dW) {
   __shared__ float s_part[4][2 * 4 * 4 * 32];              // the second row-tile stream's accumulators, per offset group
@@ -143,7 +155,7 @@ __global__ void __launch_bounds__(256, 2) k_stem_wgrad(const TI* __restrict__ x,
     for (int nt = 0; nt < 4; ++nt)
 #pragma unroll
       for (int e = 0; e < 4; ++e) acc[mt][nt][e] = 0.f;
-  const unsigned short* du = reinterpret_cast<const unsigned short*>(dout);
+  constexpr bool SPLIT_D = std::is_same<TD, float>::value;
   auto load_idx = [&](int64_t r0, int2* idx) {
 #pragma unroll
     for (int mt = 0; mt < 2; ++mt)
@@ -163,16 +175,24 @@ __global__ void __launch_bounds__(256, 2) k_stem_wgrad(const TI* __restrict__ x,
   for (; tile < tiles; tile += tstride) {
     const int64_t r0 = tile * 16;
     if (tile + tstride < tiles) load_idx((tile + tstride) * 16, nxt);
-    // B fragments: b0 = dout[r0 + 2t, 2t + 1][n], b1 = dout[r0 + 2t + 8, 2t + 9][n], n = 8 nt + g; rows past the end are zeros
-    uint32_t b[4][2];
+    // B fragments: b0 = dout[r0 + 2t, 2t + 1][n], b1 = dout[r0 + 2t + 8, 2t + 9][n], n = 8 nt + g; rows past the end are
+    // zeros.  bl: the lo parts of an fp32 dout.
+    uint32_t b[4][2], bl[4][2];
 #pragma unroll
     for (int nt = 0; nt < 4; ++nt)
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int64_t ra = r0 + 2 * t + 8 * h;
-        const unsigned short lo = ra < n_rows ? du[ra * NOUT + nt * 8 + g] : (unsigned short)0;
-        const unsigned short hi = ra + 1 < n_rows ? du[(ra + 1) * NOUT + nt * 8 + g] : (unsigned short)0;
-        b[nt][h] = (uint32_t)lo | ((uint32_t)hi << 16);
+        if constexpr (SPLIT_D) {
+          const float v0 = ra < n_rows ? ldd(dout, ra * NOUT + nt * 8 + g) : 0.f;
+          const float v1 = ra + 1 < n_rows ? ldd(dout, (ra + 1) * NOUT + nt * 8 + g) : 0.f;
+          split2(v0, v1, b[nt][h], bl[nt][h]);
+        } else {
+          const unsigned short lo = ra < n_rows ? ldd(dout, ra * NOUT + nt * 8 + g) : (unsigned short)0;
+          const unsigned short hi = ra + 1 < n_rows ? ldd(dout, (ra + 1) * NOUT + nt * 8 + g) : (unsigned short)0;
+          b[nt][h] = (uint32_t)lo | ((uint32_t)hi << 16);
+          bl[nt][h] = 0u;
+        }
       }
 #pragma unroll
     for (int mt = 0; mt < 2; ++mt) {
@@ -187,6 +207,7 @@ __global__ void __launch_bounds__(256, 2) k_stem_wgrad(const TI* __restrict__ x,
       for (int nt = 0; nt < 4; ++nt) {
         mma16816(acc[mt][nt], ahi, b[nt][0], b[nt][1]);
         mma16816(acc[mt][nt], alo, b[nt][0], b[nt][1]);
+        if constexpr (SPLIT_D) mma16816(acc[mt][nt], ahi, bl[nt][0], bl[nt][1]);
       }
     }
 #pragma unroll
@@ -230,40 +251,48 @@ bool scn_stem_tc_enabled() {
 
 bool scn_stem_tc_shape_ok(int K, int n_in, int n_out) { return n_in == 1 && n_out == stem::NOUT && K >= 1 && K <= 16 * stem::MAXKT; }
 
-// x: fp32 or bf16 [n_in_rows, 1]; W: fp32 [K][1][32]; out: bf16 [n_rows, 32]
+// x: fp32 or bf16 [n_in_rows, 1]; W: fp32 [K][1][32]; out: bf16 or fp32 [n_rows, 32]
 int scn_stem_tc_forward(const void* x, int x_dtype, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, const float* W,
-                        const float* bias, __nv_bfloat16* out, cudaStream_t s) {
+                        const float* bias, void* out, int out_dtype, cudaStream_t s) {
   const int64_t tiles = (n_rows + 15) / 16;
   int64_t g = (tiles + 7) / 8;
   if (g > (int64_t)kNumSMs * 3) g = (int64_t)kNumSMs * 3;
   if (g < 1) g = 1;
-  if (x_dtype == SCN_F32)
-    SCN_CUDA(scn_launch_pdl(stem::k_stem_fwd<float>, dim3((unsigned)g), dim3(256), 0, s, (const float*)x, nbr, K, n_rows, n_pad, W,
-                            bias, out));
-  else if (x_dtype == SCN_BF16)
-    SCN_CUDA(scn_launch_pdl(stem::k_stem_fwd<__nv_bfloat16>, dim3((unsigned)g), dim3(256), 0, s, (const __nv_bfloat16*)x, nbr, K,
-                            n_rows, n_pad, W, bias, out));
-  else
-    return SCN_ERR_ARG;
-  SCN_LAUNCH_CHECK();
-  return SCN_OK;
+  auto launch = [&](auto kern, auto xp, auto op) -> int {
+    SCN_CUDA(scn_launch_pdl(kern, dim3((unsigned)g), dim3(256), 0, s, xp, nbr, K, n_rows, n_pad, W, bias, op));
+    SCN_LAUNCH_CHECK();
+    return SCN_OK;
+  };
+  const float* xf = (const float*)x;
+  const __nv_bfloat16* xb = (const __nv_bfloat16*)x;
+  if (out_dtype == SCN_BF16) {
+    if (x_dtype == SCN_F32) return launch(stem::k_stem_fwd<float, __nv_bfloat16>, xf, (__nv_bfloat16*)out);
+    if (x_dtype == SCN_BF16) return launch(stem::k_stem_fwd<__nv_bfloat16, __nv_bfloat16>, xb, (__nv_bfloat16*)out);
+  } else if (out_dtype == SCN_F32) {
+    if (x_dtype == SCN_F32) return launch(stem::k_stem_fwd<float, float>, xf, (float*)out);
+  }
+  return SCN_ERR_ARG;
 }
 
-// dW: fp32 [K][1][32], accumulated into
-int scn_stem_tc_wgrad(const void* x, int x_dtype, const __nv_bfloat16* dout, const int32_t* nbr, int K, int64_t n_rows,
+// dW: fp32 [K][1][32], accumulated into; dout: bf16, or fp32 with fp32 x
+int scn_stem_tc_wgrad(const void* x, int x_dtype, const void* dout, int dout_dtype, const int32_t* nbr, int K, int64_t n_rows,
                       int64_t n_pad, float* dW, cudaStream_t s) {
   const int64_t tiles = (n_rows + 15) / 16;
   int64_t g = (tiles + 1) / 2;
   if (g > (int64_t)kNumSMs * 2) g = (int64_t)kNumSMs * 2;
   if (g < 1) g = 1;
-  if (x_dtype == SCN_F32)
-    SCN_CUDA(scn_launch_pdl(stem::k_stem_wgrad<float>, dim3((unsigned)g), dim3(256), 0, s, (const float*)x, dout, nbr, K, n_rows,
-                            n_pad, dW));
-  else if (x_dtype == SCN_BF16)
-    SCN_CUDA(scn_launch_pdl(stem::k_stem_wgrad<__nv_bfloat16>, dim3((unsigned)g), dim3(256), 0, s, (const __nv_bfloat16*)x, dout, nbr,
-                            K, n_rows, n_pad, dW));
-  else
-    return SCN_ERR_ARG;
-  SCN_LAUNCH_CHECK();
-  return SCN_OK;
+  auto launch = [&](auto kern, auto xp, auto dp) -> int {
+    SCN_CUDA(scn_launch_pdl(kern, dim3((unsigned)g), dim3(256), 0, s, xp, dp, nbr, K, n_rows, n_pad, dW));
+    SCN_LAUNCH_CHECK();
+    return SCN_OK;
+  };
+  const float* xf = (const float*)x;
+  const __nv_bfloat16* db = (const __nv_bfloat16*)dout;
+  if (dout_dtype == SCN_BF16) {
+    if (x_dtype == SCN_F32) return launch(stem::k_stem_wgrad<float, __nv_bfloat16>, xf, db);
+    if (x_dtype == SCN_BF16) return launch(stem::k_stem_wgrad<__nv_bfloat16, __nv_bfloat16>, (const __nv_bfloat16*)x, db);
+  } else if (dout_dtype == SCN_F32) {
+    if (x_dtype == SCN_F32) return launch(stem::k_stem_wgrad<float, float>, xf, (const float*)dout);
+  }
+  return SCN_ERR_ARG;
 }

@@ -137,14 +137,30 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
 
 // tcgen05.mma with a disable-output-lane mask: bit r of {m0..m3} set => TMEM lane (= output row) r is NOT updated, so the
 // A-tile row r may hold anything (stale shared memory): rows without a neighbour at this offset are never gathered.
+// TF32: the kind::tf32 form (fp32 bits in shared memory, 10-bit mantissa operands, K = 8 per instruction).
+template <bool TF32 = false>
 __device__ __forceinline__ void umma_masked(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate,
                                             uint32_t m0, uint32_t m1, uint32_t m2, uint32_t m3) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %6, %7, %8}, p;\n\t}"
-      ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate), "r"(m0), "r"(m1), "r"(m2), "r"(m3)
-      : "memory");
+  if constexpr (TF32)
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, {%5, %6, %7, %8}, p;\n\t}"
+        ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate), "r"(m0), "r"(m1), "r"(m2), "r"(m3)
+        : "memory");
+  else
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %6, %7, %8}, p;\n\t}"
+        ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate), "r"(m0), "r"(m1), "r"(m2), "r"(m3)
+        : "memory");
+}
+// fp32 -> TF32 bits, rounded to nearest (ties away from zero); the low 13 bits of the result are zero
+__device__ __forceinline__ float to_tf32_rna(float v) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));
+  return __uint_as_float(r);
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");

@@ -1,5 +1,5 @@
 // Weight gradient of the sparse convolutions on 5th-generation tensor cores (sm_100a only):
-//     dW[k] (+)= sum over pairs (i, o) of rules[k]   x[i, :]^T . dout[o, :]          (bf16 operands, fp32 accumulate)
+//     dW[k] (+)= sum over pairs (i, o) of rules[k]   x[i, :]^T . dout[o, :]          (bf16 or TF32 operands, fp32 accumulate)
 //
 // The contraction index is the PAIR, so -- unlike the forward, where missing neighbours are masked output rows -- the
 // live pairs of an offset can be compacted freely: a stage is 64 compacted pairs, its A operand the 64 gathered x rows
@@ -14,6 +14,13 @@
 // to a ring and emits a stage whenever 64 are pending; LDGSTS copies that signal their own landing), one issuing warp
 // that consumes the producers' stages in a fixed round-robin order (so dW is bitwise reproducible), 4 epilogue warps
 // (tcgen05.ld -> red.global.add.f32).
+//
+// TF32 instantiation (precision SCN_PREC_TF32, fp32 x and dout): a stage row is 128 bytes = 32 fp32 channels, so blocks
+// are 32 channels wide (nca, ncb up to 8: runtime counts, one instantiation per pairs-per-stage) and one
+// tcgen05.mma (kind::tf32) contracts K = 8 pairs.  MN-major TF32 operands must use the 128-byte swizzle with 32-byte
+// atomicity (SWIZZLE_128B_BASE32B, descriptor layout type 1; CUTLASS cute/arch/mma_sm100_desc.hpp and
+// Layout_MN_SW128_32B_Atom = Swizzle<2,5,2>): the 32-byte granule g of row r sits at g ^ (r & 3), 4-row atoms of
+// 512 bytes (SBO), instead of the 16-byte chunk c at c ^ (r & 7) in 8-row atoms of 1024 bytes.
 //
 // Replaces SCN's dConvolution_KMxKN_backward_dW_A/B (SURVEY.md 2.2); reference call sites
 // src/networks/sparse_building_blocks.py:29-34,110-117 (backward).
@@ -36,41 +43,54 @@ constexpr int MAX_SLOTS = 2 * PROD_WARPS;
 constexpr int RING = 256;                 // pending-pair ring per producer warp (entries), a power of two
 
 struct Params {
-  const __nv_bfloat16* x;       // [n_in_rows, Cin]
-  const __nv_bfloat16* dout;    // [n_rows, Cout]
+  const void* x;                // [n_in_rows, Cin] bf16 (fp32 for the TF32 instantiation)
+  const void* dout;             // [n_rows, Cout], the element type of x
   const int32_t* nbr;           // [K][n_pad]: input row of output row o at offset k, or -1
   float* dW;                    // [K][Cin][Cout], accumulated into (by k_wgrad_reduce, or by atomics when part == nullptr)
   float* part;                  // [gridDim.x][Cin][Cout] partial sums, one slab per CTA, or nullptr
   int64_t n_rows, n_pad;
   int K, Cin, Cout;
-  int nca, ncb;                 // 64-channel blocks per stage: A (even: M = 128 reads two), B
+  int nca, ncb;                 // channel blocks (128-byte rows: 64 bf16 / 32 fp32 channels) per stage: A, B
   int nmb;                      // M blocks of 128 input channels
   int slots, npw;               // stage slots, active producer warps (slots == 2 * npw)
   int s_other, s_centre, centre;   // CTAs per ordinary offset / for the centre offset (or -1)
 };
 
-// MN-major SWIZZLE_128B descriptor: rows of 128 bytes (64 elements along M/N), 8 K-rows per 1024-byte atom (SBO),
-// `lbo` bytes between consecutive 64-element blocks along M/N.
+// MN-major 128-byte-swizzled descriptor: rows of 128 bytes along M/N, `lbo` bytes between consecutive 128-byte blocks
+// along M/N.  bf16: SWIZZLE_128B, 8 K-rows per 1024-byte atom (SBO); TF32: SWIZZLE_128B_BASE32B, 4 K-rows per 512-byte
+// atom.
+template <bool TF32>
 __device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t saddr, uint32_t lbo_bytes) {
   uint64_t d = 0;
   d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
   d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
+  d |= (uint64_t)((TF32 ? 512 : 1024) >> 4) << 32;
   d |= (uint64_t)1 << 46;       // descriptor version 1 (sm_100)
-  d |= (uint64_t)2 << 61;       // LayoutType::SWIZZLE_128B
+  d |= (uint64_t)(TF32 ? 1 : 2) << 61;   // LayoutType::SWIZZLE_128B_BASE32B / SWIZZLE_128B
   return d;
 }
-// kind::f16, bf16 x bf16 -> fp32, A and B MN-major, M = 128, N = n
+// fp32 accumulate, A and B MN-major, M = 128, N = n; bf16 (kind::f16) or TF32 (kind::tf32) operands
+template <bool TF32>
 __device__ __forceinline__ uint32_t make_idesc_mn(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(n >> 3) << 17) | (8u << 24);
+  constexpr uint32_t fmt = TF32 ? 2u : 1u;
+  return (1u << 4) | (fmt << 7) | (fmt << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(n >> 3) << 17) | (8u << 24);
 }
+template <bool TF32>
 __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
-      : "memory");
+  if constexpr (TF32)
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
+        : "memory");
+  else
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
+        : "memory");
 }
 
 // NA / NB: 64-channel blocks of a stage's A (x rows) / B (dout rows) operand = ceil(Cin / 64), ceil(Cout / 64)
@@ -78,16 +98,21 @@ __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, 
 // PAIRS: pairs (MMA K rows) per stage: 64, or 32 for the wide layers (NA + NB >= 5: a 64-pair stage is 40-48 KB, only 4
 // slots = 2 producer warps fit; measured 78 us for 258 k pairs at 160 channels against 73 us for 805 k pairs at 128).
 // (Two-warp producer teams per stage were measured too and are slower: 117 -> 168 us at 96 channels.)
-template <int NA, int NB, bool HALF, int PAIRS>
+// TF32: NA == NB == 0, the block counts (1..8 each) are p.nca / p.ncb; PAIRS 64, 32 or 16 (see scn_wgrad_tc).
+template <int NA, int NB, bool HALF, int PAIRS, bool TF32 = false>
 __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
-  constexpr int BLK_BYTES = PAIRS * 128;                 // one 64-channel block of a stage: PAIRS rows x 128 B
+  static_assert(TF32 == (NA == 0 && NB == 0), "TF32 takes its block counts at run time");
+  static_assert(!(TF32 && HALF), "fp32 rows of 32 channels are whole 128-byte rows");
+  constexpr int NAM = TF32 ? 8 : NA, NBM = TF32 ? 8 : NB;   // bounds of the (unrolled) block loops
+  const int na = TF32 ? p.nca : NA, nb = TF32 ? p.ncb : NB;
+  constexpr int BLK_BYTES = PAIRS * 128;                 // one channel block of a stage: PAIRS rows x 128 B
   extern __shared__ unsigned char smem_raw[];
   pdl_launch_dependents();                               // see common.cuh: programmatic dependent launch
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
   unsigned char* gbase = smem_raw + (base - raw);
   const int slots = p.slots, NPW = p.npw;
-  constexpr uint32_t slot_bytes = (uint32_t)(NA + NB) * BLK_BYTES;
+  const uint32_t slot_bytes = (uint32_t)(na + nb) * BLK_BYTES;
   const uint32_t bar0 = base + (uint32_t)slots * slot_bytes;
   auto afull = [&](int s) { return bar0 + 8u * (uint32_t)s; };
   auto aempty = [&](int s) { return bar0 + 8u * (uint32_t)(MAX_SLOTS + s); };
@@ -139,7 +164,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
     const int pw = warp - EPI_WARPS;
     if (pw < NPW) {
       int2* ring = rings + pw * RING;                       // .x: x row offset / 16 B, .y: dout row offset / 16 B
-      const uint32_t xvec = (uint32_t)p.Cin >> 3, dvec = (uint32_t)p.Cout >> 3;
+      const uint32_t xvec = (uint32_t)p.Cin >> (TF32 ? 2 : 3), dvec = (uint32_t)p.Cout >> (TF32 ? 2 : 3);
       const uint32_t lt = (1u << lane) - 1u;
       constexpr int LPR = HALF ? 4 : 8;                     // lanes per row
       constexpr int RPP = 32 / LPR;                         // rows per pass
@@ -149,12 +174,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
       const unsigned char* db = reinterpret_cast<const unsigned char*>(p.dout);
       int head = 0, pending = 0, emitted = 0;
 
-      // per-lane invariants of the copies: this lane moves 16-byte chunk `chunk` of every 64-channel block
-      bool a_ok[NA], b_ok[NB];
+      // per-lane invariants of the copies: this lane moves 16-byte chunk `chunk` of every channel block (TF32: the
+      // channel counts are multiples of 32, every block is a whole row)
+      bool a_ok[NAM], b_ok[NBM];
 #pragma unroll
-      for (int b = 0; b < NA; ++b) a_ok[b] = b * 64 + chunk * 8 < p.Cin;
+      for (int b = 0; b < NAM; ++b) a_ok[b] = TF32 || b * 64 + chunk * 8 < p.Cin;
 #pragma unroll
-      for (int b = 0; b < NB; ++b) b_ok[b] = b * 64 + chunk * 8 < p.Cout;
+      for (int b = 0; b < NBM; ++b) b_ok[b] = TF32 || b * 64 + chunk * 8 < p.Cout;
       const unsigned char* xsrc = xb + ((uint32_t)chunk << 4);
       const unsigned char* dsrc = db + ((uint32_t)chunk << 4);
 
@@ -169,18 +195,23 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
           const int row = pass * RPP + sub;                  // stage row (pair), LPR lanes per row
           const bool live = row < take;
           const int2 e = live ? ring[(head + row) & (RING - 1)] : make_int2(0, 0);
-          const uint32_t dst = (sbase + (uint32_t)row * 128u + ((uint32_t)(row & 7) << 4)) ^ csw;
+          // SWIZZLE_128B: 16-byte chunk c at c ^ (row & 7); TF32 (SWIZZLE_128B_BASE32B): 32-byte granule c / 2 at
+          // (c / 2) ^ (row & 3)
+          const uint32_t rsw = TF32 ? ((uint32_t)(row & 3) << 5) : ((uint32_t)(row & 7) << 4);
+          const uint32_t dst = (sbase + (uint32_t)row * 128u + rsw) ^ csw;
           const unsigned char* xs = xsrc + ((uint64_t)(uint32_t)e.x << 4);
           const unsigned char* ds = dsrc + ((uint64_t)(uint32_t)e.y << 4);
 #pragma unroll
-          for (int b = 0; b < NA; ++b) {                     // x row -> A blocks
+          for (int b = 0; b < NAM; ++b) {                    // x row -> A blocks
+            if (TF32 && b >= na) break;
             const bool ok = live && a_ok[b];
             cp_async16(dst + (uint32_t)b * BLK_BYTES, ok ? xs + b * 128 : xs, ok ? 16u : 0u);
           }
 #pragma unroll
-          for (int b = 0; b < NB; ++b) {                     // dout row -> B blocks
+          for (int b = 0; b < NBM; ++b) {                    // dout row -> B blocks
+            if (TF32 && b >= nb) break;
             const bool ok = live && b_ok[b];
-            cp_async16(dst + (uint32_t)(NA + b) * BLK_BYTES, ok ? ds + b * 128 : ds, ok ? 16u : 0u);
+            cp_async16(dst + (uint32_t)(na + b) * BLK_BYTES, ok ? ds + b * 128 : ds, ok ? 16u : 0u);
           }
         }
         cp_async_arrive_noinc(afull(slot));
@@ -225,7 +256,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
     }
   } else if (warp == WARP_MMA) {
     // ================================ MMA issuer ============================================
-    const uint32_t idesc = make_idesc_mn(p.Cout);
+    const uint32_t idesc = make_idesc_mn<TF32>(p.Cout);
     const uint32_t a_lbo = BLK_BYTES, b_lbo = BLK_BYTES;
     int consumed[PROD_WARPS];
 #pragma unroll
@@ -257,17 +288,22 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
         tc_fence_after();
         const uint32_t sbase = base + (uint32_t)slot * slot_bytes;
         if (elect_one()) {
+          // M = 128 reads BPM blocks (two of 64 bf16 / four of 32 fp32 channels); a single last block is read BPM times
+          // (LBO = 0), a last M block of 2 or 3 TF32 blocks reads on into the following blocks: accumulator rows beyond
+          // Cin are never looked at by the epilogue
+          constexpr int BPM = TF32 ? 4 : 2;
+          constexpr int KPM = TF32 ? 8 : 16;                 // pairs (K rows) per MMA: 32 bytes of K
 #pragma unroll
-          for (int mb = 0; mb < (NA + 1) / 2; ++mb) {
+          for (int mb = 0; mb < (NAM + BPM - 1) / BPM; ++mb) {
+            if (TF32 && mb * BPM >= na) break;
             const uint32_t tmem_d = tmem_base + (uint32_t)(mb * p.Cout);
-            // M = 128 reads two 64-channel blocks; an odd last block is read twice (LBO = 0): accumulator rows
-            // 64..127 of that M block are then copies the epilogue never looks at
-            const uint32_t lbo = (2 * mb + 1 < NA) ? a_lbo : 0u;
+            const uint32_t lbo = (BPM * mb + 1 < na) ? a_lbo : 0u;
 #pragma unroll
-            for (int kk = 0; kk < PAIRS / 16; ++kk) {
-              const uint64_t da = make_desc_mn_sw128(sbase + (uint32_t)(2 * mb) * BLK_BYTES + (uint32_t)kk * 2048u, lbo);
-              const uint64_t db = make_desc_mn_sw128(sbase + (uint32_t)NA * BLK_BYTES + (uint32_t)kk * 2048u, b_lbo);
-              umma(tmem_d, da, db, idesc, (first && kk == 0) ? 0u : 1u);
+            for (int kk = 0; kk < PAIRS / KPM; ++kk) {
+              const uint32_t koff = (uint32_t)kk * (uint32_t)(KPM * 128);
+              const uint64_t da = make_desc_mn_sw128<TF32>(sbase + (uint32_t)(BPM * mb) * BLK_BYTES + koff, lbo);
+              const uint64_t db = make_desc_mn_sw128<TF32>(sbase + (uint32_t)na * BLK_BYTES + koff, b_lbo);
+              umma<TF32>(tmem_d, da, db, idesc, (first && kk == 0) ? 0u : 1u);
             }
           }
           umma_commit(aempty(slot));
@@ -292,7 +328,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
     // The CTA's Cin x Cout partial sum goes to its own slab with plain 16-byte stores; k_wgrad_reduce then adds the slabs of
     // an offset in a fixed order (deterministic).  Atomics straight into dW were ~44% of the kernel's time on the
     // deep levels (148-296 CTAs x 25-37 k red.global.add each; ncu: the other warps idle at the exit barrier meanwhile).
-    for (int mb = 0; mb < (NA + 1) / 2; ++mb) {
+    for (int mb = 0; mb < (TF32 ? p.nmb : (NA + 1) / 2); ++mb) {
       const int cin = mb * 128 + warp * 32 + lane;                            // accumulator row == input channel
       const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(mb * p.Cout);
       for (int c0 = 0; c0 < p.Cout; c0 += 32) {
@@ -406,20 +442,25 @@ bool scn_wgrad_tc_enabled() {
   return v == 1;
 }
 
-// dW[K][Cin][Cout] += ...; x, dout bf16.  Returns SCN_ERR_UNSUPPORTED for shapes outside the kernel (caller falls back).
-// Gathered rows are addressed through 32-bit offsets in 16-byte units: x and dout up to 64 GB each.
-int scn_wgrad_tc(const __nv_bfloat16* x, const __nv_bfloat16* dout, const int32_t* nbr, int K, int64_t n_rows,
-                 int64_t n_pad, int Cin, int Cout, float* dW, cudaStream_t s) {
+// dW[K][Cin][Cout] += ...; x, dout bf16, or fp32 with tf32 != 0 (TF32 MMAs).  Returns SCN_ERR_UNSUPPORTED for shapes
+// outside the kernel (caller falls back).  Gathered rows are addressed through 32-bit offsets in 16-byte units: x and
+// dout up to 64 GB each.
+int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int Cin, int Cout,
+                 int tf32, float* dW, cudaStream_t s) {
   if ((Cin % 32) || (Cout % 32) || Cin < 32 || Cout < 32 || Cin > 256 || Cout > 256 || K < 1) return SCN_ERR_UNSUPPORTED;
-  if ((uint64_t)n_rows * (uint64_t)(Cout >> 3) >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;
+  if ((uint64_t)n_rows * (uint64_t)(Cout * (tf32 ? 4 : 2) / 16) >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;
   if (n_pad < ((n_rows + 127) / 128) * 128) return SCN_ERR_ARG;      // whole 128-row blocks are read
   wg::Params p;
   p.x = x; p.dout = dout; p.nbr = nbr; p.dW = dW; p.n_rows = n_rows; p.n_pad = n_pad; p.K = K; p.Cin = Cin; p.Cout = Cout;
   p.nmb = (Cin + 127) / 128;
-  p.nca = (Cin + 63) / 64;
-  p.ncb = (Cout + 63) / 64;
+  const int blk = tf32 ? 32 : 64;                            // channels per 128-byte block
+  p.nca = (Cin + blk - 1) / blk;
+  p.ncb = (Cout + blk - 1) / blk;
   if (p.nmb * Cout > 512) return SCN_ERR_UNSUPPORTED;
-  const int pairs = (p.nca + p.ncb) >= 5 ? 32 : 64;          // pairs per stage (see the kernel)
+  // pairs per stage (see the kernel).  TF32 blocks hold half the channels of bf16 ones: the same thresholds in bytes per
+  // pair, and one more halving for the widest layers (a 32-pair stage of 256 x 256 fp32 is 64 KB: 2 slots only)
+  const int nbl = p.nca + p.ncb;
+  const int pairs = tf32 ? (nbl >= 10 ? 16 : (nbl >= 5 ? 32 : 64)) : (nbl >= 5 ? 32 : 64);
   const uint32_t slot_bytes = (uint32_t)(p.nca + p.ncb) * (uint32_t)pairs * 128u;
   const uint32_t fixed = 1024u + 8u * (2 * wg::MAX_SLOTS + 2) + 16u + 4u * wg::MAX_SLOTS + 4u * wg::PROD_WARPS + 8u +
                          (uint32_t)wg::PROD_WARPS * wg::RING * 8u;
@@ -486,6 +527,11 @@ int scn_wgrad_tc(const __nv_bfloat16* x, const __nv_bfloat16* dout, const int32_
     }
     return SCN_OK;
   };
+  if (tf32) {
+    if (pairs == 64) return launch(wg::k_wgrad_tc<0, 0, false, 64, true>);
+    if (pairs == 32) return launch(wg::k_wgrad_tc<0, 0, false, 32, true>);
+    return launch(wg::k_wgrad_tc<0, 0, false, 16, true>);
+  }
   if (Cin == 32 && Cout == 32) return launch(wg::k_wgrad_tc<1, 1, true, 64>);
 #define WG_CASE(a, b) if (p.nca == a && p.ncb == b) return launch(wg::k_wgrad_tc<a, b, false, ((a) + (b) >= 5 ? 32 : 64)>)
   WG_CASE(1, 1); WG_CASE(1, 2); WG_CASE(1, 3); WG_CASE(1, 4);

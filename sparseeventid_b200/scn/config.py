@@ -8,6 +8,11 @@ what bench.py and BASELINE.json config 3 ("bf16 tensor-core convs") select.
   "fp32"  : fp32 features, exact fp32 FMA convolutions (parity mode; SCN itself is fp32,
             SURVEY.md App. C).
   "mixed" : fp32 features in HBM, bf16 tensor-core operands, fp32 accumulate.
+  "tf32"  : fp32 features in HBM, TF32 operands (10-bit mantissa) on the tcgen05 tensor cores, fp32
+            accumulate -- what PyTorch's dense fp32 convolutions use by default (cudnn.allow_tf32).
+            Shapes outside the tcgen05 kernels keep the exact fp32 kernels; the one-channel stem runs
+            its ~fp32-accurate hi/lo bf16 split.  BatchNorm, elementwise layers, parameters and
+            gradients are exactly as in "fp32".
   "bf16"  : bf16 features in HBM, bf16 tensor-core operands, fp32 accumulate; BatchNorm
             statistics, parameters and parameter gradients stay fp32 (BASELINE.json config 3).
 """
@@ -17,9 +22,9 @@ import os
 
 import torch
 
-from .._lib import PREC_BF16, PREC_FP32
+from .._lib import PREC_BF16, PREC_FP32, PREC_TF32
 
-_MODES = ("fp32", "mixed", "bf16")
+_MODES = ("fp32", "mixed", "tf32", "bf16")
 _state = {"mode": os.environ.get("SCN_B200_PRECISION", "fp32"),
           "fusion": os.environ.get("SCN_B200_FUSION", "1") not in ("0", "false", "False")}
 if _state["mode"] not in _MODES:
@@ -41,7 +46,7 @@ def feature_dtype() -> torch.dtype:
 
 
 def precision_code() -> int:
-    return PREC_FP32 if _state["mode"] == "fp32" else PREC_BF16
+    return {"fp32": PREC_FP32, "tf32": PREC_TF32}.get(_state["mode"], PREC_BF16)
 
 
 def set_fusion(flag: bool) -> None:

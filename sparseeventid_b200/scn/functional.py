@@ -98,9 +98,9 @@ def prepare_weight_images(modules) -> int:
             if ws.path != 2 or ops.conv_path(K, cout, cin, prec, fdt) != 2:
                 continue
             bwd = ws.bwd_buffer(K, cin, cout, prec, fdt, w.device)
-            rows.append([w.data_ptr(), ws.fwd.data_ptr(), K, cin, cout, 0, first, 0])
+            rows.append([w.data_ptr(), ws.fwd.data_ptr(), K, cin, cout, 0, first, prec])
             first += K * cin * cout
-            rows.append([w.data_ptr(), bwd.data_ptr(), K, cin, cout, 1 | (2 if m.mirror_dgrad else 0), first, 0])
+            rows.append([w.data_ptr(), bwd.data_ptr(), K, cin, cout, 1 | (2 if m.mirror_dgrad else 0), first, prec])
             first += K * cin * cout
             wss.append(ws)
         plan = _ImagePlan()
