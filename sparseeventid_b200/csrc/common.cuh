@@ -29,19 +29,10 @@ extern unsigned long long g_scn_launch_count;
 // -- all prerequisite grids complete and their memory visible -- BEFORE its first access to global memory that a
 // preceding kernel may have written or may still read, so results do not change.  A dependent grid is only launched
 // once every CTA of its primary has started, so a waiting CTA never starves the grid it waits for.  The instructions
-// are no-ops for a kernel launched the ordinary way.  SCN_B200_PDL=0 turns the attribute off.
-#include <cstdlib>
+// are no-ops for a kernel launched the ordinary way.
 #include <utility>
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-inline bool scn_pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = std::getenv("SCN_B200_PDL");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
 template <typename... KArgs, typename... Args>
 inline cudaError_t scn_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -51,7 +42,7 @@ inline cudaError_t scn_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block,
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = scn_pdl_enabled() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);

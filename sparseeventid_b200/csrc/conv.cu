@@ -1,19 +1,17 @@
 // Convolution arithmetic, first generation: output-stationary gather-GEMM on the neighbour table.
 //   * exact fp32 FMA kernels (precision SCN_PREC_FP32, odd channel counts, and the Cin=1 stem in that mode)
-//   * bf16-operand / fp32-accumulate tensor-core kernels built on mma.sync (HMMA) -- the
-//     baseline that conv_tc.cu (tcgen05 + TMEM) supersedes for the hot layer shapes.
+//   * bf16-operand / fp32-accumulate tensor-core kernels built on mma.sync (HMMA): the fp32 features of the "mixed"
+//     mode, and the bf16 weight gradient where the tcgen05 kernel (wgrad_tc.cu) does not apply (the bf16
+//     forward and dgrad at these shapes run on tcgen05 + TMEM, conv_tc.cu).
 // Replaces SCN's Convolution.cu dConvolution_KMxKN_forward/backward_dW (SURVEY.md 2.2; reference
 // call sites src/networks/sparse_building_blocks.py:29-34,110-117,207-213).
 #include "common.cuh"
 
 // conv_tc.cu (tcgen05 path)
-bool scn_tc_disabled();
 bool scn_tc_shape_ok(int K, int n_in, int n_out);
 size_t scn_tc_image_bytes(int K, int n_in, int n_out, int tf32);
 int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mirror, int tf32, void* out, cudaStream_t s);
-bool scn_wgrad_tc_enabled();
-bool scn_stem_tc_enabled();                       // stem_tc.cu
-bool scn_stem_tc_shape_ok(int K, int n_in, int n_out);
+bool scn_stem_tc_shape_ok(int K, int n_in, int n_out);   // stem_tc.cu
 int scn_stem_tc_forward(const void* x, int x_dtype, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, const float* W,
                         const float* bias, void* out, int out_dtype, cudaStream_t s);
 int scn_stem_tc_wgrad(const void* x, int x_dtype, const void* dout, int dout_dtype, const int32_t* nbr, int K, int64_t n_rows,
@@ -535,7 +533,7 @@ int wgrad_generic_t(const TI* in, const TO* dout, const int32_t* nbr, int K, int
 static int conv_path(int K, int n_in, int n_out, int precision, int feat_dtype) {
   const bool tc_mode = (precision == SCN_PREC_BF16 && feat_dtype == SCN_BF16) ||
                        (precision == SCN_PREC_TF32 && feat_dtype == SCN_F32);
-  if (tc_mode && !scn_tc_disabled() && scn_tc_shape_ok(K, n_in, n_out)) return 2;
+  if (tc_mode && scn_tc_shape_ok(K, n_in, n_out)) return 2;
   return mma_ok(K, n_in, n_out, precision) ? 1 : 0;
 }
 // the tcgen05 path of a precision runs its TF32 instantiation
@@ -580,19 +578,17 @@ extern "C" int scn_conv_forward(const void* in, int in_dtype, int64_t n_in_rows,
   if (in_dtype == out_dtype && conv_path(K, n_in, n_out, precision, in_dtype) == 2)
     return scn_tc_forward(in, n_in_rows, nbr, K, n_out_rows, n_pad, n_in, n_out, Bprep, bias, out, tc_tf32(precision), s);
   if (mma_ok(K, n_in, n_out, precision) && in_dtype == out_dtype) {
+    // fp32 features of the "mixed" mode (bf16 features at these shapes took the tcgen05 path above)
     if (in_dtype == SCN_F32)
       return conv_mma_t<float>((const float*)in, nbr, K, n_out_rows, n_pad, n_in, n_out, (const __nv_bfloat16*)Bprep,
                                bias, (float*)out, s);
-    if (in_dtype == SCN_BF16)
-      return conv_mma_t<__nv_bfloat16>((const __nv_bfloat16*)in, nbr, K, n_out_rows, n_pad, n_in, n_out,
-                                       (const __nv_bfloat16*)Bprep, bias, (__nv_bfloat16*)out, s);
     return SCN_ERR_ARG;
   }
   if (mma_ok(K, n_in, n_out, precision)) return SCN_ERR_UNSUPPORTED;   // Bprep is bf16 for this shape
   const float* B = (const float*)Bprep;
   // the stem (one input channel) as a dense GEMM over the neighbour table on tensor cores (stem_tc.cu): bf16 outputs,
   // and fp32 outputs in the tf32 mode; the exact fp32 mode keeps the FFMA kernel
-  if (precision != SCN_PREC_FP32 && (out_dtype == SCN_BF16 || precision == SCN_PREC_TF32) && scn_stem_tc_enabled() &&
+  if (precision != SCN_PREC_FP32 && (out_dtype == SCN_BF16 || precision == SCN_PREC_TF32) &&
       scn_stem_tc_shape_ok(K, n_in, n_out))
     return scn_stem_tc_forward(in, in_dtype, nbr, K, n_out_rows, n_pad, B, bias, out, out_dtype, s);
   if (in_dtype == SCN_F32 && out_dtype == SCN_F32)
@@ -618,7 +614,7 @@ extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, in
   if (precision == SCN_PREC_FP32 && (in_dtype != SCN_F32 || dout_dtype != SCN_F32)) return SCN_ERR_ARG;
   const bool tc_bf16 = precision == SCN_PREC_BF16 && in_dtype == SCN_BF16 && dout_dtype == SCN_BF16;
   const bool tc_tf = precision == SCN_PREC_TF32 && in_dtype == SCN_F32 && dout_dtype == SCN_F32;
-  if ((tc_bf16 || tc_tf) && !scn_tc_disabled() && scn_wgrad_tc_enabled() && (n_pad & 127) == 0) {
+  if ((tc_bf16 || tc_tf) && (n_pad & 127) == 0) {
     // tcgen05 path.  The number of rows of `in` is not part of this entry point's signature; the kernel addresses
     // gathered rows through 32-bit offsets in 16-byte units, i.e. feature matrices up to 64 GB.
     int rc = scn_wgrad_tc(in, dout, nbr, K, n_rows, n_pad, n_in, n_out, tc_tf ? 1 : 0, dW, s);
@@ -627,7 +623,7 @@ extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, in
   // the stem (one input channel): dense GEMM over the neighbour table on tensor cores (stem_tc.cu); bf16 dout, and fp32
   // dout in the tf32 mode
   if (precision != SCN_PREC_FP32 && (dout_dtype == SCN_BF16 || precision == SCN_PREC_TF32) && (n_pad & 127) == 0 &&
-      scn_stem_tc_enabled() && scn_stem_tc_shape_ok(K, n_in, n_out))
+      scn_stem_tc_shape_ok(K, n_in, n_out))
     return scn_stem_tc_wgrad(in, in_dtype, dout, dout_dtype, nbr, K, n_rows, n_pad, dW, s);
   if (mma_ok(K, n_in, n_out, precision) && in_dtype == dout_dtype) {
     if (in_dtype == SCN_F32)

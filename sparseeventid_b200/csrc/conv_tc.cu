@@ -689,15 +689,6 @@ extern "C" void scn_tc_debug_exp(int flags) { g_tc_exp = flags; }
 extern "C" void scn_tc_debug_exp(int) {}
 #endif
 
-bool scn_tc_disabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = std::getenv("SCN_B200_DISABLE_TC");
-    v = (e && e[0] && e[0] != '0') ? 1 : 0;
-  }
-  return v == 1;
-}
-
 bool scn_tc_shape_ok(int K, int n_in, int n_out) {
   return K >= 1 && (n_in % 32) == 0 && (n_out % 32) == 0 && n_in >= 32 && n_in <= 256 && n_out >= 32 && n_out <= 256;
 }
@@ -731,14 +722,6 @@ int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mir
 static int env_int(const char* name) {
   const char* e = std::getenv(name);
   return e ? std::atoi(e) : 0;
-}
-static bool g_ksplit_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = std::getenv("SCN_B200_TC_KSPLIT");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
 }
 static int g_knob[4] = {-1, -1, -1, -1};      // grid, T, SA, SB: -1 = read the environment on first use
 // developer entry for the sweep tools (like scn_tc_debug_timeline: not part of the product ABI): 0 = automatic
@@ -816,10 +799,10 @@ int scn_tc_forward(const void* in, int64_t n_in_rows, const int32_t* nbr, int K,
   p.NM = T >= 4 ? 4 : (T >= 2 ? 2 : 1);         // classes (issuing warps): a power of two that divides NGRP
   // K-split (see the kernel): CTAs that own a single tile deal its stages to two classes.  Possible when a launch has two
   // classes anyway (T == 2 or 3: the deep levels with one or two tiles per CTA) or one tile per CTA and room for a second
-  // accumulator; SCN_B200_TC_KSPLIT=0 turns it off.
+  // accumulator.
   p.ksplit = 0;
   const int stages_per_tile = (pair ? (K + 1) / 2 : K) * nch;
-  if (g_ksplit_enabled() && stages_per_tile >= 2) {          // both accumulators must receive a first stage
+  if (stages_per_tile >= 2) {          // both accumulators must receive a first stage
     if (p.NM == 1 && per_cta == 1 && 2 * n_out <= 512) { p.NM = 2; p.nbuf = 1; p.ksplit = 1; }
     else if (p.NM == 2) p.ksplit = 1;
   }

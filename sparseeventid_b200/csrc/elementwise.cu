@@ -4,17 +4,12 @@
 // src/networks/sparse_building_blocks.py:39,45,80-82,96-98,122,128; src/networks/resnet.py:123-125,143).
 // All kernels are HBM-bound: 16-byte (fp32) / 8-byte (bf16) vector accesses along channels,
 // fp32 math, column reductions finished with fp64 atomics.
-#include <cooperative_groups.h>
-
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <type_traits>
 #include <utility>
 
 #include "common.cuh"
-
-namespace cg = cooperative_groups;
 
 namespace {
 
@@ -259,242 +254,7 @@ __global__ void __launch_bounds__(256) k_bn_bwd_apply_rows(const T* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------
-// Training-mode BatchNormalization in ONE cooperative launch per direction (C % 8 == 0, C <= 2048).
-// The four-launch form (memset, column reduction, finalize, apply) costs ~27 us (forward) / ~40 us (backward) of
-// launch latency and dependency bubbles even on a 7 k-row level, more than the data movement of every level below
-// the first two.  Here: phase 1 = column sums (registers -> shared memory -> one fp64 atomic per channel and block),
-// grid.sync(), phase 2 = every thread folds the statistics of ITS 8 channels into registers and streams the rows
-// (the re-read of x comes from L2 for most levels), grid.sync(), and the accumulators are zeroed again for the next
-// user -- `acc` must be all zero on entry (scn_bn_*: the scratch is zero-initialised once and every kernel that uses
-// it leaves it zero).
-// ---------------------------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(256) k_bn_fwd_fused(const T* __restrict__ x, int64_t n, int C, const float* __restrict__ gamma,
-                                                      const float* __restrict__ beta, float* running_mean,
-                                                      float* running_var, float eps, float momentum, float leak,
-                                                      float* __restrict__ save_mean, float* __restrict__ save_invstd,
-                                                      double* acc, T* __restrict__ out) {
-  extern __shared__ float sred[];                        // [RY][CV][16]
-  cg::grid_group grid = cg::this_grid();
-  const int CV = C >> 3, RY = 256 / CV;
-  const int tx = threadIdx.x % CV, ty = threadIdx.x / CV;
-  const bool active = ty < RY;
-  const int64_t stride = (int64_t)gridDim.x * RY;
-  // ---- phase 1: sum and sum of squares of (x - pivot), pivot = row 0
-  float a[8], b[8], pv[8];
-#pragma unroll
-  for (int k = 0; k < 8; ++k) a[k] = b[k] = 0.f;
-  if (active) {
-    LoadVec<T, 8>::ld(x + tx * 8, pv);
-    // 4 rows per iteration: with one 16-byte load in flight per thread the kernel was bound by bytes in flight
-    // (148 SMs x 1024 threads x 16 B = 2.4 MB against ~6.5 MB needed to cover the latency at HBM speed)
-    int64_t r = (int64_t)blockIdx.x * RY + ty;
-    for (; r + 3 * stride < n; r += 4 * stride) {
-      float v[4][8];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) LoadVec<T, 8>::ld(x + (r + u * stride) * C + tx * 8, v[u]);
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-#pragma unroll
-        for (int k = 0; k < 8; ++k) { const float d = v[u][k] - pv[k]; a[k] += d; b[k] += d * d; }
-    }
-    for (; r < n; r += stride) {
-      float v[8];
-      LoadVec<T, 8>::ld(x + r * C + tx * 8, v);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) { const float d = v[k] - pv[k]; a[k] += d; b[k] += d * d; }
-    }
-    float* dst = sred + ((size_t)ty * CV + tx) * 16;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { dst[k] = a[k]; dst[8 + k] = b[k]; }
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < CV * 16; i += 256) {
-    const int cx = i >> 4, w = i & 15;
-    float sum = 0.f;
-    for (int y = 0; y < RY; ++y) sum += sred[((size_t)y * CV + cx) * 16 + w];
-    atomicAdd(acc + (size_t)(w >> 3) * C + cx * 8 + (w & 7), (double)sum);
-  }
-  grid.sync();
-  // ---- phase 2: statistics of this thread's channels, running statistics (block 0), apply
-  float sc[8], sh[8];
-  if (active) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const int c = tx * 8 + k;
-      const double s1 = acc[c] / (double)n, s2 = acc[C + c] / (double)n;
-      const double mean = (double)pv[k] + s1;
-      double var = s2 - s1 * s1;
-      if (var < 0.0) var = 0.0;
-      const float m = (float)mean, is = (float)(1.0 / sqrt(var + (double)eps));
-      if (blockIdx.x == 0 && ty == 0) {
-        const double unbiased = var * (double)n / (double)(n > 1 ? n - 1 : 1);
-        running_mean[c] = (float)((double)momentum * running_mean[c] + (1.0 - (double)momentum) * mean);
-        running_var[c] = (float)((double)momentum * running_var[c] + (1.0 - (double)momentum) * unbiased);
-        save_mean[c] = m;
-        save_invstd[c] = is;
-      }
-      sc[k] = is * (gamma ? gamma[c] : 1.f);
-      sh[k] = (beta ? beta[c] : 0.f) - m * sc[k];
-    }
-    int64_t r = (int64_t)blockIdx.x * RY + ty;
-    for (; r + 3 * stride < n; r += 4 * stride) {
-      float v[4][8];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) LoadVec<T, 8>::ld(x + (r + u * stride) * C + tx * 8, v[u]);
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const float y = fmaf(v[u][k], sc[k], sh[k]);
-          v[u][k] = (leak != 1.f && !(y > 0.f)) ? y * leak : y;
-        }
-        LoadVec<T, 8>::st(out + (r + u * stride) * C + tx * 8, v[u]);
-      }
-    }
-    for (; r < n; r += stride) {
-      float v[8];
-      LoadVec<T, 8>::ld(x + r * C + tx * 8, v);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        const float y = fmaf(v[k], sc[k], sh[k]);
-        v[k] = (leak != 1.f && !(y > 0.f)) ? y * leak : y;
-      }
-      LoadVec<T, 8>::st(out + r * C + tx * 8, v);
-    }
-  }
-  grid.sync();
-  if (blockIdx.x == 0)
-    for (int i = threadIdx.x; i < 2 * C; i += 256) acc[i] = 0.0;
-}
-
-template <typename T>
-__global__ void __launch_bounds__(256) k_bn_bwd_fused(const T* __restrict__ x, const T* __restrict__ dout, int64_t n, int C,
-                                                      const float* __restrict__ mean, const float* __restrict__ invstd,
-                                                      const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                      float leak, double* acc, T* __restrict__ dx, float* dgamma,
-                                                      float* dbeta, int accumulate) {
-  extern __shared__ float sred[];
-  cg::grid_group grid = cg::this_grid();
-  const int CV = C >> 3, RY = 256 / CV;
-  const int tx = threadIdx.x % CV, ty = threadIdx.x / CV;
-  const bool active = ty < RY;
-  const int64_t stride = (int64_t)gridDim.x * RY;
-  float m[8], is[8], g[8], bt[8];
-  if (active) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const int c = tx * 8 + k;
-      m[k] = mean[c]; is[k] = invstd[c];
-      g[k] = gamma ? gamma[c] : 1.f;
-      bt[k] = beta ? beta[c] : 0.f;
-    }
-  }
-  // ---- phase 1: sums of d and d * xhat  (d = dout through the fused leaky ReLU)
-  float a[8], b[8];
-#pragma unroll
-  for (int k = 0; k < 8; ++k) a[k] = b[k] = 0.f;
-  if (active) {
-    int64_t r = (int64_t)blockIdx.x * RY + ty;
-    for (; r + stride < n; r += 2 * stride) {              // 2 rows x 2 tensors: four 16-byte loads in flight per thread
-      float v[2][8], d[2][8];
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        LoadVec<T, 8>::ld(x + (r + u * stride) * C + tx * 8, v[u]);
-        LoadVec<T, 8>::ld(dout + (r + u * stride) * C + tx * 8, d[u]);
-      }
-#pragma unroll
-      for (int u = 0; u < 2; ++u)
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const float xh = (v[u][k] - m[k]) * is[k];
-          const float y = xh * g[k] + bt[k];
-          const float dd = (leak != 1.f && !(y > 0.f)) ? d[u][k] * leak : d[u][k];
-          a[k] += dd;
-          b[k] += dd * xh;
-        }
-    }
-    for (; r < n; r += stride) {
-      float v[8], d[8];
-      LoadVec<T, 8>::ld(x + r * C + tx * 8, v);
-      LoadVec<T, 8>::ld(dout + r * C + tx * 8, d);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        const float xh = (v[k] - m[k]) * is[k];
-        const float y = xh * g[k] + bt[k];
-        const float dd = (leak != 1.f && !(y > 0.f)) ? d[k] * leak : d[k];
-        a[k] += dd;
-        b[k] += dd * xh;
-      }
-    }
-    float* dst = sred + ((size_t)ty * CV + tx) * 16;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { dst[k] = a[k]; dst[8 + k] = b[k]; }
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < CV * 16; i += 256) {
-    const int cx = i >> 4, w = i & 15;
-    float sum = 0.f;
-    for (int y = 0; y < RY; ++y) sum += sred[((size_t)y * CV + cx) * 16 + w];
-    atomicAdd(acc + (size_t)(w >> 3) * C + cx * 8 + (w & 7), (double)sum);
-  }
-  grid.sync();
-  // ---- phase 2: parameter gradients (block 0), dx
-  if (active) {
-    float s1[8], s2[8];
-    const float inv_n = n > 0 ? 1.f / (float)n : 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const int c = tx * 8 + k;
-      const double sa = acc[c], sb = acc[C + c];
-      if (blockIdx.x == 0 && ty == 0) {
-        if (dbeta) dbeta[c] = (accumulate ? dbeta[c] : 0.f) + (float)sa;
-        if (dgamma) dgamma[c] = (accumulate ? dgamma[c] : 0.f) + (float)sb;
-      }
-      s1[k] = (float)sa * inv_n;
-      s2[k] = (float)sb * inv_n;
-    }
-    int64_t r = (int64_t)blockIdx.x * RY + ty;
-    for (; r + stride < n; r += 2 * stride) {
-      float v[2][8], d[2][8];
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        LoadVec<T, 8>::ld(x + (r + u * stride) * C + tx * 8, v[u]);
-        LoadVec<T, 8>::ld(dout + (r + u * stride) * C + tx * 8, d[u]);
-      }
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          const float xh = (v[u][k] - m[k]) * is[k];
-          const float y = xh * g[k] + bt[k];
-          const float dd = (leak != 1.f && !(y > 0.f)) ? d[u][k] * leak : d[u][k];
-          v[u][k] = g[k] * is[k] * (dd - s1[k] - xh * s2[k]);
-        }
-        LoadVec<T, 8>::st(dx + (r + u * stride) * C + tx * 8, v[u]);
-      }
-    }
-    for (; r < n; r += stride) {
-      float v[8], d[8];
-      LoadVec<T, 8>::ld(x + r * C + tx * 8, v);
-      LoadVec<T, 8>::ld(dout + r * C + tx * 8, d);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        const float xh = (v[k] - m[k]) * is[k];
-        const float y = xh * g[k] + bt[k];
-        const float dd = (leak != 1.f && !(y > 0.f)) ? d[k] * leak : d[k];
-        v[k] = g[k] * is[k] * (dd - s1[k] - xh * s2[k]);
-      }
-      LoadVec<T, 8>::st(dx + r * C + tx * 8, v);
-    }
-  }
-  grid.sync();
-  if (blockIdx.x == 0)
-    for (int i = threadIdx.x; i < 2 * C; i += 256) acc[i] = 0.0;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Training-mode BatchNormalization as TWO ordinary launches per direction (default; C % 8 == 0, C <= 2048):
+// Training-mode BatchNormalization as TWO ordinary launches per direction (C % 8 == 0, C <= 2048):
 //   statistics kernel: column sums -> one of two sets of fp64 accumulators (zero on entry), nothing else,
 //   apply kernel:      every thread folds the statistics of its 8 channels into registers (forward: scale / shift,
 //                      block 0 also writes the saved and running statistics; backward: the three coefficients of dx,
@@ -502,9 +262,12 @@ __global__ void __launch_bounds__(256) k_bn_bwd_fused(const T* __restrict__ x, c
 //                      streams the rows.  The backward apply also sums the columns of the dx it stores: that is the
 //                      bias gradient of the convolution in front of the BatchNorm (56 column-sum launches and one read
 //                      of every dx per step otherwise).
-// Measured against the cooperative single-launch kernels above (ncu, 495 k rows x 32 channels, backward): 18% of the
-// kernel was its final grid barrier + re-zeroing, 7% the first barrier, 102 registers held it to 2 blocks per SM, a
-// cooperative launch costs ~6-10 us more than an ordinary one on the stream, and every thread folded the statistics of
+// The four-launch form (memset, column reduction, finalize, apply), which eval mode and the other channel counts use,
+// costs ~27 us (forward) / ~40 us (backward) of launch latency and dependency bubbles even on a 7 k-row level, more than
+// the data movement of every level below the first two.  A single cooperative launch per direction (column sums, grid
+// barrier, apply, grid barrier, re-zeroing) was measured too and removed (ncu, 495 k rows x 32 channels, backward): 18%
+// of the kernel was its final grid barrier + re-zeroing, 7% the first barrier, 102 registers held it to 2 blocks per SM,
+// a cooperative launch costs ~6-10 us more than an ordinary one on the stream, and every thread folded the statistics of
 // its channels with fp64 divisions and square roots (~6 us per block on the thin fp64 pipe).  Here the kernels run at
 // 3-4 blocks x 256 threads per SM with 64 B in flight per thread; the fold is 2 fp64 multiplies, one fma and a
 // Newton-refined rsqrt per channel.
@@ -910,41 +673,29 @@ __global__ void __launch_bounds__(256) k_col_sum_fused(const T* __restrict__ x, 
   }
 }
 
-// grid of a cooperative BatchNorm launch: every block must be resident at once
-template <typename K>
-int bn_coop_grid(K kern, int64_t n, int ry, size_t smem) {
-  static int per_sm = 0;
-  if (per_sm == 0) {
-    int v = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, kern, 256, smem) != cudaSuccess || v < 1) v = 1;
-    per_sm = v > 4 ? 4 : v;
-  }
-  int64_t g = (n + (int64_t)ry * 4 - 1) / ((int64_t)ry * 4);         // >= 4 rows per thread and phase
-  const int64_t cap = (int64_t)kNumSMs * per_sm;
-  if (g > cap) g = cap;
-  return (int)(g < 1 ? 1 : g);
-}
-// fp64 accumulators of the fused kernels: 2 x 2048 doubles (BatchNorm) + 2048 doubles and a ticket (column sums) per
-// (device, stream), allocated and zeroed once; every
-// fused kernel finds them zero and leaves them zero, so no memset precedes a launch.  nullptr if allocation fails
-// (the caller then takes the four-launch path).
+// fp64 accumulators of the two-launch BatchNorm kernels and k_col_sum_fused: 2 x 2048 doubles (BatchNorm) + 2048 doubles
+// and a ticket (column sums) per (device, stream), allocated and zeroed once; every such kernel finds them zero and
+// leaves them zero, so no memset precedes a launch.
 constexpr int kAcc1 = 3 * 2048 + 2;          // second set of BatchNorm accumulators (2 x 2048 doubles) behind the tickets
 constexpr size_t kScratchDoubles = (size_t)kAcc1 + 2 * 2048;
-struct ScratchEntry { double* p = nullptr; unsigned phase = 0; bool tried = false; int last_c[2] = {0, 0}; };
+struct ScratchEntry { double* p = nullptr; unsigned phase = 0; int last_c[2] = {0, 0}; };
 static std::mutex g_scratch_mu;
 static std::map<std::pair<int, cudaStream_t>, ScratchEntry> g_scratch;
-double* zero_scratch(cudaStream_t s) {
+int zero_scratch(cudaStream_t s, double** out) {
   int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
+  SCN_CUDA(cudaGetDevice(&dev));
   std::lock_guard<std::mutex> lock(g_scratch_mu);
   ScratchEntry& e = g_scratch[{dev, s}];
-  if (e.tried) return e.p;
-  e.tried = true;
-  double* p = nullptr;
-  if (cudaMalloc(&p, kScratchDoubles * sizeof(double)) != cudaSuccess) { (void)cudaGetLastError(); p = nullptr; }
-  else if (cudaMemsetAsync(p, 0, kScratchDoubles * sizeof(double), s) != cudaSuccess) { cudaFree(p); p = nullptr; }
-  e.p = p;
-  return p;
+  if (e.p == nullptr) {
+    double* p = nullptr;
+    const cudaError_t err = cudaMalloc(&p, kScratchDoubles * sizeof(double));
+    if (err != cudaSuccess) { (void)cudaGetLastError(); return (int)err; }
+    const cudaError_t err2 = cudaMemsetAsync(p, 0, kScratchDoubles * sizeof(double), s);
+    if (err2 != cudaSuccess) { cudaFree(p); return (int)err2; }
+    e.p = p;
+  }
+  *out = e.p;
+  return SCN_OK;
 }
 // which set of BatchNorm accumulators the next two-launch BatchNorm call of this stream uses (alternates per call)
 // *zero_n: how many doubles of the OTHER set this call's apply kernel must clear -- what that set's last user (the
@@ -962,16 +713,6 @@ unsigned bn_next_phase(cudaStream_t s, int C, int* zero_n) {
 }
 // (Channel-sliced kernels -- one block per 8 channels over all rows, no grid barrier -- were measured for the small levels
 // and are slower: 50 / 71 us against 36 / 24 us at 20 k rows x 160 channels: a warp then touches 32 different rows.)
-// SCN_B200_BN_FUSED: 0 = four-launch reference path, 1 = cooperative single-launch kernels, 2 (default) = two launches
-int bn_mode() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = std::getenv("SCN_B200_BN_FUSED");
-    v = (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 2;
-  }
-  return v;
-}
-bool bn_fused_enabled() { return bn_mode() != 0; }
 // grid of the two-launch kernels: >= 4 rows per thread, at most one resident wave (per_sm blocks per SM)
 int bn_grid2(int64_t n, int ry, int per_sm) {
   int64_t g = (n + (int64_t)ry * 4 - 1) / ((int64_t)ry * 4);
@@ -1169,9 +910,10 @@ int bn_forward_t(const T* x, int64_t n, int C, const float* gamma, const float* 
                  double* ws, T* out, cudaStream_t s) {
   const bool vec = (C % 4) == 0;
   const bool vec8 = (C % 8) == 0 && (((uintptr_t)x | (uintptr_t)out) & 15) == 0;
-  double* const ws_caller = ws;
-  double* zws = (training && vec8 && C <= 2048 && n > 0 && bn_fused_enabled()) ? zero_scratch(s) : nullptr;
-  if (zws != nullptr && bn_mode() == 2) {
+  if (training && vec8 && C <= 2048 && n > 0) {
+    double* zws = nullptr;
+    const int rc = zero_scratch(s, &zws);
+    if (rc != SCN_OK) return rc;
     const int ry = 256 / (C >> 3);
     const int g = bn_grid2(n, ry, 4);
     int zero_n = 0;
@@ -1184,21 +926,6 @@ int bn_forward_t(const T* x, int64_t n, int C, const float* gamma, const float* 
                             save_mean, save_invstd, (const double*)acc, other, zero_n, 1.0 / (double)n, out));
     SCN_LAUNCH_CHECK();
     return SCN_OK;
-  }
-  if (zws != nullptr) {
-    ws = zws;                                 // library-owned accumulators, all zero between kernels
-    const int ry = 256 / (C >> 3);
-    const size_t smem = (size_t)ry * (C >> 3) * 16 * sizeof(float);
-    auto kern = k_bn_fwd_fused<T>;
-    const int g = bn_coop_grid(kern, n, ry, smem);
-    void* args[] = {(void*)&x, (void*)&n, (void*)&C, (void*)&gamma, (void*)&beta, (void*)&rm, (void*)&rv, (void*)&eps,
-                    (void*)&momentum, (void*)&leak, (void*)&save_mean, (void*)&save_invstd, (void*)&ws, (void*)&out};
-    if (cudaLaunchCooperativeKernel((void*)kern, dim3((unsigned)g), dim3(256), args, smem, s) == cudaSuccess) {
-      SCN_LAUNCH_CHECK();
-      return SCN_OK;
-    }
-    (void)cudaGetLastError();                   // cooperative launch refused (e.g. MPS limits): four-launch path below
-    ws = ws_caller;
   }
   if (training) {
     SCN_CUDA(cudaMemsetAsync(ws, 0, 2 * (size_t)C * sizeof(double), s));
@@ -1235,9 +962,10 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
                   float* dgamma, float* dbeta, int accumulate, float* colsum, cudaStream_t s) {
   const bool vec = (C % 4) == 0;
   const bool vec8 = (C % 8) == 0 && (((uintptr_t)x | (uintptr_t)dout | (uintptr_t)dx) & 15) == 0;
-  double* const ws_caller = ws;
-  double* zws = (training && vec8 && C <= 2048 && n > 0 && bn_fused_enabled()) ? zero_scratch(s) : nullptr;
-  if (zws != nullptr && bn_mode() == 2) {
+  if (training && vec8 && C <= 2048 && n > 0) {
+    double* zws = nullptr;
+    const int rc = zero_scratch(s, &zws);
+    if (rc != SCN_OK) return rc;
     const int ry = 256 / (C >> 3);
     int zero_n = 0;
     const unsigned ph = bn_next_phase(s, C, &zero_n);
@@ -1258,22 +986,6 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
                               colacc, ticket, (float*)nullptr));
     SCN_LAUNCH_CHECK();
     return SCN_OK;
-  }
-  if (zws != nullptr) {
-    ws = zws;
-    const int ry = 256 / (C >> 3);
-    const size_t smem = (size_t)ry * (C >> 3) * 16 * sizeof(float);
-    auto kern = k_bn_bwd_fused<T>;
-    const int g = bn_coop_grid(kern, n, ry, smem);
-    void* args[] = {(void*)&x, (void*)&dout, (void*)&n, (void*)&C, (void*)&mean, (void*)&invstd, (void*)&gamma,
-                    (void*)&beta, (void*)&leak, (void*)&ws, (void*)&dx, (void*)&dgamma, (void*)&dbeta, (void*)&accumulate};
-    if (cudaLaunchCooperativeKernel((void*)kern, dim3((unsigned)g), dim3(256), args, smem, s) == cudaSuccess) {
-      SCN_LAUNCH_CHECK();
-      if (colsum) return scn_col_sum(dx, std::is_same<T, float>::value ? SCN_F32 : SCN_BF16, n, C, ws_caller, colsum, s);
-      return SCN_OK;
-    }
-    (void)cudaGetLastError();
-    ws = ws_caller;
   }
   SCN_CUDA(cudaMemsetAsync(ws, 0, 2 * (size_t)C * sizeof(double), s));
   if (n > 0) {
@@ -1303,7 +1015,7 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
                                                               training, ws, dx);
   SCN_LAUNCH_CHECK();
   if (colsum)      // paths without the fused column sums: one more pass over dx
-    return scn_col_sum(dx, std::is_same<T, float>::value ? SCN_F32 : SCN_BF16, n, C, ws_caller, colsum, s);
+    return scn_col_sum(dx, std::is_same<T, float>::value ? SCN_F32 : SCN_BF16, n, C, ws, colsum, s);
   return SCN_OK;
 }
 
@@ -1389,26 +1101,26 @@ extern "C" int scn_col_sum_acc(const void* x, int dtype, int64_t n, int C, doubl
                                void* stream) {
   cudaStream_t s = (cudaStream_t)stream;
   if (C < 1 || !out || !stats_ws) return SCN_ERR_ARG;
-  if (n > 0 && (C % 8) == 0 && C <= 2048 && (((uintptr_t)x) & 15) == 0 && bn_fused_enabled()) {
-    double* z = zero_scratch(s);
-    if (z != nullptr) {
-      double* acc1 = z + 2 * 2048;
-      unsigned* ticket = reinterpret_cast<unsigned*>(z + 3 * 2048);
-      const int ry = 256 / (C >> 3);
-      int64_t g = (n + (int64_t)ry * 8 - 1) / ((int64_t)ry * 8);
-      if (g > (int64_t)kNumSMs * 4) g = (int64_t)kNumSMs * 4;
-      if (g < 1) g = 1;
-      const size_t smem = (size_t)ry * (C >> 3) * 8 * sizeof(float);
-      if (dtype == SCN_F32)
-        SCN_CUDA(scn_launch_pdl(k_col_sum_fused<float>, dim3((unsigned)g), dim3(256), smem, s, (const float*)x, n, C, acc1, ticket, out, accumulate));
-      else if (dtype == SCN_BF16)
-        SCN_CUDA(scn_launch_pdl(k_col_sum_fused<__nv_bfloat16>, dim3((unsigned)g), dim3(256), smem, s, (const __nv_bfloat16*)x, n, C, acc1,
-                                ticket, out, accumulate));
-      else
-        return SCN_ERR_ARG;
-      SCN_LAUNCH_CHECK();
-      return SCN_OK;
-    }
+  if (n > 0 && (C % 8) == 0 && C <= 2048 && (((uintptr_t)x) & 15) == 0) {
+    double* z = nullptr;
+    const int rc = zero_scratch(s, &z);
+    if (rc != SCN_OK) return rc;
+    double* acc1 = z + 2 * 2048;
+    unsigned* ticket = reinterpret_cast<unsigned*>(z + 3 * 2048);
+    const int ry = 256 / (C >> 3);
+    int64_t g = (n + (int64_t)ry * 8 - 1) / ((int64_t)ry * 8);
+    if (g > (int64_t)kNumSMs * 4) g = (int64_t)kNumSMs * 4;
+    if (g < 1) g = 1;
+    const size_t smem = (size_t)ry * (C >> 3) * 8 * sizeof(float);
+    if (dtype == SCN_F32)
+      SCN_CUDA(scn_launch_pdl(k_col_sum_fused<float>, dim3((unsigned)g), dim3(256), smem, s, (const float*)x, n, C, acc1, ticket, out, accumulate));
+    else if (dtype == SCN_BF16)
+      SCN_CUDA(scn_launch_pdl(k_col_sum_fused<__nv_bfloat16>, dim3((unsigned)g), dim3(256), smem, s, (const __nv_bfloat16*)x, n, C, acc1,
+                              ticket, out, accumulate));
+    else
+      return SCN_ERR_ARG;
+    SCN_LAUNCH_CHECK();
+    return SCN_OK;
   }
   double* acc = stats_ws;
   SCN_CUDA(cudaMemsetAsync(acc, 0, 2 * (size_t)C * sizeof(double), s));

@@ -18,7 +18,6 @@
 //
 // Replaces SCN's Convolution forward / backward for the reference's initial_convolution
 // (src/networks/resnet.py:30-36: SubmanifoldConvolution(nIn=1, nOut=n_initial_filters, filter_size=5)).
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -239,15 +238,6 @@ __global__ void __launch_bounds__(256, 2) k_stem_wgrad(const TI* __restrict__ x,
 }
 
 }  // namespace stem
-
-bool scn_stem_tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = std::getenv("SCN_B200_STEM_TC");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
 
 bool scn_stem_tc_shape_ok(int K, int n_in, int n_out) { return n_in == 1 && n_out == stem::NOUT && K >= 1 && K <= 16 * stem::MAXKT; }
 

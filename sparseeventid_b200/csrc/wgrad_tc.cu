@@ -9,11 +9,12 @@
 // K=16) contracts 16 pairs and the Cin x Cout accumulator of the offset stays in TMEM for the whole CTA.
 //
 // Work split: every CTA owns ONE offset k and a contiguous range of output rows (the centre offset of a submanifold
-// table holds every row and gets proportionally more CTAs), so dW receives one pass of atomics per CTA.
+// table holds every row and gets proportionally more CTAs).  A CTA writes its Cin x Cout partial sum to a slab of its
+// own; k_wgrad_reduce adds the slabs of an offset into dW in a fixed order.
 // Roles: producer warps (each walks its share of 128-row blocks, ballots the neighbour indices, appends the live pairs
 // to a ring and emits a stage whenever 64 are pending; LDGSTS copies that signal their own landing), one issuing warp
 // that consumes the producers' stages in a fixed round-robin order (so dW is bitwise reproducible), 4 epilogue warps
-// (tcgen05.ld -> red.global.add.f32).
+// (tcgen05.ld -> slab stores).
 //
 // TF32 instantiation (precision SCN_PREC_TF32, fp32 x and dout): a stage row is 128 bytes = 32 fp32 channels, so blocks
 // are 32 channels wide (nca, ncb up to 8: runtime counts, one instantiation per pairs-per-stage) and one
@@ -46,8 +47,7 @@ struct Params {
   const void* x;                // [n_in_rows, Cin] bf16 (fp32 for the TF32 instantiation)
   const void* dout;             // [n_rows, Cout], the element type of x
   const int32_t* nbr;           // [K][n_pad]: input row of output row o at offset k, or -1
-  float* dW;                    // [K][Cin][Cout], accumulated into (by k_wgrad_reduce, or by atomics when part == nullptr)
-  float* part;                  // [gridDim.x][Cin][Cout] partial sums, one slab per CTA, or nullptr
+  float* part;                  // [gridDim.x][Cin][Cout] partial sums, one slab per CTA
   int64_t n_rows, n_pad;
   int K, Cin, Cout;
   int nca, ncb;                 // channel blocks (128-byte rows: 64 bf16 / 32 fp32 channels) per stage: A, B
@@ -321,7 +321,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
     if (elect_one()) umma_commit(accf);
     __syncwarp();
   } else if (warp < EPI_WARPS) {
-    // ================================ epilogue: TMEM -> dW atomics ============================
+    // ================================ epilogue: TMEM -> slab ==================================
     mbar_wait_long(accf, 0u);
     tc_fence_after();
     const uint32_t any = ld_acquire_u32(done + 4u * (uint32_t)PROD_WARPS);
@@ -331,6 +331,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
     for (int mb = 0; mb < (TF32 ? p.nmb : (NA + 1) / 2); ++mb) {
       const int cin = mb * 128 + warp * 32 + lane;                            // accumulator row == input channel
       const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(mb * p.Cout);
+      // one 32-column chunk at a time: unrolled, this loop takes 76-78 registers instead of 43-56
+#pragma unroll 1
       for (int c0 = 0; c0 < p.Cout; c0 += 32) {
         uint32_t v[32];
         if (any == 2u) {
@@ -340,18 +342,9 @@ __global__ void __launch_bounds__(THREADS, 1) k_wgrad_tc(const Params p) {
           for (int e = 0; e < 32; ++e) v[e] = 0u;                             // no pair in this CTA's range: a slab of zeros
         }
         if (cin < p.Cin) {
-          if (p.part != nullptr) {
-            uint4* dst = reinterpret_cast<uint4*>(p.part + ((size_t)blockIdx.x * p.Cin + cin) * p.Cout + c0);
+          uint4* dst = reinterpret_cast<uint4*>(p.part + ((size_t)blockIdx.x * p.Cin + cin) * p.Cout + c0);
 #pragma unroll
-            for (int e = 0; e < 8; ++e) dst[e] = make_uint4(v[4 * e], v[4 * e + 1], v[4 * e + 2], v[4 * e + 3]);
-          } else {
-            float* dst = p.dW + ((int64_t)k * p.Cin + cin) * p.Cout + c0;
-#pragma unroll
-            for (int e = 0; e < 32; ++e) {
-              const float f = __uint_as_float(v[e]);
-              if (f != 0.f) atomicAdd(dst + e, f);
-            }
-          }
+          for (int e = 0; e < 8; ++e) dst[e] = make_uint4(v[4 * e], v[4 * e + 1], v[4 * e + 2], v[4 * e + 3]);
         }
       }
     }
@@ -393,25 +386,28 @@ __global__ void k_wgrad_reduce(const float* __restrict__ part, float* __restrict
 }
 
 // library-owned slab buffer per (device, stream), grown on demand (a growth is a cudaFree + cudaMalloc, i.e. a device
-// synchronisation; it happens a handful of times in the first step).  nullptr if the allocation fails (atomics path).
-float* wgrad_slabs(size_t bytes, cudaStream_t s) {
+// synchronisation; it happens a handful of times in the first step)
+int wgrad_slabs(size_t bytes, cudaStream_t s, float** out) {
   static std::mutex mu;
   static std::map<std::pair<int, cudaStream_t>, std::pair<float*, size_t>> table;
   int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
+  SCN_CUDA(cudaGetDevice(&dev));
   std::lock_guard<std::mutex> lock(mu);
   auto& e = table[{dev, s}];
-  if (e.second >= bytes) return e.first;
-  if (e.first != nullptr) {
-    if (cudaStreamSynchronize(s) != cudaSuccess) return nullptr;
-    cudaFree(e.first);
-    e = {nullptr, 0};
+  if (e.second < bytes) {
+    if (e.first != nullptr) {
+      SCN_CUDA(cudaStreamSynchronize(s));
+      cudaFree(e.first);
+      e = {nullptr, 0};
+    }
+    const size_t want = bytes + bytes / 4;
+    float* p = nullptr;
+    const cudaError_t err = cudaMalloc(&p, want);
+    if (err != cudaSuccess) { (void)cudaGetLastError(); return (int)err; }
+    e = {p, want};
   }
-  const size_t want = bytes + bytes / 4;
-  float* p = nullptr;
-  if (cudaMalloc(&p, want) != cudaSuccess) { (void)cudaGetLastError(); return nullptr; }
-  e = {p, want};
-  return p;
+  *out = e.first;
+  return SCN_OK;
 }
 
 struct BiasFold { const float* colsum; float* dbias; int C; int accumulate; };
@@ -433,15 +429,6 @@ extern "C" void scn_wgrad_debug_last_launch(int32_t* out) {
   for (int i = 0; i < 7; ++i) out[i] = g_wg_last_launch[i];
 }
 
-bool scn_wgrad_tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = std::getenv("SCN_B200_WGRAD_TC");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-
 // dW[K][Cin][Cout] += ...; x, dout bf16, or fp32 with tf32 != 0 (TF32 MMAs).  Returns SCN_ERR_UNSUPPORTED for shapes
 // outside the kernel (caller falls back).  Gathered rows are addressed through 32-bit offsets in 16-byte units: x and
 // dout up to 64 GB each.
@@ -451,7 +438,7 @@ int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int
   if ((uint64_t)n_rows * (uint64_t)(Cout * (tf32 ? 4 : 2) / 16) >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;
   if (n_pad < ((n_rows + 127) / 128) * 128) return SCN_ERR_ARG;      // whole 128-row blocks are read
   wg::Params p;
-  p.x = x; p.dout = dout; p.nbr = nbr; p.dW = dW; p.n_rows = n_rows; p.n_pad = n_pad; p.K = K; p.Cin = Cin; p.Cout = Cout;
+  p.x = x; p.dout = dout; p.nbr = nbr; p.n_rows = n_rows; p.n_pad = n_pad; p.K = K; p.Cin = Cin; p.Cout = Cout;
   p.nmb = (Cin + 127) / 128;
   const int blk = tf32 ? 32 : 64;                            // channels per 128-byte block
   p.nca = (Cin + blk - 1) / blk;
@@ -473,7 +460,7 @@ int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int
   // CTAs (one per SM at a time: the kernel uses all of shared memory): ONE full wave, or two for big tables -- never
   // a few CTAs more than a wave (150 CTAs on 148 SMs run for two waves: measured 86 us instead of ~45 at 20 k rows x
   // 160 channels).  The centre offset of an odd-sized (submanifold) table holds every row -> 3.5x the share of the
-  // others.  Small tables get fewer CTAs: every CTA pays a fixed price (TMEM allocation, Cin*Cout atomics), so it
+  // others.  Small tables get fewer CTAs: every CTA pays a fixed price (TMEM allocation, a Cin*Cout slab), so it
   // should own ~500 pairs or more (about 30% of the K*n table entries are pairs in the reference's networks).
   static const int pairs_per_cta = [] {                      // developer knob for sweeps: SCN_B200_WG_PAIRS=<pairs per CTA>
     const char* e = std::getenv("SCN_B200_WG_PAIRS");
@@ -504,12 +491,9 @@ int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int
   }
   const int grid = (p.centre >= 0 ? (K - 1) * p.s_other + p.s_centre : K * p.s_other);
   const size_t smem = (size_t)fixed + (size_t)slots * slot_bytes;
-  static const bool use_slabs = [] {                         // SCN_B200_WG_ATOMICS=1: the old epilogue (atomics into dW)
-    const char* e = std::getenv("SCN_B200_WG_ATOMICS");
-    return !(e && e[0] == '1');
-  }();
   const int CC = Cin * Cout;
-  p.part = use_slabs ? wg::wgrad_slabs((size_t)grid * CC * sizeof(float), s) : nullptr;
+  const int rc = wg::wgrad_slabs((size_t)grid * CC * sizeof(float), s, &p.part);
+  if (rc != SCN_OK) return rc;
   {
     const int32_t rec[7] = {grid, p.s_other, p.s_centre, pairs, slots, p.nca, p.ncb};
     for (int i = 0; i < 7; ++i) g_wg_last_launch[i] = rec[i];
@@ -518,13 +502,11 @@ int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int
     SCN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     SCN_CUDA(scn_launch_pdl(kern, dim3((unsigned)grid), dim3(wg::THREADS), smem, s, p));
     SCN_LAUNCH_CHECK();
-    if (p.part != nullptr) {
-      const wg::BiasFold bf = wg::g_fold;
-      wg::g_fold = {nullptr, nullptr, 0, 0};
-      SCN_CUDA(scn_launch_pdl(wg::k_wgrad_reduce, dim3(grid_for((int64_t)K * CC / 4, 256)), dim3(256), 0, s, (const float*)p.part, dW,
-                              K, CC, p.s_other, p.s_centre, p.centre, bf.colsum, bf.dbias, bf.C, bf.accumulate));
-      SCN_LAUNCH_CHECK();
-    }
+    const wg::BiasFold bf = wg::g_fold;
+    wg::g_fold = {nullptr, nullptr, 0, 0};
+    SCN_CUDA(scn_launch_pdl(wg::k_wgrad_reduce, dim3(grid_for((int64_t)K * CC / 4, 256)), dim3(256), 0, s, (const float*)p.part, dW,
+                            K, CC, p.s_other, p.s_centre, p.centre, bf.colsum, bf.dbias, bf.C, bf.accumulate));
+    SCN_LAUNCH_CHECK();
     return SCN_OK;
   };
   if (tf32) {

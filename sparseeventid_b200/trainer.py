@@ -11,7 +11,6 @@ src/utils/training_utils.py:13 (Adam lr=1.0 x schedule, eps 1e-6, betas (0.8, 0.
 from __future__ import annotations
 
 import os
-import threading
 from typing import Dict, List, Optional
 
 import torch
@@ -202,9 +201,6 @@ class Trainer:
         self.sched = torch.optim.lr_scheduler.LambdaLR(self.opt, lambda s: warmup_flat_lr(s, peak_lr))
         self.peak_lr = peak_lr
         self.global_step = 0
-        self.prefetch_thread = os.environ.get("SCN_B200_PREFETCH_THREAD", "0") not in ("0", "false", "False")
-        self._prefetch_thread = None
-        self._prefetch_error = None
         self.graph_head = os.environ.get("SCN_B200_GRAPH_HEAD", "1") not in ("0", "false", "False")
         self._head_graphs = {}
         self.model.train()
@@ -238,35 +234,6 @@ class Trainer:
             return
         from .scn import core
         core.prefetch(next_batch[0], il.dimension, il.spatial_size, il._last_plan, ready_event)
-
-    def _prefetch_async(self, next_batch, ready_event):
-        """prefetch_rulebooks on a helper thread.  Building a batch's rulebooks needs a handful of row counts on the host
-        (one blocking read-back per level); on the stepping thread those waits -- ~4.5 ms per step behind the rulebook
-        kernels -- were a quarter of the time it needs to enqueue a step, and the step is within 10% of being bound by
-        that.  The waits release the GIL, so the stepping thread enqueues the backward meanwhile.  Joined at the start
-        of the next step (the InputLayer adopts the result there).
-        Opt-in (SCN_B200_PREFETCH_THREAD=1): measured on B200, it cuts the stepping thread's enqueue time from 12.9 to
-        10.8 ms per step, but the 20 ms step is GPU-bound either way (3210 vs 3196 events/s)."""
-        def work():
-            try:
-                if self.device.type == "cuda":
-                    torch.cuda.set_device(self.device)          # the current device is thread-local
-                self.prefetch_rulebooks(next_batch, ready_event)
-            except BaseException as e:                          # surfaced by the next step
-                self._prefetch_error = e
-        self._prefetch_error = None
-        th = threading.Thread(target=work, name="scn-rulebook-prefetch", daemon=True)
-        self._prefetch_thread = th
-        th.start()
-
-    def _join_prefetch(self):
-        th = getattr(self, "_prefetch_thread", None)
-        if th is not None:
-            th.join()
-            self._prefetch_thread = None
-            err, self._prefetch_error = getattr(self, "_prefetch_error", None), None
-            if err is not None:
-                raise err
 
     # ---- dense heads + focal loss as ONE CUDA graph per direction ------------------------------------------------------
     # classification_head.py:19-28 + supervised_eventID.py:168-196 on a [B, 128] pooled tensor are ~90 tiny torch launches
@@ -321,7 +288,6 @@ class Trainer:
     def step(self, batch, labels, prefetch=None, prefetch_ready=None):
         """batch: (coords [N,4], features [N,1], batch_size) on self.device; labels: dict of int64 [B].
         prefetch: the next step's batch tuple (same tensor objects that will be passed then), optional."""
-        self._join_prefetch()
         self.arena.zero()
         prep = getattr(self.scn, "prepare_weight_images", None)        # every conv weight image of the step in one launch
         if prep is not None and self.device.type == "cuda":
@@ -334,10 +300,7 @@ class Trainer:
             if loss is None:
                 loss = networks.focal_loss(labels, self.model.head(feat))
             if prefetch is not None:
-                if self.prefetch_thread and self.device.type == "cuda":
-                    self._prefetch_async(prefetch, prefetch_ready)
-                else:
-                    self.prefetch_rulebooks(prefetch, prefetch_ready)
+                self.prefetch_rulebooks(prefetch, prefetch_ready)
             loss.backward()
         finally:
             if prep is not None:

@@ -270,7 +270,7 @@ def test_down_then_deconvolution(scn, mode):
 
 
 @pytest.mark.parametrize("mode", MODES)
-@pytest.mark.parametrize("c,leak", [(32, 1), (96, 0), (160, 0.333), (5, 1)])
+@pytest.mark.parametrize("c,leak", [(32, 1), (96, 0), (160, 0.333), (5, 1), (12, 0.333)])
 def test_batchnorm_train(scn, mode, c, leak):
     grid, B = (16, 16, 16), 2
     coords = random_sites(777, grid, B, seed=11)

@@ -1,4 +1,4 @@
-"""Diagnostic (GPU box only): scn_conv_wgrad (tcgen05 path unless SCN_B200_WGRAD_TC=0) vs a plain torch
+"""Diagnostic (GPU box only): scn_conv_wgrad (tcgen05 path) vs a plain torch
 gather + matmul of the same bf16 operands; prints the error structure so a descriptor / layout mistake is identifiable."""
 import os
 import sys
