@@ -19,22 +19,26 @@ constexpr int kRedRows = 256;   // rows per block in column reductions
 // ---------------------------------------------------------------------------------------------
 // Column reductions over [n, C]: each thread owns VEC adjacent channels and strides over rows.
 // F::eval(row, c0, out_a[VEC], out_b[VEC]) yields the two per-element quantities to be summed.
+// A row has C / VEC channel groups; blockIdx.y selects a slice of CV <= 256 of them (the last slice may hold fewer),
+// so any C works: a block covers kRedRows rows of one slice.
 // ---------------------------------------------------------------------------------------------
 template <int VEC, typename F>
-__global__ void __launch_bounds__(kRedThreads) k_col_reduce2(F f, int64_t n, int C, double* __restrict__ acc /*[2][C]*/) {
+__global__ void __launch_bounds__(kRedThreads) k_col_reduce2(F f, int64_t n, int C, int CV,
+                                                             double* __restrict__ acc /*[2][C]*/) {
   extern __shared__ float sred[];   // [RY][CV][2*VEC]
-  const int CV = C / VEC;
   const int RY = kRedThreads / CV;
+  const int g0 = blockIdx.y * CV;                      // first channel group of this slice
+  const int ncv = C / VEC - g0 < CV ? C / VEC - g0 : CV;
   const int tx = threadIdx.x % CV, ty = threadIdx.x / CV;
   float a[VEC], b[VEC];
 #pragma unroll
   for (int v = 0; v < VEC; ++v) a[v] = b[v] = 0.f;
   const int64_t r0 = (int64_t)blockIdx.x * kRedRows;
   const int64_t r1 = r0 + kRedRows < n ? r0 + kRedRows : n;
-  if (ty < RY) {
+  if (ty < RY && tx < ncv) {
     for (int64_t r = r0 + ty; r < r1; r += RY) {
       float va[VEC], vb[VEC];
-      f.eval(r, tx * VEC, va, vb);
+      f.eval(r, (g0 + tx) * VEC, va, vb);
 #pragma unroll
       for (int v = 0; v < VEC; ++v) {
         a[v] += va[v];
@@ -49,12 +53,12 @@ __global__ void __launch_bounds__(kRedThreads) k_col_reduce2(F f, int64_t n, int
     }
   }
   __syncthreads();
-  // first CV*VEC*2 threads (looped) sum over ty and publish
-  for (int i = threadIdx.x; i < CV * 2 * VEC; i += kRedThreads) {
+  // first ncv*VEC*2 threads (looped) sum over ty and publish
+  for (int i = threadIdx.x; i < ncv * 2 * VEC; i += kRedThreads) {
     int cx = i / (2 * VEC), w = i % (2 * VEC);
     float s = 0.f;
     for (int y = 0; y < RY; ++y) s += sred[((size_t)y * CV + cx) * 2 * VEC + w];
-    int which = w / VEC, c = cx * VEC + (w % VEC);
+    int which = w / VEC, c = (g0 + cx) * VEC + (w % VEC);
     if (F::kTwo || which == 0) atomicAdd(acc + (size_t)which * C + c, (double)s);
   }
 }
@@ -892,14 +896,36 @@ __global__ void k_s2d_bwd(const float* __restrict__ ddense, const uint64_t* __re
   Elem<T>::st(dx + i, v);
 }
 
+// What the last call of each launcher below launched (developer entry like scn_tc_debug_last_launch, for the tests'
+// coverage check), written on the host before the launches.  Records: BatchNorm forward, BatchNorm backward, column
+// sum, LeakyReLU / AddTable, AveragePooling; fields:
+//   path    BatchNorm: 2 two-launch, 4 four-launch; column sum: 1 k_col_sum_fused, 4 k_col_reduce2;
+//           LeakyReLU / AddTable: 0 leaky forward, 1 leaky backward, 2 add
+//   vec     VEC of the statistics / column reduction (0: none, eval-mode forward), or of the elementwise / pool kernel
+//   apply   BatchNorm apply form: 1 row-streaming, 2 element-indexed
+//   avec    VEC of the apply kernel
+//   grid    grid of the statistics / reduction kernel (x), or of the elementwise / pool kernel
+//   grid2   grid of the apply kernel
+//   slices  k_col_reduce2's channel slices (gridDim.y)
+//   colsum  BatchNorm backward: 0 no column sums of dx, 1 fused into the apply kernel, 2 a separate column-sum call
+enum { kEwBnFwd = 0, kEwBnBwd = 1, kEwColSum = 2, kEwElem = 3, kEwPool = 4, kEwRecords = 5, kEwFields = 8 };
+static int32_t g_ew_last_launch[kEwRecords][kEwFields] = {};
+void ew_record(int which, int path, int vec, int apply, int avec, int64_t grid, int64_t grid2, int slices, int colsum) {
+  const int32_t rec[kEwFields] = {path, vec, apply, avec, (int32_t)grid, (int32_t)grid2, slices, colsum};
+  for (int i = 0; i < kEwFields; ++i) g_ew_last_launch[which][i] = rec[i];
+}
+
+// rec: the launch record whose reduction fields (vec, grid, slices) this launch fills in
 template <int VEC, typename F>
-int launch_col_reduce(F f, int64_t n, int C, double* acc, cudaStream_t s) {
-  int CV = C / VEC;
-  if (CV > kRedThreads) return SCN_ERR_UNSUPPORTED;
-  int RY = kRedThreads / CV;
-  size_t smem = (size_t)RY * CV * 2 * VEC * sizeof(float);
-  unsigned g = (unsigned)((n + kRedRows - 1) / kRedRows);
-  k_col_reduce2<VEC, F><<<g, kRedThreads, smem, s>>>(f, n, C, acc);
+int launch_col_reduce(F f, int64_t n, int C, double* acc, cudaStream_t s, int32_t* rec) {
+  const int groups = C / VEC;
+  const int slices = (groups + kRedThreads - 1) / kRedThreads;
+  const int CV = (groups + slices - 1) / slices;        // <= 256 channel groups per block, slices as even as possible
+  const int RY = kRedThreads / CV;
+  const size_t smem = (size_t)RY * CV * 2 * VEC * sizeof(float);
+  const unsigned g = (unsigned)((n + kRedRows - 1) / kRedRows);
+  rec[1] = VEC; rec[4] = (int32_t)g; rec[6] = slices;
+  k_col_reduce2<VEC, F><<<dim3(g, (unsigned)slices), kRedThreads, smem, s>>>(f, n, C, CV, acc);
   SCN_LAUNCH_CHECK();
   return SCN_OK;
 }
@@ -908,8 +934,9 @@ template <typename T>
 int bn_forward_t(const T* x, int64_t n, int C, const float* gamma, const float* beta, float* rm, float* rv,
                  int training, float eps, float momentum, float leak, float* save_mean, float* save_invstd,
                  double* ws, T* out, cudaStream_t s) {
-  const bool vec = (C % 4) == 0;
+  const bool vec = (C % 4) == 0 && (((uintptr_t)x | (uintptr_t)out) % (4 * sizeof(T))) == 0;
   const bool vec8 = (C % 8) == 0 && (((uintptr_t)x | (uintptr_t)out) & 15) == 0;
+  int32_t* rec = g_ew_last_launch[kEwBnFwd];
   if (training && vec8 && C <= 2048 && n > 0) {
     double* zws = nullptr;
     const int rc = zero_scratch(s, &zws);
@@ -920,6 +947,7 @@ int bn_forward_t(const T* x, int64_t n, int C, const float* gamma, const float* 
     const unsigned ph = bn_next_phase(s, C, &zero_n);
     double* acc = zws + (ph ? kAcc1 : 0);
     double* other = zws + (ph ? 0 : kAcc1);
+    ew_record(kEwBnFwd, 2, 8, 1, 8, g, g, 0, 0);
     SCN_CUDA(scn_launch_pdl(k_bn_stats2<T>, dim3((unsigned)g), dim3(256), 0, s, x, n, C, acc));
     SCN_LAUNCH_CHECK();
     SCN_CUDA(scn_launch_pdl(k_bn_apply2<T>, dim3((unsigned)g), dim3(256), 0, s, x, n, C, gamma, beta, rm, rv, eps, momentum, leak,
@@ -927,12 +955,13 @@ int bn_forward_t(const T* x, int64_t n, int C, const float* gamma, const float* 
     SCN_LAUNCH_CHECK();
     return SCN_OK;
   }
+  ew_record(kEwBnFwd, 4, 0, 0, 0, 0, 0, 0, 0);
   if (training) {
     SCN_CUDA(cudaMemsetAsync(ws, 0, 2 * (size_t)C * sizeof(double), s));
     if (n > 0) {
-      int rc = vec8 ? launch_col_reduce<8>(StatsF<T, 8>{x, C}, n, C, ws, s)
-               : vec ? launch_col_reduce<4>(StatsF<T, 4>{x, C}, n, C, ws, s)
-                     : launch_col_reduce<1>(StatsF<T, 1>{x, C}, n, C, ws, s);
+      int rc = vec8 ? launch_col_reduce<8>(StatsF<T, 8>{x, C}, n, C, ws, s, rec)
+               : vec ? launch_col_reduce<4>(StatsF<T, 4>{x, C}, n, C, ws, s, rec)
+                     : launch_col_reduce<1>(StatsF<T, 1>{x, C}, n, C, ws, s, rec);
       if (rc) return rc;
     }
   }
@@ -946,12 +975,16 @@ int bn_forward_t(const T* x, int64_t n, int C, const float* gamma, const float* 
     int64_t g = (n + (int64_t)ry * 4 - 1) / ((int64_t)ry * 4);      // >= 4 rows per thread
     if (g > (int64_t)kNumSMs * 8) g = (int64_t)kNumSMs * 8;
     if (g < 1) g = 1;
+    rec[2] = 1; rec[3] = 8; rec[5] = (int32_t)g;
     k_bn_apply_rows<T><<<(unsigned)g, 256, 0, s>>>(x, n, C, save_mean, save_invstd, gamma, beta, leak, out);
-  } else if (vec)
+  } else if (vec) {
+    rec[2] = 2; rec[3] = 4; rec[5] = (int32_t)grid_for(total / 4, 256);
     k_bn_apply<T, 4><<<grid_for(total / 4, 256), 256, 0, s>>>(x, total / 4, C, save_mean, save_invstd, gamma, beta,
                                                               leak, out);
-  else
+  } else {
+    rec[2] = 2; rec[3] = 1; rec[5] = (int32_t)grid_for(total, 256);
     k_bn_apply<T, 1><<<grid_for(total, 256), 256, 0, s>>>(x, total, C, save_mean, save_invstd, gamma, beta, leak, out);
+  }
   SCN_LAUNCH_CHECK();
   return SCN_OK;
 }
@@ -960,8 +993,9 @@ template <typename T>
 int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamma, const float* beta,
                   const float* mean, const float* invstd, int training, float leak, double* ws, T* dx,
                   float* dgamma, float* dbeta, int accumulate, float* colsum, cudaStream_t s) {
-  const bool vec = (C % 4) == 0;
+  const bool vec = (C % 4) == 0 && (((uintptr_t)x | (uintptr_t)dout | (uintptr_t)dx) % (4 * sizeof(T))) == 0;
   const bool vec8 = (C % 8) == 0 && (((uintptr_t)x | (uintptr_t)dout | (uintptr_t)dx) & 15) == 0;
+  int32_t* rec = g_ew_last_launch[kEwBnBwd];
   if (training && vec8 && C <= 2048 && n > 0) {
     double* zws = nullptr;
     const int rc = zero_scratch(s, &zws);
@@ -973,6 +1007,7 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
     double* other = zws + (ph ? 0 : kAcc1);
     double* colacc = zws + 2 * 2048;                                   // shared with k_col_sum_fused (stream-ordered)
     unsigned* ticket = reinterpret_cast<unsigned*>(zws + 3 * 2048 + 1);
+    ew_record(kEwBnBwd, 2, 8, 1, 8, bn_grid2(n, ry, 3), bn_grid2(n, ry, colsum ? 3 : 4), 0, colsum ? 1 : 0);
     SCN_CUDA(scn_launch_pdl(k_bn_bwd_stats2<T>, dim3((unsigned)bn_grid2(n, ry, 3)), dim3(256), 0, s, x, dout, n, C, mean, invstd,
                             gamma, beta, leak, acc));
     SCN_LAUNCH_CHECK();
@@ -987,11 +1022,12 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
     SCN_LAUNCH_CHECK();
     return SCN_OK;
   }
+  ew_record(kEwBnBwd, 4, 0, 0, 0, 0, 0, 0, colsum ? 2 : 0);
   SCN_CUDA(cudaMemsetAsync(ws, 0, 2 * (size_t)C * sizeof(double), s));
   if (n > 0) {
-    int rc = vec8 ? launch_col_reduce<8>(BnBwdF<T, 8>{x, dout, mean, invstd, gamma, beta, leak, C}, n, C, ws, s)
-             : vec ? launch_col_reduce<4>(BnBwdF<T, 4>{x, dout, mean, invstd, gamma, beta, leak, C}, n, C, ws, s)
-                   : launch_col_reduce<1>(BnBwdF<T, 1>{x, dout, mean, invstd, gamma, beta, leak, C}, n, C, ws, s);
+    int rc = vec8 ? launch_col_reduce<8>(BnBwdF<T, 8>{x, dout, mean, invstd, gamma, beta, leak, C}, n, C, ws, s, rec)
+             : vec ? launch_col_reduce<4>(BnBwdF<T, 4>{x, dout, mean, invstd, gamma, beta, leak, C}, n, C, ws, s, rec)
+                   : launch_col_reduce<1>(BnBwdF<T, 1>{x, dout, mean, invstd, gamma, beta, leak, C}, n, C, ws, s, rec);
     if (rc) return rc;
   }
   k_acc_to_float<<<grid_for(C, 128), 128, 0, s>>>(ws, C, dgamma, dbeta, accumulate);
@@ -1006,13 +1042,17 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
     int64_t g = (n + (int64_t)ry * 4 - 1) / ((int64_t)ry * 4);
     if (g > (int64_t)kNumSMs * 8) g = (int64_t)kNumSMs * 8;
     if (g < 1) g = 1;
+    rec[2] = 1; rec[3] = 8; rec[5] = (int32_t)g;
     k_bn_bwd_apply_rows<T><<<(unsigned)g, 256, 0, s>>>(x, dout, n, C, mean, invstd, gamma, beta, leak, training, ws, dx);
-  } else if (vec)
+  } else if (vec) {
+    rec[2] = 2; rec[3] = 4; rec[5] = (int32_t)grid_for(total / 4, 256);
     k_bn_bwd_apply<T, 4><<<grid_for(total / 4, 256), 256, 0, s>>>(x, dout, total / 4, C, n, mean, invstd, gamma, beta,
                                                                   leak, training, ws, dx);
-  else
+  } else {
+    rec[2] = 2; rec[3] = 1; rec[5] = (int32_t)grid_for(total, 256);
     k_bn_bwd_apply<T, 1><<<grid_for(total, 256), 256, 0, s>>>(x, dout, total, C, n, mean, invstd, gamma, beta, leak,
                                                               training, ws, dx);
+  }
   SCN_LAUNCH_CHECK();
   if (colsum)      // paths without the fused column sums: one more pass over dx
     return scn_col_sum(dx, std::is_same<T, float>::value ? SCN_F32 : SCN_BF16, n, C, ws, colsum, s);
@@ -1033,6 +1073,7 @@ int ew_launch3(int which, const T* a, const T* b, int64_t count, float leak, T* 
   if (vec && count % 8 == 0) {                 // 16-byte accesses for bf16, 2 x 16 bytes for fp32
     const int64_t n8 = count / 8;
     const unsigned g8 = grid_for(n8, 256);
+    ew_record(kEwElem, which, 8, 0, 0, g8, 0, 0, 0);
     if (which == 0) SCN_CUDA(scn_launch_pdl(k_leaky_fwd<T, 8>, dim3(g8), dim3(256), 0, s, a, n8, leak, out));
     else if (which == 1) SCN_CUDA(scn_launch_pdl(k_leaky_bwd<T, 8>, dim3(g8), dim3(256), 0, s, a, b, n8, leak, out));
     else SCN_CUDA(scn_launch_pdl(k_add_fwd<T, 8>, dim3(g8), dim3(256), 0, s, a, b, n8, leak, out));
@@ -1041,6 +1082,7 @@ int ew_launch3(int which, const T* a, const T* b, int64_t count, float leak, T* 
   }
   int64_t nv = vec ? count / 4 : count;
   unsigned g = grid_for(nv, 256);
+  ew_record(kEwElem, which, vec ? 4 : 1, 0, 0, g, 0, 0, 0);
   if (which == 0) {
     if (vec) k_leaky_fwd<T, 4><<<g, 256, 0, s>>>(a, nv, leak, out); else k_leaky_fwd<T, 1><<<g, 256, 0, s>>>(a, nv, leak, out);
   } else if (which == 1) {
@@ -1053,6 +1095,11 @@ int ew_launch3(int which, const T* a, const T* b, int64_t count, float leak, T* 
 }
 
 }  // namespace
+
+extern "C" void scn_ew_debug_last_launch(int32_t* out) {
+  for (int r = 0; r < kEwRecords; ++r)
+    for (int i = 0; i < kEwFields; ++i) out[r * kEwFields + i] = g_ew_last_launch[r][i];
+}
 
 extern "C" int scn_bn_forward(const void* x, int dtype, int64_t n, int C, const float* gamma, const float* beta,
                               float* running_mean, float* running_var, int training, float eps, float momentum,
@@ -1112,6 +1159,7 @@ extern "C" int scn_col_sum_acc(const void* x, int dtype, int64_t n, int C, doubl
     if (g > (int64_t)kNumSMs * 4) g = (int64_t)kNumSMs * 4;
     if (g < 1) g = 1;
     const size_t smem = (size_t)ry * (C >> 3) * 8 * sizeof(float);
+    ew_record(kEwColSum, 1, 8, 0, 0, g, 0, 0, 0);
     if (dtype == SCN_F32)
       SCN_CUDA(scn_launch_pdl(k_col_sum_fused<float>, dim3((unsigned)g), dim3(256), smem, s, (const float*)x, n, C, acc1, ticket, out, accumulate));
     else if (dtype == SCN_BF16)
@@ -1123,16 +1171,19 @@ extern "C" int scn_col_sum_acc(const void* x, int dtype, int64_t n, int C, doubl
     return SCN_OK;
   }
   double* acc = stats_ws;
+  ew_record(kEwColSum, 4, 0, 0, 0, 0, 0, 0, 0);
+  int32_t* rec = g_ew_last_launch[kEwColSum];
   SCN_CUDA(cudaMemsetAsync(acc, 0, 2 * (size_t)C * sizeof(double), s));
   int rc = SCN_OK;
   if (n > 0) {
-    const bool vec = (C % 4) == 0;
+    const size_t esz = dtype == SCN_F32 ? sizeof(float) : sizeof(__nv_bfloat16);
+    const bool vec = (C % 4) == 0 && ((uintptr_t)x % (4 * esz)) == 0;
     if (dtype == SCN_F32)
-      rc = vec ? launch_col_reduce<4>(SumF<float, 4>{(const float*)x, C}, n, C, acc, s)
-               : launch_col_reduce<1>(SumF<float, 1>{(const float*)x, C}, n, C, acc, s);
+      rc = vec ? launch_col_reduce<4>(SumF<float, 4>{(const float*)x, C}, n, C, acc, s, rec)
+               : launch_col_reduce<1>(SumF<float, 1>{(const float*)x, C}, n, C, acc, s, rec);
     else if (dtype == SCN_BF16)
-      rc = vec ? launch_col_reduce<4>(SumF<__nv_bfloat16, 4>{(const __nv_bfloat16*)x, C}, n, C, acc, s)
-               : launch_col_reduce<1>(SumF<__nv_bfloat16, 1>{(const __nv_bfloat16*)x, C}, n, C, acc, s);
+      rc = vec ? launch_col_reduce<4>(SumF<__nv_bfloat16, 4>{(const __nv_bfloat16*)x, C}, n, C, acc, s, rec)
+               : launch_col_reduce<1>(SumF<__nv_bfloat16, 1>{(const __nv_bfloat16*)x, C}, n, C, acc, s, rec);
     else
       rc = SCN_ERR_ARG;
   }
@@ -1230,6 +1281,7 @@ static int launch_pool_rows(const void* x, int ldx, const int32_t* nbr, int K, i
                             float scale, void* out, cudaStream_t s) {
   const size_t vb = 4 * sizeof(T);      // bytes of one 4-element access
   const bool vec = C % 4 == 0 && ldx % 4 == 0 && (uintptr_t)x % vb == 0 && (uintptr_t)out % vb == 0;
+  ew_record(kEwPool, 0, vec ? 4 : 1, 0, 0, vec ? grid_for(n_rows * (C / 4), 256) : grid_for(n_rows * C, 256), 0, 0, 0);
   if (vec)
     k_pool_rows<T, 4><<<grid_for(n_rows * (C / 4), 256), 256, 0, s>>>((const T*)x, ldx, nbr, K, n_rows, n_pad, C, scale,
                                                                        (T*)out);
