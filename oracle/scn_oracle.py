@@ -43,27 +43,26 @@ def as_triple(v, dimension: int = 3) -> Tuple[int, ...]:
 
 
 def pack_keys(coords: np.ndarray) -> np.ndarray:
-    """(x0..x_{D-1}, batch) int rows -> one int64 key (batch | x0 | x1 | x2), 16 bits each.
+    """(x0..x_{D-1}, batch) int rows -> one uint64 key (batch | x0 | x1 | x2), 16 bits each.
 
-    Lexicographic order of (batch, x0, x1, x2) == numeric order of the key.
+    Lexicographic order of (batch, x0, x1, x2) == numeric order of the key.  The key is unsigned, as on the device:
+    batch indices 32768..65534 set the top bit and must still sort after batch 0.
     """
-    coords = np.asarray(coords, dtype=np.int64)
+    coords = np.asarray(coords, dtype=np.int64).astype(np.uint64)
     d = coords.shape[1] - 1
-    key = coords[:, d].astype(np.int64)
+    key = coords[:, d]
     for a in range(3):
-        key = key << 16
+        key = key << np.uint64(16)
         if a < d:
             key = key | coords[:, a]
     return key
 
 
 def unpack_keys(keys: np.ndarray, dimension: int = 3) -> np.ndarray:
-    keys = np.asarray(keys, dtype=np.int64)
-    cols = []
-    for a in range(3):
-        cols.append((keys >> (16 * (2 - a))) & 0xFFFF)
-    b = keys >> 48
-    return np.stack(cols[:dimension] + [b], axis=1)
+    """uint64 (or int64 bit pattern) keys -> int64 rows (x0..x_{D-1}, batch)."""
+    keys = np.asarray(keys).astype(np.uint64)
+    field = [((keys >> np.uint64(s)) & np.uint64(0xFFFF)).astype(np.int64) for s in (32, 16, 0, 48)]
+    return np.stack(field[:dimension] + [field[3]], axis=1)
 
 
 # ----------------------------------------------------------------------------

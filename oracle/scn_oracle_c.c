@@ -43,8 +43,11 @@ static void map_put(Map* m, int64_t key, int32_t row) {
   m->head[b] = (int32_t)m->n++;
 }
 
-/* (x0, x1, x2, batch) -> batch:16 | x0:16 | x1:16 | x2:16 ; lexicographic (batch, x0, x1, x2) == numeric order */
-static int64_t pack(const int64_t* c) { return (c[3] << 48) | (c[0] << 32) | (c[1] << 16) | c[2]; }
+/* (x0, x1, x2, batch) -> batch:16 | x0:16 | x1:16 | x2:16 ; lexicographic (batch, x0, x1, x2) == numeric order of the
+ * UNSIGNED key (batch indices >= 32768 set the top bit) */
+static uint64_t pack(const int64_t* c) {
+  return ((uint64_t)c[3] << 48) | ((uint64_t)c[0] << 32) | ((uint64_t)c[1] << 16) | (uint64_t)c[2];
+}
 
 /* InputLayer: coords int64 [n][4] (batch LAST).  Writes row_of_input[n], active[n_active][4]; returns n_active. */
 int64_t oc_input_rules(const int64_t* coords, int64_t n, int64_t* row_of_input, int64_t* active) {
@@ -91,8 +94,8 @@ int oc_subm_rules(const int64_t* coords, int64_t n, int f0, int f1, int f2, int3
   return 0;
 }
 
-static int cmp_i64(const void* a, const void* b) {
-  int64_t x = *(const int64_t*)a, y = *(const int64_t*)b;
+static int cmp_u64(const void* a, const void* b) {
+  uint64_t x = *(const uint64_t*)a, y = *(const uint64_t*)b;
   return x < y ? -1 : (x > y ? 1 : 0);
 }
 
@@ -101,7 +104,7 @@ static int cmp_i64(const void* a, const void* b) {
  * Writes out_coords[n_out][4] (capacity n), out_row_of_in[n], off_of_in[n]; returns n_out. */
 int64_t oc_strided_rules(const int64_t* coords, int64_t n, int s0, int s1, int s2, int64_t* out_coords,
                          int32_t* out_row_of_in, int32_t* off_of_in) {
-  int64_t* keys = (int64_t*)calloc((size_t)(n > 0 ? n : 1), sizeof(int64_t));
+  uint64_t* keys = (uint64_t*)calloc((size_t)(n > 0 ? n : 1), sizeof(uint64_t));
   if (!keys) return -1;
   const int s[3] = {s0, s1, s2};
   for (int64_t i = 0; i < n; ++i) {
@@ -115,15 +118,15 @@ int64_t oc_strided_rules(const int64_t* coords, int64_t n, int s0, int s1, int s
     keys[i] = pack(q);
     off_of_in[i] = k;
   }
-  int64_t* sorted = (int64_t*)malloc(sizeof(int64_t) * (size_t)(n > 0 ? n : 1));
+  uint64_t* sorted = (uint64_t*)malloc(sizeof(uint64_t) * (size_t)(n > 0 ? n : 1));
   if (!sorted) { free(keys); return -1; }
-  memcpy(sorted, keys, sizeof(int64_t) * (size_t)n);
-  qsort(sorted, (size_t)n, sizeof(int64_t), cmp_i64);
+  memcpy(sorted, keys, sizeof(uint64_t) * (size_t)n);
+  qsort(sorted, (size_t)n, sizeof(uint64_t), cmp_u64);
   int64_t m = 0;
   for (int64_t i = 0; i < n; ++i)
     if (i == 0 || sorted[i] != sorted[i - 1]) sorted[m++] = sorted[i];
   for (int64_t r = 0; r < m; ++r) {
-    out_coords[4 * r + 3] = sorted[r] >> 48;
+    out_coords[4 * r + 3] = (int64_t)(sorted[r] >> 48);
     out_coords[4 * r + 0] = (sorted[r] >> 32) & 0xFFFF;
     out_coords[4 * r + 1] = (sorted[r] >> 16) & 0xFFFF;
     out_coords[4 * r + 2] = sorted[r] & 0xFFFF;

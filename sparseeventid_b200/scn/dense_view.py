@@ -91,7 +91,8 @@ class SparseDenseTensor(torch.Tensor):
 
     def _batch_index(self):
         if self._batch_of_row is None:
-            self._batch_of_row = (self._keys >> 48).to(torch.int32).contiguous()
+            # keys are int64 and the shift is arithmetic: mask so that batch indices >= 32768 stay non-negative
+            self._batch_of_row = ((self._keys >> 48) & 0xFFFF).to(torch.int32).contiguous()
         return self._batch_of_row
 
     def _full_extent(self, nd, kernel_size, stride, padding, ceil_mode, count_include_pad, divisor_override):

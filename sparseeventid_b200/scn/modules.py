@@ -428,7 +428,7 @@ class SparseGroupNorm(nn.Module):
         n, c = x.shape
         assert c == self.num_channels
         g, cg = self.num_groups, c // self.num_groups
-        b = (md.levels[input._sp()].keys >> 48).long()                        # sample of every active row
+        b = ((md.levels[input._sp()].keys >> 48) & 0xFFFF).long()             # sample of every active row (int64 keys)
         nb = max(int(md.batch_size), 1)
         xf = x.float().view(n, g, cg)
         cnt = torch.zeros(nb, device=x.device).index_add_(0, b, torch.ones(n, device=x.device)).clamp_min(1.0) * cg

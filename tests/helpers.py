@@ -40,12 +40,15 @@ def blob_sites(n, grid, batch, seed):
 BENCH_BATCH, BENCH_SEED = 64, 1234
 
 
-def bench_batch(batch=BENCH_BATCH, seed=BENCH_SEED):
-    """The benchmark's first batch (64 synthetic dune3d events, ~5e5 active sites): float64 coordinates, float32 features,
-    batch size."""
+def bench_batch(batch=BENCH_BATCH, seed=BENCH_SEED, dataset="dune3d"):
+    """The benchmark's first batch (64 synthetic events: ~5e5 active sites for dune3d, ~9e5 over three planes for
+    dune2d), as bench.host_batch builds it: float64 coordinates, float32 features, batch size."""
     from sparseeventid_b200 import synthetic
-    from sparseeventid_b200.data_transforms import larcvsparse_to_scnsparse_3d
-    c, f, bs = larcvsparse_to_scnsparse_3d(synthetic.larcv_batch_3d(batch, seed=seed))
+    from sparseeventid_b200.data_transforms import larcvsparse_to_scnsparse_2d, larcvsparse_to_scnsparse_3d
+    if dataset == "dune3d":
+        c, f, bs = larcvsparse_to_scnsparse_3d(synthetic.larcv_batch_3d(batch, seed=seed))
+    else:
+        c, f, bs = larcvsparse_to_scnsparse_2d(synthetic.larcv_batch_2d(batch, seed=seed))
     return np.ascontiguousarray(c, dtype=np.float64), np.ascontiguousarray(f, dtype=np.float32), bs
 
 

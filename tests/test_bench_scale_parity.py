@@ -40,36 +40,32 @@ def rules_to_table(rules, n_out):
     return t
 
 
-@pytest.mark.gpu
-def test_bench_batch_rulebooks_bit_exact():
-    import sparseconvnet as scn
-    coords, feats, bs = bench_batch()
-    ci = coords.astype(np.int64)
-    assert np.unique(O.pack_keys(ci)).shape[0] == ci.shape[0], "the synthetic batch has no duplicate sites"
-    x = scn.InputLayer(3, list(synthetic.GRID_3D))((torch.as_tensor(coords).cuda(), torch.as_tensor(feats).cuda(), bs))
-    md = x.metadata
-    sp = tuple(synthetic.GRID_3D)
+def to_oracle(table, rows_map, vals_map):
+    """GPU table [K, n] (rows / entries in GPU numbering) -> the same table in the oracle's numbering."""
+    out = np.full_like(table, -1)
+    out[:, rows_map] = np.where(table >= 0, vals_map[np.maximum(table, 0)], -1)
+    return out
+
+
+def check_level_rulebooks(md, ci, sp, stem, filt, stride, levels=6):
+    """The tables of `levels` resolution levels of an InputLayer's metadata `md` on the duplicate-free sites `ci` (int64
+    [n, 4], input order) at grid `sp`: the `stem` filter on level 0, `filt` on every level and the `stride` maps between
+    them with their transposes, bit-exact against the oracle rulebooks.  Returns the oracle sites of the deepest level."""
+    assert np.unique(O.pack_keys(ci)).shape[0] == ci.shape[0], "the batch has no duplicate sites"
     assert np.array_equal(md.coords(sp).cpu().numpy(), ci)               # level 0 rows == input order
     cur = ci                                     # oracle rows of the level
     gmap = np.arange(ci.shape[0])                # GPU row -> oracle row (level 0: identical numbering)
-
-    def to_oracle(table, rows_map, vals_map):
-        """GPU table [K, n] (rows / entries in GPU numbering) -> the same table in the oracle's numbering."""
-        out = np.full_like(table, -1)
-        out[:, rows_map] = np.where(table >= 0, vals_map[np.maximum(table, 0)], -1)
-        return out
-
-    for level in range(6):
+    for level in range(levels):
         n = cur.shape[0]
-        for filt in ([(5, 5, 5)] if level == 0 else []) + [(3, 3, 3)]:
-            got = md.subm_table(sp, filt)[:, :n].cpu().numpy().astype(np.int64)
-            want = rules_to_table(O.submanifold_rulebook(cur, filt), n)
-            assert np.array_equal(to_oracle(got, gmap, gmap), want), f"level {level} filter {filt}: neighbour table differs from the oracle rulebook"
-            assert bool((md.subm_table(sp, filt)[:, n:] == -1).all())
-        if level == 5:
+        for f in ([stem] if level == 0 else []) + [filt]:
+            got = md.subm_table(sp, f)[:, :n].cpu().numpy().astype(np.int64)
+            want = rules_to_table(O.submanifold_rulebook(cur, f), n)
+            assert np.array_equal(to_oracle(got, gmap, gmap), want), f"level {level} filter {f}: neighbour table differs from the oracle rulebook"
+            assert bool((md.subm_table(sp, f)[:, n:] == -1).all())
+        if level == levels - 1:
             break
-        rule = md.strided_rule(sp, (2, 2, 2), (2, 2, 2))
-        out_coords, rules, out_sp = O.strided_rulebook(cur, (2, 2, 2), (2, 2, 2), sp)
+        rule = md.strided_rule(sp, stride, stride)
+        out_coords, rules, out_sp = O.strided_rulebook(cur, stride, stride, sp)
         assert rule.out_spatial == out_sp and rule.n_out == out_coords.shape[0]
         # same output sites; the GPU numbers them in first-appearance order, the oracle by ascending key
         gloc = md.coords(out_sp).cpu().numpy()
@@ -77,11 +73,21 @@ def test_bench_batch_rulebooks_bit_exact():
         assert np.array_equal(np.sort(gkeys), okeys)
         gmap_next = np.searchsorted(okeys, gkeys)
         down = rule.down[:, :rule.n_out].cpu().numpy().astype(np.int64)
-        assert np.array_equal(to_oracle(down, gmap_next, gmap), rules_to_table(rules, rule.n_out)), f"level {level}: stride-2 map differs"
+        assert np.array_equal(to_oracle(down, gmap_next, gmap), rules_to_table(rules, rule.n_out)), f"level {level}: {stride} map differs"
         up = rule.up[:, :n].cpu().numpy().astype(np.int64)
         want_up = rules_to_table([r[:, ::-1] for r in rules], n)
-        assert np.array_equal(to_oracle(up, gmap, gmap_next), want_up), f"level {level}: transposed stride-2 map differs"
+        assert np.array_equal(to_oracle(up, gmap, gmap_next), want_up), f"level {level}: transposed {stride} map differs"
         cur, sp, gmap = out_coords, out_sp, gmap_next
+    return cur
+
+
+@pytest.mark.gpu
+def test_bench_batch_rulebooks_bit_exact():
+    import sparseconvnet as scn
+    coords, feats, bs = bench_batch()
+    ci = coords.astype(np.int64)
+    x = scn.InputLayer(3, list(synthetic.GRID_3D))((torch.as_tensor(coords).cuda(), torch.as_tensor(feats).cuda(), bs))
+    cur = check_level_rulebooks(x.metadata, ci, tuple(synthetic.GRID_3D), (5, 5, 5), (3, 3, 3), (2, 2, 2))
     assert cur.shape[0] > 1000
 
 

@@ -58,3 +58,28 @@ def test_reference_head_path_matches_dense_and_backpropagates():
     z = torch.tanh(x)
     assert isinstance(z, SparseDenseTensor)
     assert torch.allclose(z.dense(), torch.tanh(_dense(feats, coords, grid, batch)))
+
+
+def test_batch_indices_above_32767_decode_unsigned():
+    """The batch field is the top 16 bits of an int64 key: batch 32768..65534 makes the key negative, and the row's
+    sample must still come out as that index (not index - 65536) on the pooled head path."""
+    grid, c, batch = (2, 2, 3), 3, 65535
+    coords = torch.as_tensor(random_sites(30, grid, 3, seed=5))
+    coords[:, 3] = torch.tensor([32767, 32768, 65534])[coords[:, 3]]
+    feats = torch.randn(coords.shape[0], c, requires_grad=True)
+    keys = (coords[:, 3] << 48) | (coords[:, 0] << 32) | (coords[:, 1] << 16) | coords[:, 2]
+    assert bool((keys[coords[:, 3] >= 32768] < 0).all())
+
+    def pooled(f, b_of_row, nb, vol):
+        return torch.zeros(nb, f.shape[1]).index_add(0, b_of_row.long(), f) / vol
+    x = SparseDenseTensor(feats, keys, batch, grid, lambda f: _dense(f, coords, grid, batch), pooled)
+    assert torch.equal(x._batch_index().long(), coords[:, 3])
+    y = F.avg_pool3d(torch.tanh(x), list(grid))
+    assert x._dense is None
+    feats2 = feats.detach().clone().requires_grad_(True)
+    y_ref = F.avg_pool3d(_dense(torch.tanh(feats2), coords, grid, batch), list(grid))
+    assert torch.allclose(y, y_ref, atol=1e-6)
+    w = torch.randn(y.shape)
+    (y * w).sum().backward()
+    (y_ref * w).sum().backward()
+    assert torch.allclose(feats.grad, feats2.grad, atol=1e-6)

@@ -741,7 +741,7 @@ def test_sparse_to_dense(dtype):
     outside = np.array([[6, 0, 0, 0], [0, 5, 0, 1], [0, 0, 7, 2], [1, 1, 1, 3], [5, 4, 6, 7], [6, 5, 7, 3]], dtype=np.int64)
     coords = np.concatenate([inside, outside])
     coords = coords[np.random.default_rng(1).permutation(coords.shape[0])]
-    keys = torch.as_tensor(O.pack_keys(coords)).cuda()
+    keys = torch.as_tensor(O.pack_keys(coords).view(np.int64)).cuda()
     g = torch.Generator(device="cuda").manual_seed(5)
     n = coords.shape[0]
     x = torch.randn(n, C, device="cuda", generator=g).to(dtype)

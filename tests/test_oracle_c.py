@@ -40,14 +40,20 @@ def test_submanifold_rulebook(filt, kind, seed):
         assert np.array_equal(a, b)
 
 
-@pytest.mark.parametrize("stride,grid", [((2, 2, 2), (20, 16, 24)), ((1, 2, 2), (3, 16, 24))])
-def test_strided_rulebook(stride, grid):
+@pytest.mark.parametrize("stride,grid,batch0", [((2, 2, 2), (20, 16, 24), 0), ((1, 2, 2), (3, 16, 24), 0),
+                                                ((2, 2, 2), (20, 16, 24), 32767), ((1, 2, 2), (3, 16, 24), 32767)],
+                         ids=["stride0-grid0", "stride1-grid1", "stride0-grid0-batch32767", "stride1-grid1-batch32767"])
+def test_strided_rulebook(stride, grid, batch0):
+    """batch0 = 32767: the samples 32767 and 32768 straddle the top bit of the packed key, whose order is unsigned."""
     rng = np.random.default_rng(8)
-    pts = np.unique(np.stack([rng.integers(0, grid[a], 500) for a in range(3)] + [rng.integers(0, 2, 500)], 1), axis=0)
+    b = batch0 + rng.integers(0, 2, 500)
+    pts = np.unique(np.stack([rng.integers(0, grid[a], 500) for a in range(3)] + [b], 1), axis=0)
     _, active = O.input_layer_rules(pts.astype(np.int64))
     out_py, rules_py, _ = O.strided_rulebook(active, stride, stride, grid)
     out_c, rules_c = OC.strided_rules(active, stride)
-    assert np.array_equal(out_py, out_c)
+    k = O.pack_keys(out_py)
+    assert np.array_equal(out_py, out_c) and np.all(k[1:] > k[:-1])
+    assert np.array_equal(np.unique(out_py[:, 3]), np.unique(active[:, 3]))
     for a, b in zip(O.normalize_rulebook(rules_c, active, out_c), O.normalize_rulebook(rules_py, active, out_py)):
         assert np.array_equal(a, b)
 
