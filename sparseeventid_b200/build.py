@@ -1,6 +1,7 @@
 """In-tree build of libscn_b200.so (hand-written CUDA for sm_100a, C ABI in include/scn_b200.h).
 
-``python -m sparseeventid_b200.build`` or ``build()``; nvcc cross-compiles without a GPU.
+``python -m sparseeventid_b200.build`` builds it and the thin PyTorch C++ layer (build_torch_ext below); ``build()``
+builds the library alone.  nvcc cross-compiles without a GPU.
 The .so stays in the tree (git-ignored) so it travels to the GPU box with the snapshot.
 """
 from __future__ import annotations
@@ -93,5 +94,4 @@ def build_torch_ext(verbose: bool = False) -> str:
 
 if __name__ == "__main__":
     print(build(force="--force" in sys.argv, verbose=True))
-    if "--torch" in sys.argv:
-        print(build_torch_ext(verbose=True))
+    print(build_torch_ext(verbose=True))

@@ -38,7 +38,6 @@
 //
 // Replaces SCN's dConvolution_KMxKN_forwardA/B (SURVEY.md 2.2); reference call sites
 // src/networks/sparse_building_blocks.py:29-34,110-117.
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -717,14 +716,9 @@ int scn_tc_prep(const float* W, int K, int Cin, int Cout, int transpose, int mir
   return SCN_OK;
 }
 
-// developer knobs for sweeps (read once): SCN_B200_TC_GRID caps the CTAs, SCN_B200_TC_T forces the tiles per group,
-// SCN_B200_TC_SA / SCN_B200_TC_SB force the A / B ring depths
-static int env_int(const char* name) {
-  const char* e = std::getenv(name);
-  return e ? std::atoi(e) : 0;
-}
-static int g_knob[4] = {-1, -1, -1, -1};      // grid, T, SA, SB: -1 = read the environment on first use
-// developer entry for the sweep tools (like scn_tc_debug_timeline: not part of the product ABI): 0 = automatic
+// developer knobs for sweeps: a cap on the CTAs, forced tiles per group, forced A / B ring depths; 0 = automatic
+static int g_knob[4] = {0, 0, 0, 0};          // grid, T, SA, SB
+// developer entry for the sweep tools (like scn_tc_debug_timeline: not part of the product ABI)
 extern "C" void scn_tc_debug_knobs(int grid, int t, int sa, int sb) {
   g_knob[0] = grid; g_knob[1] = t; g_knob[2] = sa; g_knob[3] = sb;
 }
@@ -740,10 +734,6 @@ int scn_tc_forward(const void* in, int64_t n_in_rows, const int32_t* nbr, int K,
                    int n_out, const void* bimg, const float* bias, void* out, int tf32, cudaStream_t s) {
   const uint64_t row_units = (uint64_t)n_in * (tf32 ? 4u : 2u) / 16u;                // 16-byte units per input row
   if ((uint64_t)n_in_rows * row_units >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;   // 32-bit offsets in 16-byte units (64 GB)
-  if (g_knob[0] < 0) {
-    g_knob[0] = env_int("SCN_B200_TC_GRID"); g_knob[1] = env_int("SCN_B200_TC_T");
-    g_knob[2] = env_int("SCN_B200_TC_SA"); g_knob[3] = env_int("SCN_B200_TC_SB");
-  }
   const int force_grid = g_knob[0], force_t = g_knob[1], force_sa = g_knob[2], force_sb = g_knob[3];
   tc::Params p;
   p.dbg = g_tc_dbg;

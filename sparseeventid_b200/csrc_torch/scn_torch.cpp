@@ -2,8 +2,9 @@
 // (convolutions, BatchNormalization(+leaky), AddTable+LeakyReLU, LeakyReLU) as torch::autograd::Function, so that a
 // module forward/backward costs one native call instead of a Python autograd.Function round trip.  No arithmetic
 // here: torch supplies device memory, the current stream and the autograd tape; every kernel is in libscn_b200.so.
-// Mirrors sparseeventid_b200/scn/functional.py (the Python functions remain the readable reference and are used
-// when this extension is not built).  SCN counterpart: the pybind11 module `sparseconvnet.SCN` (SURVEY.md 8b).
+// Required: the modules (scn/modules.py::_native) run these outside ops.Profiler and for contiguous fp32 parameters;
+// scn/functional.py holds the per-kernel functions for the rest.  SCN counterpart: the pybind11 module
+// `sparseconvnet.SCN` (SURVEY.md 8b).
 #include <c10/cuda/CUDAStream.h>
 #include <torch/extension.h>
 

@@ -1,7 +1,7 @@
 """B200-native implementation of the ``sparseconvnet`` module surface (see modules.py)."""
-from .config import feature_dtype, get_precision, set_fusion, set_precision
-from .core import Metadata, SparseConvNetTensor, prefetch, set_rulebook_stream
-from .dense_view import SparseDenseTensor, set_lazy_dense
+from .config import feature_dtype, get_precision, set_precision
+from .core import Metadata, SparseConvNetTensor, prefetch
+from .dense_view import SparseDenseTensor
 from .functional import prepare_weight_images, release_weight_images
 from .modules import (AddTable, AveragePooling, BatchNormalization, BatchNormLeakyReLU, BatchNormReLU, Convolution, Deconvolution,
                       Identity, InputLayer, LeakyReLU, OutputLayer, ReLU, Sequential, Sigmoid, SparseGroupNorm, SparseToDense,
@@ -11,5 +11,5 @@ __all__ = [
     "AddTable", "AveragePooling", "BatchNormalization", "BatchNormLeakyReLU", "BatchNormReLU", "Convolution", "Deconvolution",
     "Identity", "InputLayer", "LeakyReLU", "OutputLayer", "ReLU", "Sequential", "Sigmoid", "SparseGroupNorm", "SparseToDense",
     "SubmanifoldConvolution", "Tanh", "SparseConvNetTensor", "Metadata", "set_precision", "get_precision",
-    "feature_dtype", "set_lazy_dense", "SparseDenseTensor", "set_fusion", "set_rulebook_stream", "prefetch", "prepare_weight_images", "release_weight_images",
+    "feature_dtype", "SparseDenseTensor", "prefetch", "prepare_weight_images", "release_weight_images",
 ]

@@ -25,8 +25,7 @@ import torch
 from .._lib import PREC_BF16, PREC_FP32, PREC_TF32
 
 _MODES = ("fp32", "mixed", "tf32", "bf16")
-_state = {"mode": os.environ.get("SCN_B200_PRECISION", "fp32"),
-          "fusion": os.environ.get("SCN_B200_FUSION", "1") not in ("0", "false", "False")}
+_state = {"mode": os.environ.get("SCN_B200_PRECISION", "fp32")}
 if _state["mode"] not in _MODES:
     raise ValueError(f"SCN_B200_PRECISION must be one of {_MODES}")
 
@@ -48,11 +47,3 @@ def feature_dtype() -> torch.dtype:
 def precision_code() -> int:
     return {"fp32": PREC_FP32, "tf32": PREC_TF32}.get(_state["mode"], PREC_BF16)
 
-
-def set_fusion(flag: bool) -> None:
-    """Cross-module fusion of BatchNormalization/AddTable with a following LeakyReLU/ReLU (one kernel instead of two)."""
-    _state["fusion"] = bool(flag)
-
-
-def fusion_enabled() -> bool:
-    return _state["fusion"]

@@ -7,7 +7,6 @@ It is shared by reference by every tensor derived from one InputLayer call.
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass
 from typing import Dict, Tuple
 
@@ -58,13 +57,6 @@ class StridedRule:
 
 
 _side_streams: Dict[torch.device, "torch.cuda.Stream"] = {}
-_side_enabled = os.environ.get("SCN_B200_RULEBOOK_STREAM", "1") not in ("0", "false", "False")
-
-
-def set_rulebook_stream(flag: bool) -> None:
-    """Rulebooks on their own CUDA stream (default) or on the caller's stream."""
-    global _side_enabled
-    _side_enabled = bool(flag)
 
 
 class _RulebookStream:
@@ -84,38 +76,34 @@ class _RulebookStream:
         md = self.md
         self.main = torch.cuda.current_stream(md.device)
         self.prefetch = md._prefetch is not None
-        self.active = (_side_enabled or self.prefetch) and md.device.type == "cuda"
-        if self.active:
-            side = _side_streams.get(md.device)
-            if side is None:
-                side = _side_streams[md.device] = torch.cuda.Stream(device=md.device)
-            self.side = side
-            if self.join_first:
-                if not self.prefetch:        # the coordinates were produced on the caller's stream
-                    side.wait_stream(self.main)
-                elif md._prefetch["ready"] is not None:      # ... or by a copy whose completion event we were given
-                    side.wait_event(md._prefetch["ready"])
-            torch.cuda.set_stream(side)
+        side = _side_streams.get(md.device)
+        if side is None:
+            side = _side_streams[md.device] = torch.cuda.Stream(device=md.device)
+        self.side = side
+        if self.join_first:
+            if not self.prefetch:        # the coordinates were produced on the caller's stream
+                side.wait_stream(self.main)
+            elif md._prefetch["ready"] is not None:      # ... or by a copy whose completion event we were given
+                side.wait_event(md._prefetch["ready"])
+        torch.cuda.set_stream(side)
         return self
 
     def publish(self, *tensors):
-        if self.active:
-            for t in tensors:
-                if t is not None:
-                    if self.prefetch:        # the consuming stream is not known yet: registered when the metadata is taken
-                        self.md._prefetch["tensors"].append(t)
-                    else:
-                        t.record_stream(self.main)
+        for t in tensors:
+            if t is not None:
+                if self.prefetch:        # the consuming stream is not known yet: registered when the metadata is taken
+                    self.md._prefetch["tensors"].append(t)
+                else:
+                    t.record_stream(self.main)
         return tensors[0] if len(tensors) == 1 else tensors
 
     def __exit__(self, *exc):
-        if self.active:
-            ev = self.side.record_event()
-            torch.cuda.set_stream(self.main)
-            if self.prefetch:
-                self.md._prefetch["event"] = ev      # nobody waits yet: that is the point of prefetching
-            else:
-                self.main.wait_event(ev)
+        ev = self.side.record_event()
+        torch.cuda.set_stream(self.main)
+        if self.prefetch:
+            self.md._prefetch["event"] = ev      # nobody waits yet: that is the point of prefetching
+        else:
+            self.main.wait_event(ev)
         return False
 
 

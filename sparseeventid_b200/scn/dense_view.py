@@ -9,7 +9,7 @@ all of it moving zeros.  Both commute with sparsity: ``tanh(0) == 0`` and the me
 ``sum over active rows / V``.  ``SparseDenseTensor`` intercepts exactly those calls through
 ``__torch_function__`` and evaluates them on the ``[N, C]`` rows; ANY other use (indexing, arithmetic, printing,
 a pooling window that is not the full extent, ...) first materialises the real dense tensor with the
-SparseToDense kernel, so semantics never change.  ``scn.set_lazy_dense(False)`` turns the mechanism off.
+SparseToDense kernel, so semantics never change.
 """
 from __future__ import annotations
 
@@ -18,16 +18,6 @@ import torch.nn.functional as F_torch
 from torch.autograd import Function
 
 from . import ops
-
-_state = {"lazy": True}
-
-
-def set_lazy_dense(flag: bool) -> None:
-    _state["lazy"] = bool(flag)
-
-
-def lazy_dense_enabled() -> bool:
-    return _state["lazy"]
 
 
 class _PooledMeanFn(Function):

@@ -1,5 +1,7 @@
 """autograd.Function wrappers: the host-side mirror of SCN's ``X_updateOutput`` / ``X_backward``
 pairs (SURVEY.md §8b).  Forward and backward both run on the C ABI; nothing is computed by torch.
+The hot modules use the C++ functions of csrc_torch/scn_torch.cpp instead, except under ops.Profiler and for
+parameters that are not contiguous fp32 (modules._native).
 """
 from __future__ import annotations
 
@@ -119,105 +121,44 @@ def prepare_weight_images(modules) -> int:
 
 
 class ConvFn(Function):
-    """out[o] = bias + sum_k x[nbr_fwd[k][o]] @ W[k].
+    """out[o] = bias + sum_k x[nbr_fwd[k][o]] @ W[k], with weight re-layout, contraction, dgrad, wgrad and bias gradient
+    each a C-ABI call of its own (so that ops.Profiler times each kernel).
 
     mirror=True  (submanifold): dgrad uses the same table with B_k = W[K-1-k]^T.
     mirror=False (strided / deconvolution): dgrad uses nbr_bwd (the transposed table) with W[k]^T.
-    `owner` (the module) keeps the weight-image workspaces; with it, forward and backward are ONE C-ABI call each.
     """
 
     @staticmethod
-    def forward(ctx, x, weight, bias, nbr_fwd, nbr_bwd, n_out_rows, mirror, owner=None):
-        return _conv_forward(ctx, x, weight, bias, nbr_fwd, nbr_bwd, n_out_rows, mirror, owner)
+    def forward(ctx, x, weight, bias, nbr_fwd, nbr_bwd, n_out_rows, mirror):
+        x = x.contiguous()
+        prec = config.precision_code()
+        fdt = config.feature_dtype()
+        cin, cout = weight.shape[-2], weight.shape[-1]
+        bprep = ops.prep_weights(_w3(weight), False, False, prec, fdt)
+        b = bias.detach().float().contiguous() if bias is not None else None
+        out = ops.conv_forward(x, nbr_fwd, n_out_rows, cin, cout, bprep, b, prec, fdt)
+        ctx.save_for_backward(x, weight, bias)
+        ctx.nbr_fwd, ctx.nbr_bwd, ctx.mirror, ctx.prec = nbr_fwd, nbr_bwd, mirror, prec
+        ctx.n_out_rows = n_out_rows
+        return out
 
     @staticmethod
     def backward(ctx, dout):
-        return _conv_backward(ctx, dout) + (None,) * 5
-
-
-def _conv_forward(ctx, x, weight, bias, nbr_fwd, nbr_bwd, n_out_rows, mirror, owner):
-    x = x.contiguous()
-    prec = config.precision_code()
-    fdt = config.feature_dtype()
-    K, cin, cout = weight.shape[0], weight.shape[-2], weight.shape[-1]
-    fat = (owner is not None and not ops.profiling() and weight.dtype == torch.float32 and weight.is_contiguous()
-           and (bias is None or (bias.dtype == torch.float32 and bias.is_contiguous())))
-    ctx.fat = fat
-    if fat:
-        ws = owner.workspace(K, cin, cout, prec, fdt, x.device)
-        if ws.path > 0 and x.dtype != fdt:
-            x = ops.convert(x, fdt)
-        # always re-laid: fused optimizers update parameters without bumping Tensor._version (see modules._conv)
-        out = ops.conv_module_forward(x, weight, bias, nbr_fwd, n_out_rows, K, cin, cout, prec, fdt, ws.fwd,
-                                      weight_images_current(ws))
-        ctx.ws = ws
-    else:
+        x, weight, bias = ctx.saved_tensors
+        dout = dout.contiguous()
+        cin, cout = weight.shape[-2], weight.shape[-1]
+        dx = dw = db = None
         w3 = _w3(weight)
-        bprep = ops.prep_weights(w3, False, False, prec, fdt)
-        b = bias.detach().float().contiguous() if bias is not None else None
-        out = ops.conv_forward(x, nbr_fwd, n_out_rows, cin, cout, bprep, b, prec, fdt)
-    ctx.save_for_backward(x, weight, bias)
-    ctx.nbr_fwd, ctx.nbr_bwd, ctx.mirror, ctx.prec = nbr_fwd, nbr_bwd, mirror, prec
-    ctx.n_out_rows = n_out_rows
-    return out
-
-
-def _conv_backward(ctx, dout):
-    """-> (dx, dw, db)"""
-    x, weight, bias = ctx.saved_tensors
-    dout = dout.contiguous()
-    K, cin, cout = weight.shape[0], weight.shape[-2], weight.shape[-1]
-    need_dx, need_dw = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-    need_db = bias is not None and ctx.needs_input_grad[2]
-    dx = dw = db = None
-    if ctx.fat:
-        ws = ctx.ws
-        xw = x
-        if ws.path > 0 and x.dtype != dout.dtype:
-            xw = ops.convert(x, dout.dtype)
-        # parameter gradients: straight into .grad when the trainer asked for it, else into fresh buffers
-        gw = _direct_grad(weight) if need_dw else None
-        gb = _direct_grad(bias) if need_db else None
-        if need_dw and gw is None:
-            dw = torch.empty(weight.shape, dtype=torch.float32, device=x.device)
-        if need_db and gb is None:
-            db = torch.empty(bias.shape, dtype=torch.float32, device=x.device)
-        wimg_t, skip = None, False
-        if need_dx:
-            wimg_t = ws.bwd_buffer(K, cin, cout, ctx.prec, xw.dtype, x.device)
-            skip = weight_images_current(ws)
-        # bias gradient already summed by the BatchNorm backward that produced this grad_output?
-        bdx, colsum = _last_bn_colsum
-        _last_bn_colsum[:] = [None, None]
-        if not (need_db and bdx is not None and bdx.data_ptr() == dout.data_ptr() and bdx.shape == dout.shape
-                and colsum.numel() == cout):
-            colsum = None
-        dx = ops.conv_module_backward(xw, dout, weight, ctx.nbr_fwd, ctx.nbr_bwd, ctx.n_out_rows, K, cin, cout,
-                                      ctx.mirror, ctx.prec, wimg_t, skip, need_dx,
-                                      gw if gw is not None else dw, gw is None,
-                                      gb if gb is not None else db, gb is not None, colsum)
-        if dx is not None and dx.dtype != x.dtype:
-            dx = ops.convert(dx, x.dtype)
-        if gw is not None:
-            _grad_ready(weight)
-        if gb is not None:
-            _grad_ready(bias)
-        return dx, dw, db
-    w3 = _w3(weight)
-    if need_dx:
-        bt = ops.prep_weights(w3, True, ctx.mirror, ctx.prec, x.dtype)
-        dx = ops.conv_forward(dout, ctx.nbr_bwd, x.shape[0], cout, cin, bt, None, ctx.prec, x.dtype,
-                              kind="conv_dgrad")
-    if need_dw:
-        dw = ops.conv_wgrad(x, dout, ctx.nbr_fwd, ctx.n_out_rows, cin, cout, ctx.prec).view_as(weight)
-        dw = dw.to(weight.dtype)
-    if need_db:
-        db = ops.col_sum(dout)
-    return dx, dw, db
-
-
-# [dx, column sums of dx] of the latest training-mode BatchNorm backward (dx kept alive: its address cannot be recycled)
-_last_bn_colsum = [None, None]
+        if ctx.needs_input_grad[0]:
+            bt = ops.prep_weights(w3, True, ctx.mirror, ctx.prec, x.dtype)
+            dx = ops.conv_forward(dout, ctx.nbr_bwd, x.shape[0], cout, cin, bt, None, ctx.prec, x.dtype,
+                                  kind="conv_dgrad")
+        if ctx.needs_input_grad[1]:
+            dw = ops.conv_wgrad(x, dout, ctx.nbr_fwd, ctx.n_out_rows, cin, cout, ctx.prec).view_as(weight)
+            dw = dw.to(weight.dtype)
+        if bias is not None and ctx.needs_input_grad[2]:
+            db = ops.col_sum(dout)
+        return dx, dw, db, None, None, None, None
 
 
 class BatchNormFn(Function):
@@ -242,13 +183,9 @@ class BatchNormFn(Function):
             gw, gb = _direct_grad(ctx.params[0]), _direct_grad(ctx.params[1])
             if gw is None or gb is None:
                 gw = gb = None
-        if ctx.training and x.shape[0] > 0:
-            # the column sums of dx come out of the same pass: the bias gradient of a convolution in front (_conv_backward)
-            dx, dg, db, colsum = ops.bn_backward(x, dout.contiguous(), g, b, stats, ctx.training, ctx.leak, gw, gb, True)
-            _last_bn_colsum[:] = [dx, colsum]
-        else:
-            dx, dg, db = ops.bn_backward(x, dout.contiguous(), g, b, stats, ctx.training, ctx.leak, gw, gb)
-            _last_bn_colsum[:] = [None, None]
+        # column sums unused here, but the profiled pass must time the BatchNorm kernel a training step runs (scn_torch.cpp)
+        colsum = ctx.training and x.shape[0] > 0
+        dx, dg, db = ops.bn_backward(x, dout.contiguous(), g, b, stats, ctx.training, ctx.leak, gw, gb, colsum)[:3]
         if gw is not None:
             _grad_ready(ctx.params[0])
             _grad_ready(ctx.params[1])

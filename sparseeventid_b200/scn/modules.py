@@ -31,6 +31,20 @@ def _mark(*params):
             p._scn_param = True
 
 
+def _native(x, *params):
+    """The C++ autograd functions (csrc_torch/scn_torch.cpp) that run a module forward / backward in one native call,
+    or None where functional.py's per-kernel functions run instead: under ops.Profiler, which times every kernel on its
+    own, and for parameters that are not contiguous fp32."""
+    ext = _ext.get()
+    L.require_cuda(x, "sparse module")
+    if ops.profiling():
+        return None
+    for p in params:
+        if p is not None and (p.dtype != torch.float32 or not p.is_contiguous()):
+            return None
+    return ext
+
+
 def _new_like(input, features, spatial_size=None):
     if spatial_size is None:
         return SparseConvNetTensor(features, input.metadata, input.spatial_size, None, input._spc)
@@ -122,12 +136,10 @@ class _ConvBase(nn.Module):
         return ws
 
     def _conv(self, x, nbr_fwd, nbr_bwd, n_out_rows, mirror):
-        """out = bias + conv(x): the C++ autograd function when the torch extension is built (one native call per
-        forward / backward), else functional.ConvFn (same kernels, more interpreter time)."""
-        ext = _ext.get()
+        """out = bias + conv(x)."""
         w, b = self.weight, self.bias
-        if (ext is not None and x.is_cuda and not ops.profiling() and w.dtype == torch.float32 and w.is_contiguous()
-                and (b is None or (b.dtype == torch.float32 and b.is_contiguous()))):
+        ext = _native(x, w, b)
+        if ext is not None:
             prec, fdt = config.precision_code(), config.feature_dtype()
             K, cin, cout = w.shape[0], w.shape[-2], w.shape[-1]
             ws = self.workspace(K, cin, cout, prec, fdt, x.device)
@@ -143,7 +155,7 @@ class _ConvBase(nn.Module):
             return ext.conv(x, w, b, nbr_fwd, nbr_bwd, n_out_rows, mirror, prec, L.SCN_BF16 if fdt == torch.bfloat16
                             else L.SCN_F32, ws.fwd, wimg_t, skip, getattr(w, "_scn_direct_grad", False),
                             b is not None and getattr(b, "_scn_direct_grad", False))
-        return F.ConvFn.apply(x, w, b, nbr_fwd, nbr_bwd, n_out_rows, mirror, self)
+        return F.ConvFn.apply(x, w, b, nbr_fwd, nbr_bwd, n_out_rows, mirror)
 
     def _check(self, input):
         assert input.features.nelement() == 0 or input.features.size(1) == self.nIn, \
@@ -280,17 +292,15 @@ class BatchNormalization(nn.Module):
             # fused into a following activation -- the running statistics were updated by the first one
             rm = self.running_mean.clone() if second and training else self.running_mean
             rv = self.running_var.clone() if second and training else self.running_var
-            ext = _ext.get()
             w, b = self.weight, self.bias
-            if (ext is not None and x.is_cuda and not ops.profiling()
-                    and (w is None or (w.dtype == torch.float32 and w.is_contiguous() and b.dtype == torch.float32
-                                       and b.is_contiguous()))):
+            ext = _native(x, w, b)
+            if ext is not None:
                 return ext.batch_norm(x, w, b, rm, rv, training, float(self.eps),
                                       float(self.momentum), leak,
                                       w is not None and getattr(w, "_scn_direct_grad", False)
                                       and getattr(b, "_scn_direct_grad", False))
             return F.BatchNormFn.apply(x, w, b, rm, rv, training, float(self.eps), float(self.momentum), leak)
-        if config.fusion_enabled() and float(self.leakiness) == 1.0:
+        if float(self.leakiness) == 1.0:
             # defer by one module: a following LeakyReLU/ReLU becomes the fused leakiness of this same kernel
             return SparseConvNetTensor(None, input.metadata, input.spatial_size, Pending("bn", run, run, lambda: run(second=True)), input._spc)
         return _new_like(input, run())
@@ -321,9 +331,9 @@ class LeakyReLU(nn.Module):
         pend = input.take_pending() if isinstance(input, SparseConvNetTensor) else None
         if pend is not None:
             return _new_like(input, pend.fuse(float(self.leak)))
-        ext = _ext.get()
         x = input.features
-        if ext is not None and x.is_cuda and not ops.profiling():
+        ext = _native(x)
+        if ext is not None:
             return _new_like(input, ext.leaky(x, float(self.leak)))
         return _new_like(input, F.LeakyReLUFn.apply(x, float(self.leak)))
 
@@ -352,15 +362,15 @@ class AddTable(nn.Module):
     """scn.AddTable(): features = sum of the list's features (rows aligned) -- sparse_building_blocks.py:82,96."""
 
     def forward(self, input):
-        if config.fusion_enabled() and len(input) == 2:
+        if len(input) == 2:
             a, b = input[0].features, input[1].features
 
             def run():
                 return F.AddFn.apply(a, b)
 
             def fuse(leak):
-                ext = _ext.get()
-                if ext is not None and a.is_cuda and not ops.profiling():
+                ext = _native(a)
+                if ext is not None:
                     return ext.add_leaky(a, b, leak)
                 return F.AddLeakyFn.apply(a, b, leak)
             return SparseConvNetTensor(None, input[0].metadata, input[0].spatial_size, Pending("add", run, fuse),
@@ -387,10 +397,8 @@ class SparseToDense(nn.Module):
 
         def materialize(feats):
             return F.SparseToDenseFn.apply(feats, lvl.keys, batch, sp3).view((batch, c) + tuple(sp))
-        if dense_view.lazy_dense_enabled():
-            # the dense tensor to every consumer, but tanh / full-extent average pooling run on the rows
-            return dense_view.SparseDenseTensor(input.features, lvl.keys, batch, tuple(sp), materialize)
-        return materialize(input.features)
+        # the dense tensor to every consumer, but tanh / full-extent average pooling run on the rows
+        return dense_view.SparseDenseTensor(input.features, lvl.keys, batch, tuple(sp), materialize)
 
 
 class Sequential(nn.Sequential):

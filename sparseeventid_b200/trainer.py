@@ -10,7 +10,6 @@ src/utils/training_utils.py:13 (Adam lr=1.0 x schedule, eps 1e-6, betas (0.8, 0.
 """
 from __future__ import annotations
 
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -70,11 +69,9 @@ class FlatGradArena:
                     self._param_of_ptr[p.data_ptr()] = p
             elif self.world > 1 and overlap:
                 self._hooks.append(p.register_post_accumulate_grad_hook(self._on_grad))
-        if self.world > 1 and overlap:
+        if self._param_of_ptr:      # the C++ autograd functions report completed in-place gradients through this
             from .scn import _ext
-            ext = _ext.get()
-            if ext is not None:      # the C++ autograd functions report completed in-place gradients through this
-                ext.set_grad_ready_callback(lambda t: self._on_grad(self._param_of_ptr[t.data_ptr()]))
+            _ext.get().set_grad_ready_callback(lambda t: self._on_grad(self._param_of_ptr[t.data_ptr()]))
 
     def _bind(self):
         """(Re-)points every parameter's .grad at its slice of the arena.  optimizer.zero_grad() / model.zero_grad()
@@ -201,7 +198,7 @@ class Trainer:
         self.sched = torch.optim.lr_scheduler.LambdaLR(self.opt, lambda s: warmup_flat_lr(s, peak_lr))
         self.peak_lr = peak_lr
         self.global_step = 0
-        self.graph_head = os.environ.get("SCN_B200_GRAPH_HEAD", "1") not in ("0", "false", "False")
+        self.graph_head = True          # False: the heads and loss run eagerly (the reference of the graphed path)
         self._head_graphs = {}
         self.model.train()
 
@@ -241,7 +238,7 @@ class Trainer:
     # size, channel count), so they are captured once with torch.cuda.make_graphed_callables (dropout included: the
     # capture registers the CUDA generator, every replay draws fresh random numbers) and replayed; the encoder -- whose
     # level sizes are data-dependent -- stays eager.  Eager fallback for anything unexpected (a different batch size, CPU,
-    # a head that does not start with the full-extent pool, SCN_B200_GRAPH_HEAD=0).
+    # a head that does not start with the full-extent pool, graph_head = False).
     def _graphed_head_loss(self, feat, labels):
         if not self.graph_head or self.device.type != "cuda" or not isinstance(feat, torch.Tensor):
             return None

@@ -126,6 +126,31 @@ def test_torch_extension_builds_and_exports_the_module_functions():
         assert hasattr(ext, name), name
 
 
+def test_missing_torch_extension_fails_at_first_forward_not_at_import(tmp_path):
+    """The C++ autograd layer is required but loaded on first use: with it missing, importing the package and building
+    a module work, and the first convolution forward raises a RuntimeError that names the build command."""
+    import subprocess
+    import sys
+    code = f"""
+import torch
+from sparseeventid_b200 import build
+build.TORCH_EXT_SO = {str(tmp_path / "scn_b200_torch.so")!r}
+import sparseconvnet as scn
+from sparseeventid_b200.scn import core
+conv = scn.SubmanifoldConvolution(3, 1, 4, 3, True)
+md, sp = core.Metadata(3, "cpu"), (4, 4, 4)       # a level and its neighbour table, as if already built
+md.levels[sp] = core.Level(torch.zeros(2, dtype=torch.int64), 2, None, None, 0)
+md.subm[(sp, (3, 3, 3))] = torch.full((27, 128), -1, dtype=torch.int32)
+try:
+    conv(core.SparseConvNetTensor(torch.zeros(2, 1), md, torch.LongTensor(list(sp))))
+except RuntimeError as e:
+    print("raised:", e)
+"""
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert "raised: scn_b200_torch.so not found" in r.stdout and "`python -m sparseeventid_b200.build`" in r.stdout, r.stdout
+
+
 @pytest.mark.gpu
 def test_plain_c_caller_runs_on_the_gpu(tmp_path):
     """tools/abi_harness.c -- a C99 program with no Python / torch in the process -- drives the hot path through
