@@ -66,10 +66,8 @@ uint64_t scn_launch_count(void);
 int64_t scn_hash_capacity(int64_t n);
 
 /* coords: [n, ncols] row-major of `coord_dtype`; ncols == dimension+1 (batch index LAST, as
- * produced by src/io/data_transforms.py:43-46,242) or ncols == dimension (single sample). */
-int scn_pack_coords(const void* coords, int coord_dtype, int64_t n, int ncols, int dimension,
-                    uint64_t* keys, void* stream);
-/* The same with a range check: info is int32[4] on the device (zeroed by the caller); info[1] |= 1 when a coordinate
+ * produced by src/io/data_transforms.py:43-46,242) or ncols == dimension (single sample).
+ * info: int32[4] on the device (zeroed by the caller), or NULL for no range check; info[1] |= 1 when a coordinate
  * is outside [0, 65535] or a batch index outside [0, 65534] (two sites would alias in the 16-bit key fields; the
  * host side raises), info[2] = max batch index seen (SCN: batch size = max(argument, max index + 1)).  info[0] and
  * info[3] are free for the caller (the InputLayer host code has scn_input_layer_rules write n_active to info[0] so
@@ -110,16 +108,10 @@ int scn_subm_rulebook(const uint64_t* keys, int64_t n, const uint64_t* table_key
                       int32_t* nbr, int64_t n_pad, void* stream);
 
 /* Strided convolution with filter == stride (every use in the reference): output site
- * q = floor(p / s), offset k = rowmajor(p mod s).  Output rows are numbered by ascending key.
- * Writes keys_out[0..n_out) (sorted), out_row_of_in[n], off_of_in[n], *n_out_dev.
- * workspace: scn_strided_workspace(n) bytes. */
-size_t scn_strided_workspace(int64_t n);
-int scn_strided_rulebook(const uint64_t* keys_in, int64_t n, int s0, int s1, int s2,
-                         uint64_t* keys_out, int32_t* out_row_of_in, int32_t* off_of_in,
-                         int32_t* n_out_dev, void* workspace, size_t workspace_bytes, void* stream);
-/* The same rulebook through the coordinate hash (what the modules use): output rows are numbered in FIRST-APPEARANCE
- * order over the input rows (SparseConvNet creates output rows on first touch), keys_out[0..n_out) is in that order,
- * and table_keys / table_vals (capacity >= scn_hash_capacity(n)) receive the coarse level's hash table.
+ * q = floor(p / s), offset k = rowmajor(p mod s).  Output rows are numbered in FIRST-APPEARANCE
+ * order over the input rows (SparseConvNet creates output rows on first touch).
+ * Writes keys_out[0..n_out) (in that order), out_row_of_in[n], off_of_in[n], *n_out_dev, and
+ * table_keys / table_vals (capacity >= scn_hash_capacity(n)) receive the coarse level's hash table.
  * workspace: scn_strided_hash_workspace(n) bytes. */
 size_t scn_strided_hash_workspace(int64_t n);
 int scn_strided_rulebook_hash(const uint64_t* keys_in, int64_t n, int s0, int s1, int s2,
@@ -194,10 +186,8 @@ int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, int dout_dtyp
                    int precision, float* dW, void* stream);
 
 
-/* dbias[c] = sum_rows dout[r][c]  (fp32 out, overwritten).  stats_ws: 2*C doubles of scratch.
- * scn_col_sum_acc: out[c] += ... when accumulate != 0 (gradient accumulated in place). */
-int scn_col_sum(const void* x, int dtype, int64_t n, int C, double* stats_ws, float* out,
-                void* stream);
+/* dbias[c] = sum_rows dout[r][c]  (fp32 out, overwritten, or out[c] += ... when accumulate != 0:
+ * gradient accumulated in place).  stats_ws: 2*C doubles of scratch. */
 int scn_col_sum_acc(const void* x, int dtype, int64_t n, int C, double* stats_ws, float* out,
                     int accumulate, void* stream);
 
@@ -209,20 +199,15 @@ int scn_col_sum_acc(const void* x, int dtype, int64_t n, int C, double* stats_ws
  *   (K,Cin,Cout) / (K,Cout,Cin); skip_prep != 0 when the workspace already holds the image of
  *   the current W.  Forward: out = bias + conv(x) through nbr.  Backward (each part optional,
  *   NULL skips it): dx through nbr_bwd with W^T (mirror: W[K-1-k]^T, submanifold), dW += x^T dout
- *   through nbr_fwd (zero_dW clears it first), dbias (+)= column sums of dout.
+ *   through nbr_fwd (zero_dW clears it first), dbias (+)= column sums of dout.  When those column
+ *   sums are already known (dout_colsum: fp32 [Cout], e.g. from scn_bn_backward_colsum), dbias
+ *   (+)= dout_colsum without another pass over dout; dout_colsum = NULL computes them (stats_ws:
+ *   2*Cout doubles of scratch).
  * ------------------------------------------------------------------------------------------ */
 int scn_conv_module_forward(const void* x, int x_dtype, int64_t n_in_rows, const int32_t* nbr,
                             int K, int64_t n_out_rows, int64_t n_pad, int Cin, int Cout,
                             const float* W, const float* bias, int precision, void* wimg,
                             int skip_prep, void* out, int out_dtype, void* stream);
-int scn_conv_module_backward(const void* x, int x_dtype, int64_t n_in_rows, const void* dout,
-                             int dout_dtype, int64_t n_out_rows, const int32_t* nbr_fwd,
-                             int64_t n_pad_fwd, const int32_t* nbr_bwd, int64_t n_pad_bwd, int K,
-                             int Cin, int Cout, const float* W, int mirror, int precision,
-                             void* wimg_t, int skip_prep, void* dx, float* dW, int zero_dW,
-                             float* dbias, int accumulate_dbias, double* stats_ws, void* stream);
-/* scn_conv_module_backward when the column sums of dout are already known (dout_colsum: fp32 [Cout], e.g. from
- * scn_bn_backward_colsum; NULL = compute them): dbias (+)= dout_colsum without another pass over dout. */
 int scn_conv_module_backward_colsum(const void* x, int x_dtype, int64_t n_in_rows, const void* dout,
                              int dout_dtype, int64_t n_out_rows, const int32_t* nbr_fwd,
                              int64_t n_pad_fwd, const int32_t* nbr_bwd, int64_t n_pad_bwd, int K,
@@ -243,15 +228,11 @@ int scn_bn_forward(const void* x, int dtype, int64_t n, int C, const float* gamm
                    float eps, float momentum, float leakiness, float* save_mean,
                    float* save_invstd, double* stats_ws, void* out, void* stream);
 /* dx, dgamma[C], dbeta[C] (fp32; overwritten, or accumulated into when accumulate_params != 0).
- * `training` selects batch- or running-stat form. */
-int scn_bn_backward(const void* x, const void* dout, int dtype, int64_t n, int C,
-                    const float* gamma, const float* beta, const float* save_mean,
-                    const float* save_invstd, int training, float leakiness, double* stats_ws,
-                    void* dx, float* dgamma, float* dbeta, int accumulate_params, void* stream);
-/* scn_bn_backward that also writes dx_colsum[c] = sum over the n rows of dx[:, c] as stored (fp32 [C]; may be NULL):
- * when the BatchNormalization follows a convolution with a bias (src/networks/sparse_building_blocks.py:29-39) that
- * IS the convolution's bias gradient (SCN: Convolution backward, d_bias = column sums of d_output), produced in the
- * pass that writes dx instead of by one more pass over it. */
+ * `training` selects batch- or running-stat form.  dx_colsum (fp32 [C], or NULL to skip it) receives
+ * the sum over the n rows of dx[:, c] as stored: when the BatchNormalization follows a convolution
+ * with a bias (src/networks/sparse_building_blocks.py:29-39) that IS the convolution's bias gradient
+ * (SCN: Convolution backward, d_bias = column sums of d_output), produced in the pass that writes dx
+ * instead of by one more pass over it. */
 int scn_bn_backward_colsum(const void* x, const void* dout, int dtype, int64_t n, int C,
                            const float* gamma, const float* beta, const float* save_mean,
                            const float* save_invstd, int training, float leakiness, double* stats_ws,

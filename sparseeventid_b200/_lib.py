@@ -25,7 +25,6 @@ SIGNATURES = {
     "scn_version": (C.c_char_p, []),
     "scn_launch_count": (C.c_uint64, []),
     "scn_hash_capacity": (_i64, [_i64]),
-    "scn_pack_coords": (_i, [_p, _i, _i64, _i, _i, _p, _p]),
     "scn_pack_coords_checked": (_i, [_p, _i, _i64, _i, _i, _p, _p, _p]),
     "scn_unpack_keys": (_i, [_p, _i64, _p, _p]),
     "scn_hash_build": (_i, [_p, _i64, _p, _p, _i64, _p]),
@@ -33,8 +32,6 @@ SIGNATURES = {
     "scn_input_rules_workspace": (_sz, [_i64]),
     "scn_input_layer_rules": (_i, [_p, _i64, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "scn_subm_rulebook": (_i, [_p, _i64, _p, _p, _i64, _i, _i, _i, _p, _i64, _p]),
-    "scn_strided_workspace": (_sz, [_i64]),
-    "scn_strided_rulebook": (_i, [_p, _i64, _i, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "scn_strided_hash_workspace": (_sz, [_i64]),
     "scn_strided_rulebook_hash": (_i, [_p, _i64, _i, _i, _i, _p, _p, _i64, _p, _p, _p, _p, _p, _sz, _p]),
     "scn_strided_tables": (_i, [_p, _p, _i64, _i, _p, _i64, _p, _i64, _p]),
@@ -47,15 +44,11 @@ SIGNATURES = {
     "scn_conv_prep_bytes": (_sz, [_i, _i, _i, _i, _i]),
     "scn_conv_forward": (_i, [_p, _i, _i64, _p, _i, _i64, _i64, _i, _i, _p, _p, _i, _p, _i, _p]),
     "scn_conv_wgrad": (_i, [_p, _i, _p, _i, _p, _i, _i64, _i64, _i, _i, _i, _p, _p]),
-    "scn_col_sum": (_i, [_p, _i, _i64, _i, _p, _p, _p]),
     "scn_col_sum_acc": (_i, [_p, _i, _i64, _i, _p, _p, _i, _p]),
     "scn_conv_module_forward": (_i, [_p, _i, _i64, _p, _i, _i64, _i64, _i, _i, _p, _p, _i, _p, _i, _p, _i, _p]),
-    "scn_conv_module_backward": (_i, [_p, _i, _i64, _p, _i, _i64, _p, _i64, _p, _i64, _i, _i, _i, _p, _i, _i, _p, _i,
-                                      _p, _p, _i, _p, _i, _p, _p]),
     "scn_conv_module_backward_colsum": (_i, [_p, _i, _i64, _p, _i, _i64, _p, _i64, _p, _i64, _i, _i, _i, _p, _i, _i, _p, _i,
                                       _p, _p, _i, _p, _i, _p, _p, _p]),
     "scn_bn_forward": (_i, [_p, _i, _i64, _i, _p, _p, _p, _p, _i, _f, _f, _f, _p, _p, _p, _p, _p]),
-    "scn_bn_backward": (_i, [_p, _p, _i, _i64, _i, _p, _p, _p, _p, _i, _f, _p, _p, _p, _p, _i, _p]),
     "scn_bn_backward_colsum": (_i, [_p, _p, _i, _i64, _i, _p, _p, _p, _p, _i, _f, _p, _p, _p, _p, _i, _p, _p]),
     "scn_leaky_forward": (_i, [_p, _i, _i64, _f, _p, _p]),
     "scn_leaky_backward": (_i, [_p, _p, _i, _i64, _f, _p, _p]),

@@ -17,7 +17,7 @@ int scn_stem_tc_forward(const void* x, int x_dtype, const int32_t* nbr, int K, i
 int scn_stem_tc_wgrad(const void* x, int x_dtype, const void* dout, int dout_dtype, const int32_t* nbr, int K, int64_t n_rows,
                       int64_t n_pad, float* dW, cudaStream_t s);
 int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int Cin, int Cout,
-                 int tf32, float* dW, cudaStream_t s);
+                 int tf32, float* dW, const float* colsum, float* dbias, int accumulate, cudaStream_t s);
 int scn_tc_forward(const void* in, int64_t n_in_rows, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int n_in,
                    int n_out, const void* bimg, const float* bias, void* out, int tf32, cudaStream_t s);
 
@@ -605,10 +605,12 @@ extern "C" int scn_conv_forward(const void* in, int in_dtype, int64_t n_in_rows,
   return SCN_ERR_ARG;
 }
 
-extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, int dout_dtype, const int32_t* nbr,
-                              int K, int64_t n_rows, int64_t n_pad, int n_in, int n_out, int precision, float* dW,
-                              void* stream) {
-  cudaStream_t s = (cudaStream_t)stream;
+// scn_conv_wgrad that also adds dbias[n_out] (+)= colsum (accumulate_dbias) when colsum != NULL and the tcgen05 path can
+// fold it into its reduction kernel; *bias_folded tells whether it did (otherwise the caller adds it: module_api.cu).
+int scn_conv_wgrad_fold(const void* in, int in_dtype, const void* dout, int dout_dtype, const int32_t* nbr, int K,
+                        int64_t n_rows, int64_t n_pad, int n_in, int n_out, int precision, float* dW, const float* colsum,
+                        float* dbias, int accumulate_dbias, bool* bias_folded, cudaStream_t s) {
+  *bias_folded = false;
   if (n_rows == 0) return SCN_OK;
   if (!in || !dout || !nbr || !dW || K < 1 || n_pad < n_rows) return SCN_ERR_ARG;
   if (precision == SCN_PREC_FP32 && (in_dtype != SCN_F32 || dout_dtype != SCN_F32)) return SCN_ERR_ARG;
@@ -617,7 +619,9 @@ extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, in
   if ((tc_bf16 || tc_tf) && (n_pad & 127) == 0) {
     // tcgen05 path.  The number of rows of `in` is not part of this entry point's signature; the kernel addresses
     // gathered rows through 32-bit offsets in 16-byte units, i.e. feature matrices up to 64 GB.
-    int rc = scn_wgrad_tc(in, dout, nbr, K, n_rows, n_pad, n_in, n_out, tc_tf ? 1 : 0, dW, s);
+    int rc = scn_wgrad_tc(in, dout, nbr, K, n_rows, n_pad, n_in, n_out, tc_tf ? 1 : 0, dW, colsum, dbias,
+                          accumulate_dbias, s);
+    *bias_folded = rc == SCN_OK && colsum != nullptr;
     if (rc != SCN_ERR_UNSUPPORTED) return rc;
   }
   // the stem (one input channel): dense GEMM over the neighbour table on tensor cores (stem_tc.cu); bf16 dout, and fp32
@@ -645,4 +649,12 @@ extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, in
     return wgrad_generic_t<__nv_bfloat16, __nv_bfloat16>((const __nv_bfloat16*)in, (const __nv_bfloat16*)dout, nbr, K,
                                                          n_rows, n_pad, n_in, n_out, dW, s);
   return SCN_ERR_ARG;
+}
+
+extern "C" int scn_conv_wgrad(const void* in, int in_dtype, const void* dout, int dout_dtype, const int32_t* nbr,
+                              int K, int64_t n_rows, int64_t n_pad, int n_in, int n_out, int precision, float* dW,
+                              void* stream) {
+  bool bias_folded;
+  return scn_conv_wgrad_fold(in, in_dtype, dout, dout_dtype, nbr, K, n_rows, n_pad, n_in, n_out, precision, dW, nullptr,
+                             nullptr, 0, &bias_folded, (cudaStream_t)stream);
 }

@@ -1055,7 +1055,7 @@ int bn_backward_t(const T* x, const T* dout, int64_t n, int C, const float* gamm
   }
   SCN_LAUNCH_CHECK();
   if (colsum)      // paths without the fused column sums: one more pass over dx
-    return scn_col_sum(dx, std::is_same<T, float>::value ? SCN_F32 : SCN_BF16, n, C, ws, colsum, s);
+    return scn_col_sum_acc(dx, std::is_same<T, float>::value ? SCN_F32 : SCN_BF16, n, C, ws, colsum, 0, s);
   return SCN_OK;
 }
 
@@ -1130,18 +1130,6 @@ extern "C" int scn_bn_backward_colsum(const void* x, const void* dout, int dtype
                                                  save_mean, save_invstd, training, leakiness, stats_ws,
                                                  (__nv_bfloat16*)dx, dgamma, dbeta, accumulate_params, dx_colsum, s));
   return SCN_OK;
-}
-
-extern "C" int scn_bn_backward(const void* x, const void* dout, int dtype, int64_t n, int C, const float* gamma,
-                               const float* beta, const float* save_mean, const float* save_invstd, int training,
-                               float leakiness, double* stats_ws, void* dx, float* dgamma, float* dbeta,
-                               int accumulate_params, void* stream) {
-  return scn_bn_backward_colsum(x, dout, dtype, n, C, gamma, beta, save_mean, save_invstd, training, leakiness, stats_ws,
-                                dx, dgamma, dbeta, accumulate_params, nullptr, stream);
-}
-
-extern "C" int scn_col_sum(const void* x, int dtype, int64_t n, int C, double* stats_ws, float* out, void* stream) {
-  return scn_col_sum_acc(x, dtype, n, C, stats_ws, out, 0, stream);
 }
 
 extern "C" int scn_col_sum_acc(const void* x, int dtype, int64_t n, int C, double* stats_ws, float* out, int accumulate,

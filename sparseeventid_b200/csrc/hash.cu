@@ -174,11 +174,6 @@ extern "C" int scn_pack_coords_checked(const void* coords, int coord_dtype, int6
   return SCN_OK;
 }
 
-extern "C" int scn_pack_coords(const void* coords, int coord_dtype, int64_t n, int ncols, int dimension,
-                               uint64_t* keys, void* stream) {
-  return scn_pack_coords_checked(coords, coord_dtype, n, ncols, dimension, keys, nullptr, stream);
-}
-
 extern "C" int scn_unpack_keys(const uint64_t* keys, int64_t n, int32_t* coords4, void* stream) {
   if (n == 0) return SCN_OK;
   if (!keys || !coords4) return SCN_ERR_ARG;

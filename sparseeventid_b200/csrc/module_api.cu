@@ -18,8 +18,10 @@ extern "C" int scn_conv_module_forward(const void* x, int x_dtype, int64_t n_in_
                           out_dtype, stream);
 }
 
-void scn_wgrad_set_bias_fold(const float* colsum, float* dbias, int C, int accumulate);   // wgrad_tc.cu
-bool scn_wgrad_bias_fold_pending();
+// conv.cu
+int scn_conv_wgrad_fold(const void* in, int in_dtype, const void* dout, int dout_dtype, const int32_t* nbr, int K,
+                        int64_t n_rows, int64_t n_pad, int n_in, int n_out, int precision, float* dW, const float* colsum,
+                        float* dbias, int accumulate_dbias, bool* bias_folded, cudaStream_t s);
 
 namespace {
 __global__ void k_bias_from_colsum(const float* __restrict__ colsum, float* dbias, int C, int accumulate) {
@@ -27,17 +29,6 @@ __global__ void k_bias_from_colsum(const float* __restrict__ colsum, float* dbia
   if (c < C) dbias[c] = (accumulate ? dbias[c] : 0.f) + colsum[c];
 }
 }  // namespace
-
-extern "C" int scn_conv_module_backward(const void* x, int x_dtype, int64_t n_in_rows, const void* dout, int dout_dtype,
-                                        int64_t n_out_rows, const int32_t* nbr_fwd, int64_t n_pad_fwd,
-                                        const int32_t* nbr_bwd, int64_t n_pad_bwd, int K, int Cin, int Cout,
-                                        const float* W, int mirror, int precision, void* wimg_t, int skip_prep,
-                                        void* dx, float* dW, int zero_dW, float* dbias, int accumulate_dbias,
-                                        double* stats_ws, void* stream) {
-  return scn_conv_module_backward_colsum(x, x_dtype, n_in_rows, dout, dout_dtype, n_out_rows, nbr_fwd, n_pad_fwd, nbr_bwd,
-                                         n_pad_bwd, K, Cin, Cout, W, mirror, precision, wimg_t, skip_prep, dx, dW, zero_dW,
-                                         dbias, accumulate_dbias, nullptr, stats_ws, stream);
-}
 
 extern "C" int scn_conv_module_backward_colsum(const void* x, int x_dtype, int64_t n_in_rows, const void* dout,
                                                int dout_dtype, int64_t n_out_rows, const int32_t* nbr_fwd,
@@ -51,7 +42,7 @@ extern "C" int scn_conv_module_backward_colsum(const void* x, int x_dtype, int64
   // the column sums of dout are known (scn_bn_backward_colsum): the bias gradient needs no pass over dout; the addition
   // rides on the weight gradient's reduction kernel when that runs, else on a C-thread kernel below
   const bool fold = dbias != nullptr && dout_colsum != nullptr;
-  if (fold) scn_wgrad_set_bias_fold(dout_colsum, dbias, Cout, accumulate_dbias);
+  bool bias_folded = false;
   int rc = SCN_OK;
   if (dx) {                                   // dgrad: the same gather-GEMM on the transposed (mirrored) weights
     if (!wimg_t || !nbr_bwd) return SCN_ERR_ARG;
@@ -61,18 +52,17 @@ extern "C" int scn_conv_module_backward_colsum(const void* x, int x_dtype, int64
     }
     rc = scn_conv_forward(dout, dout_dtype, n_out_rows, nbr_bwd, K, n_in_rows, n_pad_bwd, Cout, Cin, wimg_t, nullptr,
                           precision, dx, x_dtype, stream);
-    if (rc != SCN_OK) { scn_wgrad_set_bias_fold(nullptr, nullptr, 0, 0); return rc; }
+    if (rc != SCN_OK) return rc;
   }
   if (dW) {
     if (!x || !nbr_fwd) return SCN_ERR_ARG;
     if (zero_dW) SCN_CUDA(cudaMemsetAsync(dW, 0, (size_t)K * Cin * Cout * sizeof(float), s));
-    rc = scn_conv_wgrad(x, x_dtype, dout, dout_dtype, nbr_fwd, K, n_out_rows, n_pad_fwd, Cin, Cout, precision, dW,
-                        stream);
-    if (rc != SCN_OK) { scn_wgrad_set_bias_fold(nullptr, nullptr, 0, 0); return rc; }
+    rc = scn_conv_wgrad_fold(x, x_dtype, dout, dout_dtype, nbr_fwd, K, n_out_rows, n_pad_fwd, Cin, Cout, precision, dW,
+                             fold ? dout_colsum : nullptr, dbias, accumulate_dbias, &bias_folded, s);
+    if (rc != SCN_OK) return rc;
   }
   if (fold) {
-    if (scn_wgrad_bias_fold_pending()) {       // no reduction kernel ran (no dW wanted, or another wgrad path)
-      scn_wgrad_set_bias_fold(nullptr, nullptr, 0, 0);
+    if (!bias_folded) {                        // no reduction kernel ran (no dW wanted, or another wgrad path)
       k_bias_from_colsum<<<(Cout + 255) / 256, 256, 0, s>>>(dout_colsum, dbias, Cout, accumulate_dbias);
       SCN_LAUNCH_CHECK();
     }

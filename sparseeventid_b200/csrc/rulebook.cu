@@ -50,35 +50,6 @@ __global__ void k_identity_rows(int32_t* __restrict__ dst, int64_t n) {
   if (i < n) dst[i] = (int)i;
 }
 
-__global__ void k_coarse_keys(const uint64_t* __restrict__ keys, int64_t n, int s0, int s1, int s2,
-                              uint64_t* __restrict__ qkeys, int32_t* __restrict__ idx, int32_t* __restrict__ off) {
-  int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  int x0, x1, x2, b;
-  key_unpack(keys[i], x0, x1, x2, b);
-  int q0 = x0 / s0, q1 = x1 / s1, q2 = x2 / s2;
-  qkeys[i] = key_pack(q0, q1, q2, b);
-  idx[i] = (int)i;
-  off[i] = ((x0 - q0 * s0) * s1 + (x1 - q1 * s1)) * s2 + (x2 - q2 * s2);
-}
-
-__global__ void k_head_flags(const uint64_t* __restrict__ sorted, int64_t n, int32_t* __restrict__ flag) {
-  int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (j < n) flag[j] = (j == 0 || sorted[j] != sorted[j - 1]) ? 1 : 0;
-}
-
-__global__ void k_assign_coarse(const uint64_t* __restrict__ sorted, const int32_t* __restrict__ sorted_idx,
-                                const int32_t* __restrict__ flag, const int32_t* __restrict__ incl, int64_t n,
-                                uint64_t* __restrict__ keys_out, int32_t* __restrict__ out_row_of_in,
-                                int32_t* __restrict__ n_out) {
-  int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (j >= n) return;
-  int row = incl[j] - 1;
-  out_row_of_in[sorted_idx[j]] = row;
-  if (flag[j]) keys_out[row] = sorted[j];
-  if (j == n - 1) *n_out = row + 1;
-}
-
 __global__ void k_strided_tables(const int32_t* __restrict__ out_row_of_in, const int32_t* __restrict__ off_of_in,
                                  int64_t n_in, int32_t* __restrict__ down, int64_t n_out_pad,
                                  int32_t* __restrict__ up, int64_t n_in_pad) {
@@ -122,12 +93,6 @@ __global__ void k_fill_pairs(const int32_t* __restrict__ nbr, const int32_t* __r
   if (i == total - 1) offsets[K] = p + (v >= 0);
 }
 
-size_t sort_temp_bytes(int64_t n) {
-  size_t b = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, b, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const int32_t*)nullptr,
-                                  (int32_t*)nullptr, (int)n);
-  return (size_t)round_up_i64((int64_t)b, 256);
-}
 using ValidIter = cub::TransformInputIterator<int32_t, ValidFlag, cub::CountingInputIterator<int64_t>>;
 size_t pairs_scan_temp(int64_t total) {
   size_t b = 0;
@@ -136,14 +101,6 @@ size_t pairs_scan_temp(int64_t total) {
   cub::DeviceScan::ExclusiveSum(nullptr, b, it, (int32_t*)nullptr, (int)total);
   return (size_t)round_up_i64((int64_t)b, 256);
 }
-size_t scan_temp_bytes2(int64_t n) {
-  size_t b = 0;
-  cub::DeviceScan::InclusiveSum(nullptr, b, (const int32_t*)nullptr, (int32_t*)nullptr, (int)n);
-  size_t b2 = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, b2, (const int32_t*)nullptr, (int32_t*)nullptr, (int)n);
-  return (size_t)round_up_i64((int64_t)(b > b2 ? b : b2), 256);
-}
-
 }  // namespace
 
 extern "C" int scn_subm_rulebook(const uint64_t* keys, int64_t n, const uint64_t* table_keys,
@@ -169,49 +126,11 @@ extern "C" int scn_subm_rulebook(const uint64_t* keys, int64_t n, const uint64_t
   return SCN_OK;
 }
 
-extern "C" size_t scn_strided_workspace(int64_t n) {
-  size_t seg8 = (size_t)round_up_i64(n * 8, 256), seg4 = (size_t)round_up_i64(n * 4, 256);
-  size_t a = sort_temp_bytes(n), b = scan_temp_bytes2(n);
-  return 2 * seg8 + 4 * seg4 + (a > b ? a : b) + 256;
-}
-
-extern "C" int scn_strided_rulebook(const uint64_t* keys_in, int64_t n, int s0, int s1, int s2, uint64_t* keys_out,
-                                    int32_t* out_row_of_in, int32_t* off_of_in, int32_t* n_out_dev, void* workspace,
-                                    size_t workspace_bytes, void* stream) {
-  cudaStream_t s = (cudaStream_t)stream;
-  if (s0 < 1 || s1 < 1 || s2 < 1 || !n_out_dev) return SCN_ERR_ARG;
-  if (n == 0) {
-    SCN_CUDA(cudaMemsetAsync(n_out_dev, 0, sizeof(int32_t), s));
-    return SCN_OK;
-  }
-  if (!workspace || workspace_bytes < scn_strided_workspace(n)) return SCN_ERR_WORKSPACE;
-  size_t seg8 = (size_t)round_up_i64(n * 8, 256), seg4 = (size_t)round_up_i64(n * 4, 256);
-  char* w = (char*)workspace;
-  uint64_t* qkeys = (uint64_t*)w;
-  uint64_t* qsorted = (uint64_t*)(w + seg8);
-  int32_t* idx = (int32_t*)(w + 2 * seg8);
-  int32_t* idx_sorted = (int32_t*)(w + 2 * seg8 + seg4);
-  int32_t* flag = (int32_t*)(w + 2 * seg8 + 2 * seg4);
-  int32_t* incl = (int32_t*)(w + 2 * seg8 + 3 * seg4);
-  void* tmp = w + 2 * seg8 + 4 * seg4;
-  size_t tmp_sort = sort_temp_bytes(n), tmp_scan = scan_temp_bytes2(n);
-  k_coarse_keys<<<grid_for(n, 256), 256, 0, s>>>(keys_in, n, s0, s1, s2, qkeys, idx, off_of_in);
-  SCN_LAUNCH_CHECK();
-  SCN_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_sort, qkeys, qsorted, idx, idx_sorted, (int)n, 0, 64, s));
-  k_head_flags<<<grid_for(n, 256), 256, 0, s>>>(qsorted, n, flag);
-  SCN_LAUNCH_CHECK();
-  SCN_CUDA(cub::DeviceScan::InclusiveSum(tmp, tmp_scan, flag, incl, (int)n, s));
-  k_assign_coarse<<<grid_for(n, 256), 256, 0, s>>>(qsorted, idx_sorted, flag, incl, n, keys_out, out_row_of_in,
-                                                   n_out_dev);
-  SCN_LAUNCH_CHECK();
-  return SCN_OK;
-}
-
-// ---- the same rulebook through the coordinate hash (the path the modules use) --------------------------------------
+// ---- strided rulebook (filter == stride) through the coordinate hash ------------------------------------------------
 // Output sites are the distinct coarse keys; they are found and NUMBERED IN FIRST-APPEARANCE ORDER over the input rows
 // by the InputLayer machinery (hash insert with smallest-index-wins, flag, scan), which is SparseConvNet's own order
 // (output rows are created on first touch) and leaves behind the coarse level's hash table, so the next level needs no
-// separate build.  Replaces a 64-bit radix sort (8 onesweep passes per level, ~135 us even for 7 k sites).
+// separate build.  A 64-bit radix sort of the coarse keys costs 8 onesweep passes per level (~135 us even for 7 k sites).
 namespace {
 __global__ void k_coarse_keys_off(const uint64_t* __restrict__ keys, int64_t n, int s0, int s1, int s2,
                                   uint64_t* __restrict__ qkeys, int32_t* __restrict__ off) {

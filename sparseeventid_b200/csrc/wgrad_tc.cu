@@ -410,17 +410,7 @@ int wgrad_slabs(size_t bytes, cudaStream_t s, float** out) {
   return SCN_OK;
 }
 
-struct BiasFold { const float* colsum; float* dbias; int C; int accumulate; };
-static thread_local BiasFold g_fold = {nullptr, nullptr, 0, 0};
-
 }  // namespace wg
-
-// module_api.cu: "dbias (+)= colsum" is pending for the next weight-gradient launch of this thread; scn_wgrad_tc folds
-// it into its reduction kernel when it runs one (and clears it), otherwise the caller does it itself.
-void scn_wgrad_set_bias_fold(const float* colsum, float* dbias, int C, int accumulate) {
-  wg::g_fold = {colsum, dbias, C, accumulate};
-}
-bool scn_wgrad_bias_fold_pending() { return wg::g_fold.colsum != nullptr; }
 
 // the configuration of the last k_wgrad_tc launch (developer entry like scn_tc_debug_knobs, for the tests' coverage
 // check): grid, s_other, s_centre, pairs per stage, slots, nca, ncb; written on the host just before the launch
@@ -431,9 +421,10 @@ extern "C" void scn_wgrad_debug_last_launch(int32_t* out) {
 
 // dW[K][Cin][Cout] += ...; x, dout bf16, or fp32 with tf32 != 0 (TF32 MMAs).  Returns SCN_ERR_UNSUPPORTED for shapes
 // outside the kernel (caller falls back).  Gathered rows are addressed through 32-bit offsets in 16-byte units: x and
-// dout up to 64 GB each.
+// dout up to 64 GB each.  With colsum != NULL the reduction kernel also writes dbias[Cout] (+)= colsum (accumulate):
+// done whenever this returns SCN_OK.
 int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int64_t n_rows, int64_t n_pad, int Cin, int Cout,
-                 int tf32, float* dW, cudaStream_t s) {
+                 int tf32, float* dW, const float* colsum, float* dbias, int accumulate, cudaStream_t s) {
   if ((Cin % 32) || (Cout % 32) || Cin < 32 || Cout < 32 || Cin > 256 || Cout > 256 || K < 1) return SCN_ERR_UNSUPPORTED;
   if ((uint64_t)n_rows * (uint64_t)(Cout * (tf32 ? 4 : 2) / 16) >= 0xffffffffull) return SCN_ERR_UNSUPPORTED;
   if (n_pad < ((n_rows + 127) / 128) * 128) return SCN_ERR_ARG;      // whole 128-row blocks are read
@@ -502,10 +493,8 @@ int scn_wgrad_tc(const void* x, const void* dout, const int32_t* nbr, int K, int
     SCN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     SCN_CUDA(scn_launch_pdl(kern, dim3((unsigned)grid), dim3(wg::THREADS), smem, s, p));
     SCN_LAUNCH_CHECK();
-    const wg::BiasFold bf = wg::g_fold;
-    wg::g_fold = {nullptr, nullptr, 0, 0};
     SCN_CUDA(scn_launch_pdl(wg::k_wgrad_reduce, dim3(grid_for((int64_t)K * CC / 4, 256)), dim3(256), 0, s, (const float*)p.part, dW,
-                            K, CC, p.s_other, p.s_centre, p.centre, bf.colsum, bf.dbias, bf.C, bf.accumulate));
+                            K, CC, p.s_other, p.s_centre, p.centre, colsum, dbias, Cout, accumulate));
     SCN_LAUNCH_CHECK();
     return SCN_OK;
   };

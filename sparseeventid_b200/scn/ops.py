@@ -89,7 +89,7 @@ def pack_coords(coords: torch.Tensor, dimension: int, info: torch.Tensor = None)
     n, ncols = coords.shape
     keys = torch.empty((n,), dtype=torch.int64, device=coords.device)
     L.check(L.lib().scn_pack_coords_checked(L.ptr(coords), L.COORD_CODES[coords.dtype], n, ncols, dimension, L.ptr(keys),
-                                            L.ptr(info), L.stream()), "scn_pack_coords")
+                                            L.ptr(info), L.stream()), "scn_pack_coords_checked")
     return keys
 
 
@@ -296,7 +296,8 @@ def col_sum(x) -> torch.Tensor:
     n, c = x.shape
     ws = torch.empty((2 * c,), dtype=torch.float64, device=x.device)
     out = torch.empty((c,), dtype=torch.float32, device=x.device)
-    L.check(L.lib().scn_col_sum(L.ptr(x), L.dtype_code(x), n, c, L.ptr(ws), L.ptr(out), L.stream()), "scn_col_sum")
+    L.check(L.lib().scn_col_sum_acc(L.ptr(x), L.dtype_code(x), n, c, L.ptr(ws), L.ptr(out), 0, L.stream()),
+            "scn_col_sum_acc")
     return out
 
 

@@ -1,6 +1,6 @@
 """Direct checks of the bandwidth-bound kernels of csrc/elementwise.cu through the C ABI, against float64 references.
 
-BatchNorm (forward, backward, fused column sums of dx) and the column sums (`scn_col_sum`) run in two arms.  Every bar
+BatchNorm (forward, backward, fused column sums of dx) and the column sums (`scn_col_sum_acc`) run in two arms.  Every bar
 is per element, or per channel for statistics and sums; none is relative to the largest element or to a norm.
   * exact: x and dout are integers in [-8, 8] (exact in bf16 and fp32), gamma in {0.5, 1, 2}, beta = 0, leak in
     {1, 0.5}.  Preconditions, asserted from the grid and rows per block of the launch record: every fp32 partial sum
@@ -382,7 +382,7 @@ def bn_inputs(n, C, dtype, case, seed):
 
 
 def check_col_sum(x, what, accumulate=None):
-    """scn_col_sum (or scn_col_sum_acc with `accumulate` as the initial value) against float64."""
+    """scn_col_sum_acc, overwriting (accumulate=None) or onto `accumulate` as the initial value, against float64."""
     from sparseeventid_b200 import _lib as L
     from sparseeventid_b200.scn import ops
     n, C = x.shape
@@ -536,7 +536,7 @@ def test_bn_unaligned_views(C, dtype, training, shift):
 
 def _sequence(second_stream):
     """Two-launch BatchNorm with the channel count rising and falling, four-launch calls (C = 12, unaligned) between
-    them, scn_col_sum and fused-colsum backwards on one stream; optionally one call on a second stream."""
+    them, scn_col_sum_acc and fused-colsum backwards on one stream; optionally one call on a second stream."""
     steps = [(3000, 160, "bn"), (5000, 32, "bn"), (777, 12, "bn4"), (900, 192, "bn"), (4000, 64, "col"),
              (7000, 32, "bn"), (2500, 128, "bn4"), (6000, 96, "bn"), (3333, 192, "col"), (64, 32, "bn")]
     side = torch.cuda.Stream() if second_stream else None

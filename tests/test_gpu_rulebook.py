@@ -612,39 +612,35 @@ def test_device_larcv_transform_edges(V, layout):
 # --------------------------------------------------------------------------------------- F: remaining entry points
 
 
-def _strided_sort(keys_u64, stride):
-    """scn_strided_rulebook (the sort path) on device keys -> (keys_out uint64 [m], out_row_of_in, off_of_in)."""
-    L = _lib()
-    n = keys_u64.shape[0]
-    kin = torch.as_tensor(keys_u64.view(np.int64)).cuda()
-    kout = torch.empty(n, dtype=torch.int64, device="cuda")
-    orow = torch.empty(n, dtype=torch.int32, device="cuda")
-    off = torch.empty(n, dtype=torch.int32, device="cuda")
-    n_out = torch.zeros(1, dtype=torch.int32, device="cuda")
-    wsb = int(L.lib().scn_strided_workspace(n))
-    ws = torch.empty(wsb, dtype=torch.uint8, device="cuda")
-    L.check(L.lib().scn_strided_rulebook(kin.data_ptr(), n, *stride, kout.data_ptr(), orow.data_ptr(), off.data_ptr(),
-                                         n_out.data_ptr(), ws.data_ptr(), wsb, L.stream()), "scn_strided_rulebook")
-    m = int(n_out.item())
-    return kout[:m].cpu().numpy().view(np.uint64), orow.cpu().numpy(), off.cpu().numpy()
+def _strided_hash(keys_u64, stride):
+    """scn_strided_rulebook_hash on device keys -> (keys_out uint64 [m], out_row_of_in, off_of_in)."""
+    kout, orow, off, _ = _ops().strided_rulebook(torch.as_tensor(keys_u64.view(np.int64)).cuda(), stride)
+    return kout.cpu().numpy().view(np.uint64), orow.cpu().numpy(), off.cpu().numpy()
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("stride", [(2, 2, 2), (1, 2, 2), (4, 4, 4)])
-def test_strided_sort_path_bit_exact(stride):
-    """Output rows in ascending UNSIGNED key order: samples 32768 and 65534 come after sample 0."""
+def test_strided_rulebook_bit_exact(stride):
+    """Output rows in FIRST-APPEARANCE order over the input rows (SparseConvNet's order), across batch indices 0, 1,
+    32767, 32768 and 65534 and the 16-bit edge coordinates.  The oracle numbers rows by ascending key: its rows are
+    renumbered by the first input row that reaches each."""
     c = blob_sites(800, (40, 30, 50), 5, seed=12)
     c[:, 3] = np.array([0, 1, 32767, 32768, 65534])[c[:, 3]]
     c = np.concatenate([c, edge_sites()])
     c = c[np.random.default_rng(13).permutation(c.shape[0])]
     out_coords, rules, _ = O.strided_rulebook(c, stride, stride, FULL)
+    sorted_row, want_off = np.full(c.shape[0], -1), np.full(c.shape[0], -1)
+    for k, r in enumerate(rules):
+        sorted_row[r[:, 0]], want_off[r[:, 0]] = r[:, 1], k
+    assert sorted_row.min() >= 0
+    rows, first = np.unique(sorted_row, return_index=True)
+    order = rows[np.argsort(first)]                      # oracle rows in first-appearance order
+    renumber = np.empty_like(order)
+    renumber[order] = np.arange(order.shape[0])
     for run in range(2):
-        kout, orow, off = _strided_sort(O.pack_keys(c), stride)
-        assert np.array_equal(kout, O.pack_keys(out_coords))
-        want_row, want_off = np.full(c.shape[0], -1), np.full(c.shape[0], -1)
-        for k, r in enumerate(rules):
-            want_row[r[:, 0]], want_off[r[:, 0]] = r[:, 1], k
-        assert np.array_equal(orow, want_row) and np.array_equal(off, want_off)
+        kout, orow, off = _strided_hash(O.pack_keys(c), stride)
+        assert np.array_equal(kout, O.pack_keys(out_coords)[order])
+        assert np.array_equal(orow, renumber[sorted_row]) and np.array_equal(off, want_off)
 
 
 @pytest.mark.gpu

@@ -168,7 +168,7 @@ int main(void) {
   int32_t* coords_dev = (int32_t*)dmalloc(sizeof coords);
   h2d(coords_dev, coords, sizeof coords);
   uint64_t* keys_in = (uint64_t*)dmalloc(N_IN * 8);
-  CK(scn_pack_coords(coords_dev, SCN_COORD_I32, N_IN, 4, 3, keys_in, NULL));
+  CK(scn_pack_coords_checked(coords_dev, SCN_COORD_I32, N_IN, 4, 3, keys_in, NULL, NULL));
   int64_t cap = scn_hash_capacity(N_IN);
   uint64_t* tkeys = (uint64_t*)dmalloc((size_t)cap * 8);
   int32_t* tvals = (int32_t*)dmalloc((size_t)cap * 4);
@@ -229,13 +229,17 @@ int main(void) {
 
   /* ---- AveragePooling 2x2x2: strided rulebook, tables, gather-sum ---- */
   {
-    size_t sws_bytes = scn_strided_workspace(n_act);
+    size_t sws_bytes = scn_strided_hash_workspace(n_act);
     void* sws = dmalloc(sws_bytes);
+    int64_t ocap = scn_hash_capacity(n_act);
+    uint64_t* otkeys = (uint64_t*)dmalloc((size_t)ocap * 8);
+    int32_t* otvals = (int32_t*)dmalloc((size_t)ocap * 4);
     uint64_t* keys_out = (uint64_t*)dmalloc((size_t)n_act * 8);
     int32_t* out_row = (int32_t*)dmalloc((size_t)n_act * 4);
     int32_t* off = (int32_t*)dmalloc((size_t)n_act * 4);
     int32_t* n_out_dev = (int32_t*)dmalloc(4);
-    CK(scn_strided_rulebook(keys_act, n_act, 2, 2, 2, keys_out, out_row, off, n_out_dev, sws, sws_bytes, NULL));
+    CK(scn_strided_rulebook_hash(keys_act, n_act, 2, 2, 2, otkeys, otvals, ocap, keys_out, out_row, off, n_out_dev, sws,
+                                 sws_bytes, NULL));
     int32_t n_out = 0;
     d2h(&n_out, n_out_dev, 4);
     int64_t n_out_pad = (n_out + 127) / 128 * 128;

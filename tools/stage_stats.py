@@ -77,8 +77,7 @@ def main():
         coarse = active.copy()
         coarse[:, :3] //= 2
         _, first = np.unique(pack(coarse), return_index=True)
-        active = coarse[np.sort(first)]                  # sorted-key order = what scn_strided_rulebook produces
-        active = active[np.argsort(pack(active), kind="stable")]
+        active = coarse[np.sort(first)]                  # first appearance = what scn_strided_rulebook_hash produces
 
 
 if __name__ == "__main__":
